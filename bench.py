@@ -4,6 +4,7 @@ joint-VAE, K=128, L=16, C=10, batch 512 per GPU, bf16 GEMMs; plus OOD-scoring sa
 
   python bench.py --gpus N --steps K --warmup W          (N>1: launched by torch.distributed.run, one rank per GPU)
   python bench.py --impl reference ...                    the reference's algorithm (oracle port) on the host cores
+  python bench.py ... --dump-outputs DIR                  also writes the last timed step's outputs as DIR/<name>.npy
 
 A "step" is one full optimisation step of the path: zero_grad, weight re-pack, features/encoder/sampler/decoder/classifier
 forward, fused ELBO forward + backward, network backward, gradient all-reduce (N > 1), global-norm clip, Adam.
@@ -21,6 +22,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree, which may be read-only
 
 OPT = {'optim_type': 'adam', 'lr': 1e-3, 'weight_decay': 3e-5, 'grad_clipping': 100}
 
@@ -49,6 +51,7 @@ WORKLOADS = {
 }
 PRIOR = {'init_mean': 1.0, 'learned_means': True, 'var_dim': 'scalar', 'seed': 1}
 C5_SAMPLES = 1 << 20          # configs[4]: 1 Mi synthetic test samples (half of them drawn as the OOD set)
+PREROLL_STEPS = 48            # untimed steps right before the timed region (run_native)
 
 
 def peaks():
@@ -227,7 +230,7 @@ def run_native(args, wl):
     if world > 1:
         os.environ.setdefault('MASTER_ADDR', '127.0.0.1')
         dist.init_process_group('nccl', device_id=dev)
-    pkg = g.build()
+    pkg = g.load()
     nat = pkg._native
 
     def barrier():
@@ -235,16 +238,21 @@ def run_native(args, wl):
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(fn, steps):
-        """CUDA-event time of `steps` calls bracketed by barrier + synchronize, max over ranks (ms)"""
+    def timed(fn, steps, before_last=None):
+        """CUDA-event time of `steps` calls bracketed by barrier + synchronize, max over ranks (ms); `before_last` is enqueued
+        ahead of the last call and its device time is left out"""
         barrier()
-        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a, b, c, d = (torch.cuda.Event(enable_timing=True) for _ in range(4))
         a.record()
         for i in range(steps):
+            if before_last is not None and i == steps - 1:
+                c.record()
+                before_last()
+                d.record()
             fn(i)
         b.record()
         barrier()
-        ms = a.elapsed_time(b)
+        ms = a.elapsed_time(b) - (c.elapsed_time(d) if before_last is not None else 0.0)
         if world > 1:
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -268,6 +276,17 @@ def run_native(args, wl):
     # ================================================================ headline workload: train step
     net = build_net(wl)
     net.train()
+    # the seeded initial state, restored ahead of the last timed step: the training trajectory is not bit-reproducible (fp32
+    # atomics in the weight-gradient reductions, amplified by Adam), so only a step that starts from these parameters computes
+    # the same outputs from the same batch and noise in every run (--dump-outputs)
+    initial = {k: v.detach().clone() for k, v in net.state_dict().items()}
+
+    def restore_initial():
+        with torch.no_grad():
+            for k, v in net.state_dict().items():
+                v.copy_(initial[k])
+        pkg.engine.bump_params()
+        pkg.engine.bump_stats()
     B = args.batch or wl['batch']
     C = wl['ctor']['num_labels']
     shape = tuple(wl['ctor']['input_shape'])
@@ -275,7 +294,10 @@ def run_native(args, wl):
     xs_h, ys_h, xs, ys = train_inputs(wl, B, npool)
     use_graph = args.graph                     # N > 1: the NCCL all-reduce is a node of the captured step
     step_eager = lambda i: net.train_step(xs[i % npool], ys[i % npool])
-    step_dev = lambda i: net.train_step(xs[i % npool], ys[i % npool], graph=use_graph)
+    last = {}           # what the latest step returned: the last timed step's losses / measures for --dump-outputs
+
+    def step_dev(i):
+        last['out'] = net.train_step(xs[i % npool], ys[i % npool], graph=use_graph)
 
     def step_e2e(i):
         x = xs_h[i % npool].to(dev, non_blocking=True)
@@ -309,16 +331,17 @@ def run_native(args, wl):
     # the published value: the same steps without per-launch events, through the public train_step (CUDA-graph replays when
     # --graph, the default on one GPU: same kernels, same arithmetic, no per-launch host cost)
     clocks = ClockSampler(local)        # started ahead of the timed region: nvidia-smi needs ~0.1-0.3 s for its first row
-    # the same steps, untimed, for ~0.5 s while the sampler starts; the count comes from the (max-over-ranks) eager step time, so
-    # every rank runs the same number of data-parallel steps
-    n_w = max(3, min(100, int(500.0 / max(1e-3, ms_eager / args.steps)) + 1))
-    for i in range(n_w):
+    # the same steps, untimed, while the sampler starts (~0.5 s of c2 at batch 512); a fixed count rather than a time, so every
+    # rank runs the same number of data-parallel steps and the last timed step draws the same noise in every run
+    for i in range(PREROLL_STEPS):
         step_dev(i)
     torch.cuda.synchronize()
     clocks.mark(True)
-    ms = timed(step_dev, args.steps)
+    ms = timed(step_dev, args.steps, before_last=restore_initial)
     clocks.mark(False)
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last['out'])      # before later steps overwrite the graph's output buffers
     ms_plain = ms_eager
     # ---- end-to-end timing through the public API with host buffers
     step_e2e(0)
@@ -437,6 +460,19 @@ def run_native(args, wl):
     _finish(world)
 
 
+def dump_outputs(path, losses, measures):
+    """What a caller of train_step receives from the last timed step, as <path>/<name>.npy: the per-sample losses
+    (`loss.<key>`, float32) and the running measures (`measure.<key>`, float64 scalars).  That step starts from the seeded
+    initial parameters, and its batch and noise follow from the seeds and the arguments alone, so two builds run with the
+    same arguments can be compared output for output."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {'loss.' + k: v.detach().float().cpu().numpy() for k, v in losses.items()}
+    arrays.update({'measure.' + k: np.float64(float(v)) for k, v in measures.items()})
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), a)
+
+
 def _finish(world):
     """End of a rank.  With N > 1 the captured data-parallel steps hold NCCL kernels inside CUDA graphs; tearing the communicator
     down under them can block, so the rank synchronises, meets the others at a barrier and leaves without the teardown."""
@@ -541,7 +577,13 @@ def main():
     ap.add_argument('--c5-samples', type=int, default=C5_SAMPLES)
     ap.add_argument('--no-extra', dest='extra', action='store_false', help='skip the c3 / c4 train-step sub-results')
     ap.add_argument('--traffic', type=float, default=None, help='ncu dram bytes per launch of the dominant kernel (from profiles/)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write the losses and measures of the last timed train step (rank 0's) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'native':
+        ap.error('--dump-outputs writes the outputs of the native path')
     wl = WORKLOADS[args.workload]
     if args.impl == 'reference':
         run_reference(args, wl)

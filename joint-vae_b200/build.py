@@ -33,6 +33,14 @@ def _digest():
     return h.hexdigest()
 
 
+def current():
+    """Whether the library was built from the present sources and flags (reads only)."""
+    if not (os.path.exists(LIB) and os.path.exists(STAMP)):
+        return False
+    with open(STAMP) as f:
+        return f.read().strip() == _digest()
+
+
 def build(force=False, verbose=False):
     """Compiles csrc/*.cu when the sources changed since the last build.  Safe to call from several processes at once
     (one rank per GPU under torchrun): an exclusive file lock serialises them and the late comers find the fresh stamp."""
@@ -49,7 +57,7 @@ def build(force=False, verbose=False):
 def _build_locked(force, verbose):
     nvcc = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
     dig = _digest()
-    if not force and os.path.exists(LIB) and os.path.exists(STAMP) and open(STAMP).read().strip() == dig:
+    if not force and current():
         return LIB
     if not os.path.exists(nvcc):
         if os.path.exists(LIB):      # GPU box without toolkit changes: use the prebuilt library

@@ -27,6 +27,16 @@ def rel(a, b):
     return float(np.abs(a - b).max() / max(1e-6, np.abs(b).max()))
 
 
+def _load(name):
+    """the golden as a dict; the torch.rand inputs (multiples of 2^-24) are stored as their 24-bit integers, three
+    little-endian bytes per value (tests/golden/make_multistep_golden.py), and decode exactly to the float32 inputs"""
+    d = dict(np.load(os.path.join(GOLDEN, name + '.npz')))
+    for k in [k for k in d if k.endswith('.u24')]:
+        b = d.pop(k).astype(np.uint32)
+        d[k[:-4]] = (b[..., 0] | b[..., 1] << 8 | b[..., 2] << 16).astype(np.float32) * np.float32(2 ** -24)
+    return d
+
+
 def _build(pkg, cfg_json, sd):
     kw = json.loads(cfg_json)
     kw['input_shape'] = tuple(kw['input_shape'])
@@ -36,9 +46,9 @@ def _build(pkg, cfg_json, sd):
 
 
 def _drive(pkg, name):
-    d = np.load(os.path.join(GOLDEN, name + '.npz'))
+    d = _load(name)
     cfg = str(d['cfg'])
-    net = _build(pkg, cfg, {k[3:]: torch.from_numpy(np.asarray(d[k])) for k in d.files if k.startswith('sd.')})
+    net = _build(pkg, cfg, {k[3:]: torch.from_numpy(np.asarray(d[k])) for k in d if k.startswith('sd.')})
     T = int(d['steps'])
     t = lambda k: torch.from_numpy(d[k]).to(DEV)
     out = {'d': d, 'errs': [], 'meas': [], 'twin': {}}
@@ -48,7 +58,7 @@ def _drive(pkg, name):
         losses, measures = net.train_step(t(f'x.{i}'), t(f'y.{i}'), batch=batch, current_measures=current)
         out['errs'].append({k: rel(v.detach().cpu().numpy(), d[f'step{i}.loss.{k}']) for k, v in losses.items()})
         pre = f'step{i}.measure.'
-        out['meas'].append({k[len(pre):]: (float(measures[k[len(pre):]]), float(d[k])) for k in d.files if k.startswith(pre)})
+        out['meas'].append({k[len(pre):]: (float(measures[k[len(pre):]]), float(d[k])) for k in d if k.startswith(pre)})
         return losses, measures
 
     def evaluate(tag):
