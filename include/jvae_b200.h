@@ -305,6 +305,27 @@ int jvae_bn_apply_fwd(const void* y, size_t P, int C, int ld_y, const double* st
 int jvae_bn_bwd(const void* da, int ld_da, const void* y, int ld_y, size_t P, int C, const float* save_mean_rstd,
                 const float* gamma, const float* beta, int act, double* sums, void* dy, int ld_dy, float* dgamma, float* dbeta,
                 int skip_reduce, void* stream);
+/* DenseNet blocks (torchvision _DenseBlock): every layer appends its channels to ONE (P, C_total) bf16 buffer, whose batch
+ * statistics live in ONE (2, C_total) f64 array (row stride stats_ld = C_total) written once per channel and read by every
+ * later pre-activation BatchNorm; the backward accumulates the channel gradients of all consumers in ONE fp32 buffer.
+ * jvae_bn_stats_ld: stats[c] / stats[stats_ld + c] += sum / sum of squares of y (P, C) for c < C (pass the statistics of
+ * the channel slice's first channel; stats_ld == C is jvae_bn_stats) */
+int jvae_bn_stats_ld(const void* y, size_t P, int C, int ld, double* stats, int stats_ld, void* stream);
+/* jvae_bn_apply_fwd on a channel prefix of a dense block: statistics with row stride stats_ld (sums at stats[c], sums of
+ * squares at stats[stats_ld + c]); gamma / beta / running statistics / num_batches of THIS consumer.  C, ld_y, ld_out
+ * multiples of 8, rows 16-byte aligned. */
+int jvae_bn_preact_fwd(const void* y, size_t P, int C, int ld_y, const double* stats, int stats_ld, const float* gamma,
+                       const float* beta, float eps, float momentum, float* running_mean, float* running_var,
+                       int64_t* num_batches, int training, int act, void* out, int ld_out, float* save_mean_rstd, void* stream);
+/* backward of act(BN(y)) given da, ACCUMULATED: dx (P, C) fp32 with row stride ld_dx += dL/dy.  training != 0: batch
+ * statistics (save_mean_rstd from the forward), sums (2,C) f64 scratch, dgamma / dbeta += (either may be NULL); training == 0:
+ * running statistics, dx += da * act' * gamma * rsqrt(running_var + eps) (the input gradient of an eval-mode network),
+ * sums / dgamma / dbeta unused.  C and every ld multiples of 8, rows 16-byte aligned. */
+int jvae_bn_preact_bwd(const void* da, int ld_da, const void* y, int ld_y, size_t P, int C, const float* save_mean_rstd,
+                       const float* gamma, const float* beta, const float* running_mean, const float* running_var, float eps,
+                       int training, int act, double* sums, float* dx, int ld_dx, float* dgamma, float* dbeta, void* stream);
+/* dst (P, C) bf16 with row stride ld_dst = src (P, C) fp32 with row stride ld_src (a slice of the gradient accumulator) */
+int jvae_cast_f32_bf16_ld(const float* src, int ld_src, void* dst, int ld_dst, size_t P, int C, void* stream);
 /* dy = da * act'(.) expressed with the activation OUTPUT a_out (relu, sigmoid; act none: dy = da, dy may be NULL);
  * dbias (C) f32 += sum over pixels of dy (NULL = not wanted) */
 int jvae_act_bwd(const void* da, int ld_da, const void* a_out, int ld_a, size_t P, int C, int act, void* dy, int ld_dy,

@@ -119,6 +119,12 @@ def lib():
                                     P, P]
     L.jvae_bn_bwd.argtypes = [P, c_int, P, c_int, c_size_t, c_int, P, P, P, c_int, P, P, c_int, P, P, c_int, P]
     L.jvae_act_bwd.argtypes = [P, c_int, P, c_int, c_size_t, c_int, c_int, P, c_int, P, P]
+    L.jvae_bn_stats_ld.argtypes = [P, c_size_t, c_int, c_int, P, c_int, P]
+    L.jvae_bn_preact_fwd.argtypes = [P, c_size_t, c_int, c_int, P, c_int, P, P, c_float, c_float, P, P, P, c_int, c_int, P,
+                                     c_int, P, P]
+    L.jvae_bn_preact_bwd.argtypes = [P, c_int, P, c_int, c_size_t, c_int, P, P, P, P, P, c_float, c_int, c_int, P, P, c_int,
+                                     P, P, P]
+    L.jvae_cast_f32_bf16_ld.argtypes = [P, c_int, P, c_int, c_size_t, c_int, P]
     L.jvae_maxpool_fwd.argtypes = [P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P, c_int, P]
     L.jvae_maxpool_bwd.argtypes = [P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P, c_int, P, c_int, P]
     L.jvae_upsample2.argtypes = [P, c_int, P, c_int, c_int, c_int, c_int, c_int, c_int, P]
@@ -621,6 +627,29 @@ def bn_apply_fwd(y, P, C, ld_y, stats, gamma, beta, eps, momentum, running_mean,
 def bn_bwd(da, ld_da, y, ld_y, P, C, save, gamma, beta, act, sums, dy, ld_dy, dgamma, dbeta, skip_reduce=False):
     check(lib().jvae_bn_bwd(rawptr(da), ld_da, rawptr(y), ld_y, P, C, rawptr(save), rawptr(gamma), rawptr(beta), act,
                             rawptr(sums), rawptr(dy), ld_dy, rawptr(dgamma), rawptr(dbeta), int(skip_reduce), stream()))
+
+
+def bn_stats_ld(y, P, C, ld, stats, stats_ld):
+    """y: (N, H, W, >= C) view whose first channel is the slice's; stats: flat f64 view starting at the slice's channel"""
+    check(lib().jvae_bn_stats_ld(rawptr(y), P, C, ld, rawptr(stats), stats_ld, stream()))
+
+
+def bn_preact_fwd(y, P, C, ld_y, stats, stats_ld, gamma, beta, eps, momentum, running_mean, running_var, num_batches, training,
+                  act, out, ld_out, save):
+    check(lib().jvae_bn_preact_fwd(rawptr(y), P, C, ld_y, rawptr(stats), stats_ld, rawptr(gamma), rawptr(beta), float(eps),
+                                   float(momentum), rawptr(running_mean), rawptr(running_var), rawptr(num_batches),
+                                   int(training), act, rawptr(out), ld_out, rawptr(save), stream()))
+
+
+def bn_preact_bwd(da, ld_da, y, ld_y, P, C, save, gamma, beta, running_mean, running_var, eps, training, act, sums, dx, ld_dx,
+                  dgamma, dbeta):
+    check(lib().jvae_bn_preact_bwd(rawptr(da), ld_da, rawptr(y), ld_y, P, C, rawptr(save), rawptr(gamma), rawptr(beta),
+                                   rawptr(running_mean), rawptr(running_var), float(eps), int(training), act, rawptr(sums),
+                                   rawptr(dx), ld_dx, rawptr(dgamma), rawptr(dbeta), stream()))
+
+
+def cast_f32_bf16_ld(src, ld_src, dst, ld_dst, P, C):
+    check(lib().jvae_cast_f32_bf16_ld(rawptr(src), ld_src, rawptr(dst), ld_dst, P, C, stream()))
 
 
 def act_bwd(da, ld_da, a_out, ld_a, P, C, act, dy, ld_dy, dbias):

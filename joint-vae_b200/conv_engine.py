@@ -93,7 +93,8 @@ class NativeKernels:
     @staticmethod
     def gather(x, Cin, wmat, cout_pad, taps, in_stride, Hq, Wq, out, Cout, out_s, out_o, bias, act, stats, bn=None):
         N, H, W, ld_in = x.shape
-        _, Ho, Wo, ld_out = out.shape
+        _, Ho, Wo, _ = out.shape
+        ld_out = out.stride(2)          # `out` may be a channel slice of a wider buffer (a dense block's new channels)
         return nat.conv_gather_gemm(x, N, H, W, Cin, ld_in, wmat, cout_pad, wmat.shape[1], taps, in_stride, Hq, Wq, out, Ho,
                                     Wo, Cout, ld_out, out_s, out_o, bias, act, stats, bn=bn)
 
@@ -141,6 +142,10 @@ class NativeKernels:
                                       ld_out, out_s, bias, act, stats)
 
     bn_stats = staticmethod(nat.bn_stats)
+    bn_stats_ld = staticmethod(nat.bn_stats_ld)
+    bn_preact_fwd = staticmethod(nat.bn_preact_fwd)
+    bn_preact_bwd = staticmethod(nat.bn_preact_bwd)
+    cast_f32_bf16_ld = staticmethod(nat.cast_f32_bf16_ld)
     bn_apply_fwd = staticmethod(nat.bn_apply_fwd)
     bn_bwd = staticmethod(nat.bn_bwd)
     act_bwd = staticmethod(nat.act_bwd)
@@ -517,7 +522,11 @@ class ConvStep:
         pk = self._pack()
         bias = self.conv.bias.detach() if self.conv.bias is not None else None
         fused_act = self.act if bn is None else 0
-        y = K.empty((N, self.Ho, self.Wo, self.ld_y), x)
+        y = st.pop('out', None)          # a channel slice of a dense block's buffer (DenseBlockStep)
+        if y is None:
+            y = K.empty((N, self.Ho, self.Wo, self.ld_y), x)
+        else:
+            assert bn is None and not (self.gemm1x1 or self.dense_small or self.separable or self.merged_fwd)
         stats = (st.pop('stats_buf', None) if bn_train else None)
         if bn_train and stats is None:
             stats = K.zeros((2, self.Co), x, torch.float64)
@@ -766,11 +775,14 @@ class PoolStep:
 
     def forward(self, x, st, training):
         N, _, _, ld = x.shape
-        out = K.empty((N, self.Ho, self.Wo, ld), x)
+        out = st.pop('out', None)        # the first channels of a dense block's buffer (DenseBlockStep)
+        if out is None:
+            out = K.empty((N, self.Ho, self.Wo, ld), x)
+        ldo = out.stride(2)
         if self.general:
-            K.maxpool_pad_fwd(x, N, self.H, self.W, ld, ld, self.k, self.s, self.p, out, ld)
+            K.maxpool_pad_fwd(x, N, self.H, self.W, ld, ld, self.k, self.s, self.p, out, ldo)
         else:
-            K.maxpool_fwd(x, N, self.H, self.W, ld, ld, self.k, self.s, out, ld)      # padded channels are pooled as well
+            K.maxpool_fwd(x, N, self.H, self.W, ld, ld, self.k, self.s, out, ldo)      # padded channels are pooled as well
         st['x'] = x
         return out
 
@@ -811,8 +823,10 @@ class AvgStep:
 
     def forward(self, x, st, training):
         N, _, _, ld = x.shape
-        out = K.empty((N, self.H // self.k, self.W // self.k, ld), x)
-        K.avgpool(x, ld, out, ld, N, self.H, self.W, ld, self.k, False)
+        out = st.pop('out', None)        # the first channels of a dense block's buffer (DenseBlockStep)
+        if out is None:
+            out = K.empty((N, self.H // self.k, self.W // self.k, ld), x)
+        K.avgpool(x, ld, out, out.stride(2), N, self.H, self.W, ld, self.k, False)
         st['ld'] = ld
         return out
 
@@ -899,6 +913,182 @@ class ResidualStep:
         return dx, grads
 
 
+BN_MAX_C = 2048          # csrc/norm.cu: 8 channels per thread, NORM_MAX_THREADS = 256 threads per pixel row
+
+
+def is_dense_block(m):
+    """torchvision.models.densenet._DenseBlock: a ModuleDict of _DenseLayers (duck-typed like is_residual_block)"""
+    return type(m).__name__ == '_DenseBlock' and isinstance(m, nn.ModuleDict)
+
+
+def is_transition(m):
+    """torchvision.models.densenet._Transition: norm -> relu -> conv1x1 -> AvgPool2d(2, 2)"""
+    return type(m).__name__ == '_Transition' and isinstance(m, nn.Sequential)
+
+
+def is_densenet_features(m):
+    """the `features` Sequential of a torchvision DenseNet (stem, dense blocks, transitions, norm5)"""
+    return isinstance(m, nn.Sequential) and any(is_dense_block(b) for b in m)
+
+
+class DenseBlockStep:
+    """torchvision _DenseBlock plus the pre-activation BatchNorm that reads its output (a transition's norm + relu, or norm5).
+
+    The block lives in ONE NHWC bf16 buffer (N, H, W, C_total): the step before it (the stem's max pool, a transition's
+    average pool) writes the block input into channels [0, C0), and layer l appends its `growth` channels at [Cin_l, Cin_l +
+    growth) straight from conv2's epilogue, so nothing is ever concatenated.  The batch statistics of a channel are the same
+    for every consumer (same data), so they are computed ONCE, when the channel is written, into one (2, C_total) f64 array;
+    each consumer's norm1 (and the tail BatchNorm) normalises its channel prefix from there with its own gamma / beta /
+    running statistics (jvae_bn_preact_fwd).  norm2 / relu2 are conv1's ConvStep epilogue as everywhere else.
+
+    Backward: an fp32 accumulator of the buffer's shape collects every consumer's data gradient (jvae_bn_preact_bwd adds
+    into its channel prefix).  Going through the layers in reverse, the slice of layer l is complete when layer l is reached
+    (only later layers and the tail read it), so it is cast to bf16 (jvae_cast_f32_bf16_ld) and fed to conv2 / conv1's
+    backward; channels [0, C0) at the end are the block input's gradient."""
+
+    def __init__(self, block, tail_bn, tail_act, in_shape):
+        C0, H, W = in_shape
+        if tail_bn is None:
+            raise NotImplementedError('a DenseNet block must be followed by a BatchNorm2d (transition norm or norm5)')
+        self.H, self.W, self.C0 = H, W, C0
+        self.layers = []
+        c = C0
+        for lay in block.values():
+            if getattr(lay, 'drop_rate', 0) > 0 or getattr(lay, 'memory_efficient', False):
+                raise NotImplementedError('DenseNet layers with drop_rate > 0 or memory_efficient=True have no native path')
+            if c % 8:
+                raise NotImplementedError(f'DenseNet channel offset {c} is not a multiple of 8: the block buffer needs '
+                                          '16-byte aligned channel slices (growth rate and initial features multiples of 8)')
+            n1, c1, n2, c2 = lay.norm1, lay.conv1, lay.norm2, lay.conv2
+            if n1.num_features != c or c1.in_channels != c or c1.kernel_size != (1, 1) or c1.stride != (1, 1):
+                raise NotImplementedError('_DenseLayer other than norm1 -> relu1 -> conv1x1 -> norm2 -> relu2 -> conv')
+            s1 = ConvStep(c1, n2, 1, (c, H, W), final_dense=False)
+            s2 = ConvStep(c2, None, 0, s1.out_shape, final_dense=False)
+            if s2.out_shape[1:] != (H, W):
+                raise NotImplementedError('DenseNet layer that changes the map size')
+            g = c2.out_channels
+            self.layers.append((n1, s1, s2, c, g))
+            c += g
+        if c % 8:
+            raise NotImplementedError(f'DenseNet block width {c} is not a multiple of 8')
+        if tail_bn.num_features != c:
+            raise NotImplementedError('BatchNorm2d after a dense block with a different channel count')
+        self.C = c
+        # conv2's epilogue writes whole 16-channel output tiles: with a growth rate that is not a multiple of 16, the last
+        # layer's zero-filled tile padding lands in 8 spare channels instead of the next pixel's first channels
+        self.ld = c + (8 if any(g % 16 for *_, g in self.layers) else 0)
+        self.tail_bn, self.tail_act = tail_bn, tail_act
+        self.out_shape = (c, H, W)
+        self.bns = [L[0] for L in self.layers] + [tail_bn] + [L[1].bn for L in self.layers]
+        self.untracked = any(not b.track_running_stats for b in self.bns)
+
+    def convs(self):
+        return [s for L in self.layers for s in L[1:3]]
+
+    def params(self):
+        ps = []
+        for n1, s1, s2, _, _ in self.layers:
+            ps += [n1.weight, n1.bias] + s1.params() + s2.params()
+        return ps + [self.tail_bn.weight, self.tail_bn.bias]
+
+    def new_buffer(self, N, like):
+        return K.empty((N, self.H, self.W, self.ld), like)
+
+    @staticmethod
+    def _pieces(C):
+        """channel ranges of at most BN_MAX_C channels (a thread of the BatchNorm kernels owns 8 channels of a 256-thread row):
+        densenet161's widest BatchNorms (2160, 2208 channels) run as two launches"""
+        n = -(-C // BN_MAX_C)
+        w = r8(-(-C // n))
+        return [(c0, min(C, c0 + w)) for c0 in range(0, C, w)]
+
+    def _bn_fwd(self, bn, buf, P, C, stats, bt, training, act, out, save):
+        track = bn.track_running_stats and training
+        sl = lambda t, a, b: None if t is None else t[a:b]
+        for i, (a, b) in enumerate(self._pieces(C)):
+            K.bn_preact_fwd(buf[..., a:], P, b - a, self.ld, sl(stats, a, None), self.C,
+                            sl(bn.weight.detach() if bn.affine else None, a, b), sl(bn.bias.detach() if bn.affine else None, a, b),
+                            bn.eps, bn.momentum if bn.momentum is not None else 0.1,
+                            sl(bn.running_mean if track or not bt else None, a, b),
+                            sl(bn.running_var if track or not bt else None, a, b),
+                            bn.num_batches_tracked if track and i == 0 else None, bt, act, out[..., a:], out.stride(2),
+                            None if save is None else save[i])
+        if track:
+            engine.bump_stats()      # the kernel wrote running_mean / running_var behind the version counters
+
+    def forward(self, x, st, training):
+        buf = st['buf']
+        assert x.data_ptr() == buf.data_ptr(), 'the block input must be written into the block buffer'
+        N, H, W = buf.shape[0], self.H, self.W
+        P = N * H * W
+        bt = training or self.untracked          # batch statistics (train mode, or BatchNorms without running statistics)
+        stats = pool = None
+        off = 2 * self.C
+        if bt:      # the block statistics (2, C_total) and every norm2's (2, 4 growth) from ONE zeroed allocation
+            pool = K.zeros((off + sum(2 * L[1].Co for L in self.layers),), buf, torch.float64)
+            stats = pool[:off]
+            K.bn_stats_ld(x, P, self.C0, self.ld, stats, self.C)
+        saved = []
+        for n1, s1, s2, c, g in self.layers:
+            h = K.empty((N, H, W, c), buf)
+            save = self._save(c, buf) if bt else None
+            self._bn_fwd(n1, buf, P, c, stats, bt, training, 1, h, save)
+            st1 = {}
+            if bt:
+                st1['stats_buf'] = pool[off:off + 2 * s1.Co].view(2, s1.Co)
+                off += 2 * s1.Co
+            a1 = s1.forward(h, st1, training)
+            st2 = {'out': buf[..., c:c + g]}
+            s2.forward(a1, st2, training)
+            if bt:      # the new channels' statistics, once, for every later consumer
+                K.bn_stats_ld(buf[..., c:], P, g, self.ld, stats[c:], self.C)
+            saved.append((h, save, st1, st2))
+        out = K.empty((N, H, W, self.C), buf)
+        tsave = self._save(self.C, buf) if bt else None
+        self._bn_fwd(self.tail_bn, buf, P, self.C, stats, bt, training, self.tail_act, out, tsave)
+        st.update(layers=saved, tail_save=tsave, bn_train=bt)
+        return out
+
+    def _save(self, C, like):
+        """the per-piece (2, width) mean / rstd of a train-mode pre-activation BatchNorm"""
+        return [K.empty((2, b - a), like, torch.float32) for a, b in self._pieces(C)]
+
+    def _bn_bwd(self, bn, da, buf, P, C, save, bt, act, G):
+        dg = db = lg = lb = None
+        if bt and bn.affine:
+            lg, lb = _live_grad(bn.weight, buf), _live_grad(bn.bias, buf)
+            dg = lg if lg is not None else K.zeros((C,), buf)
+            db = lb if lb is not None else K.zeros((C,), buf)
+        sl = lambda t, a, b: None if t is None else t[a:b]
+        for i, (a, b) in enumerate(self._pieces(C)):
+            sums = K.empty((2, b - a), buf, torch.float64) if bt else None
+            K.bn_preact_bwd(da[..., a:], da.stride(2), buf[..., a:], self.ld, P, b - a, None if save is None else save[i],
+                            sl(bn.weight.detach() if bn.affine else None, a, b), sl(bn.bias.detach() if bn.affine else None, a, b),
+                            None if bt else bn.running_mean[a:b], None if bt else bn.running_var[a:b], bn.eps, bt, act, sums,
+                            G[..., a:], self.ld, sl(dg, a, b), sl(db, a, b))
+        return [None if lg is not None else dg, None if lb is not None else db]
+
+    def backward(self, da, st, need_dx):
+        buf, bt = st['buf'], st['bn_train']
+        N, H, W = buf.shape[0], self.H, self.W
+        P = N * H * W
+        G = K.zeros((N, H, W, self.ld), buf, torch.float32)
+        tail = self._bn_bwd(self.tail_bn, da, buf, P, self.C, st['tail_save'], bt, self.tail_act, G)
+        grads = []
+        for (n1, s1, s2, c, g), (h, save, st1, st2) in zip(reversed(self.layers), reversed(st['layers'])):
+            d2 = K.empty((N, H, W, g), buf)
+            K.cast_f32_bf16_ld(G[..., c:], self.ld, d2, g, P, g)       # complete: only later layers and the tail read it
+            da1, pg2 = s2.backward(d2, st2, True)
+            dh, pg1 = s1.backward(da1, st1, True)
+            pgn = self._bn_bwd(n1, dh, buf, P, c, save, bt, 1, G)
+            grads = pgn + pg1 + pg2 + grads
+        dx = None
+        if need_dx:
+            dx = K.empty((N, H, W, self.C0), buf)
+            K.cast_f32_bf16_ld(G, self.ld, dx, self.C0, P, self.C0)
+        return dx, grads + tail
+
+
 class UpStep:
     """UpsamplingNearest2d(scale_factor=2)"""
 
@@ -938,6 +1128,11 @@ class ConvStack:
         for m in mods:          # torchvision's layer1..4 are Sequentials of residual blocks
             if isinstance(m, nn.Sequential) and all(is_residual_block(b) for b in m):
                 flat += list(m)
+            elif is_densenet_features(m):        # DenseNet: stem, blocks, transitions (norm, relu, conv, pool), norm5
+                for b in m:
+                    flat += list(b) if is_transition(b) else [b]
+            elif is_transition(m):
+                flat += list(m)
             else:
                 flat.append(m)
         mods = flat
@@ -969,6 +1164,14 @@ class ConvStack:
             elif is_residual_block(m):
                 groups.append(('res', m))
                 i += 1
+            elif is_dense_block(m):      # + the BatchNorm (+ ReLU) that reads the block's output
+                bn, act, j = None, 0, i + 1
+                if j < n and isinstance(mods[j], nn.BatchNorm2d):
+                    bn, j = mods[j], j + 1
+                    if j < n and type(mods[j]) in (nn.ReLU, nn.Identity):
+                        act, j = _ACT_CODE[type(mods[j])], j + 1
+                groups.append(('dense', m, bn, act))
+                i = j
             elif isinstance(m, nn.UpsamplingNearest2d):
                 groups.append(('up', m))
                 i += 1
@@ -986,6 +1189,11 @@ class ConvStack:
                 stp = AvgStep(g[1], shape)
             elif g[0] == 'res':
                 stp = ResidualStep(g[1], shape)
+            elif g[0] == 'dense':
+                if not (steps and isinstance(steps[-1], (PoolStep, AvgStep))) or shape[0] % 8:
+                    raise NotImplementedError('a DenseNet block must follow a pooling layer with a multiple of 8 channels '
+                                              '(the pooling writes the block input into the block buffer)')
+                stp = DenseBlockStep(g[1], g[2], g[3], shape)
             else:
                 stp = UpStep(g[1], shape)
             steps.append(stp)
@@ -999,6 +1207,8 @@ class ConvStack:
                 convs.append(stp)
             elif isinstance(stp, ResidualStep):
                 convs += stp.chain + ([stp.ds] if stp.ds is not None else [])
+            elif isinstance(stp, DenseBlockStep):
+                convs += stp.convs()
         self.plan = PackPlan(convs)
         for c in convs:
             c.plan = self.plan
@@ -1018,11 +1228,17 @@ class ConvStack:
         pool, off = None, 0
         if bn_steps:
             pool = K.zeros((sum(2 * s.Co for s in bn_steps),), t, torch.float64)
-        for s in self.steps:
-            st = {}
+        pending = None
+        for i, s in enumerate(self.steps):
+            st, pending = pending or {}, None
             if pool is not None and any(s is b for b in bn_steps):
                 st['stats_buf'] = pool[off:off + 2 * s.Co].view(2, s.Co)
                 off += 2 * s.Co
+            nxt = self.steps[i + 1] if i + 1 < len(self.steps) else None
+            if isinstance(nxt, DenseBlockStep):      # this step writes the block input into the block's buffer
+                buf = nxt.new_buffer(N, t)
+                st['out'] = buf[..., :nxt.C0]
+                pending = {'buf': buf}
             t = s.forward(t, st, training)
             state.append(st)
         Co, Ho, Wo = self.out_shape

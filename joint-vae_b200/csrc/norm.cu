@@ -85,8 +85,10 @@ __device__ __forceinline__ float act_grad_z(float z, int act) {
 // so the statistics (and everything downstream) are reproducible run to run.
 // When the chunk count divides the warp (power of two <= 16) the lanes that own the same chunk are folded with
 // shuffles first, so shared memory sees one atomic per chunk and warp instead of 32 / nchunk conflicting ones.
+// gld: row stride of gout (0 = C, dense (NK, C)); a wider array takes the statistics of a channel slice of a dense block
 template <int V, int NK>
-__device__ __forceinline__ void block_channel_reduce(float (&acc)[NK][V], int chunk, int C, double* s_acc, double* gout) {
+__device__ __forceinline__ void block_channel_reduce(float (&acc)[NK][V], int chunk, int C, double* s_acc, double* gout,
+                                                     int gld = 0) {
   for (int i = threadIdx.x; i < NK * C; i += blockDim.x) s_acc[i] = 0.0;
   __syncthreads();
   const int nchunk = C / V;
@@ -108,7 +110,11 @@ __device__ __forceinline__ void block_channel_reduce(float (&acc)[NK][V], int ch
       for (int j = 0; j < V; ++j) atomicAdd(&s_acc[k * C + chunk * V + j], (double)acc[k][j]);
   }
   __syncthreads();
-  for (int i = threadIdx.x; i < NK * C; i += blockDim.x) atomicAdd(&gout[i], s_acc[i]);
+  if (gld == 0 || gld == C) {
+    for (int i = threadIdx.x; i < NK * C; i += blockDim.x) atomicAdd(&gout[i], s_acc[i]);
+  } else {
+    for (int i = threadIdx.x; i < NK * C; i += blockDim.x) atomicAdd(&gout[(i / C) * gld + i % C], s_acc[i]);
+  }
 }
 
 // same, for a float destination (bias gradients accumulate straight into the fp32 .grad buffer)
@@ -127,7 +133,7 @@ __device__ __forceinline__ void block_channel_reduce_f32(float (&acc)[NK][V], in
 // ------------------------------------------------------------------------------------------------ statistics
 template <int V>
 __global__ void __launch_bounds__(NORM_MAX_THREADS) bn_stats_kernel(const __nv_bfloat16* __restrict__ y, size_t P, int C, int ld,
-                                                                    int nchunk, int ppb, double* stats) {
+                                                                    int nchunk, int ppb, double* stats, int sld) {
   extern __shared__ double s_acc[];
   const int chunk = threadIdx.x % nchunk, pl = threadIdx.x / nchunk;
   float acc[2][V];
@@ -152,13 +158,14 @@ __global__ void __launch_bounds__(NORM_MAX_THREADS) bn_stats_kernel(const __nv_b
 #pragma unroll
       for (int j = 0; j < V; ++j) { acc[0][j] += v[u][j]; acc[1][j] += v[u][j] * v[u][j]; }
   }
-  block_channel_reduce<V, 2>(acc, chunk, C, s_acc, stats);
+  block_channel_reduce<V, 2>(acc, chunk, C, s_acc, stats, sld);
 }
 
 // ------------------------------------------------------------------------------------------------ BN forward
 struct BnFwd {
   const __nv_bfloat16* y; __nv_bfloat16* out;
   size_t P; int C, ld_y, ld_out, nchunk, ppb, act, training;
+  int sld;                // row stride of stats: sums at stats[c], sums of squares at stats[sld + c]
   const double* stats; const float* gamma; const float* beta;
   float* running_mean; float* running_var; long long* num_batches; float* save;
   float eps, momentum;
@@ -176,7 +183,7 @@ __global__ void __launch_bounds__(NORM_MAX_THREADS) bn_apply_fwd_kernel(const Bn
       const double inv = 1.0 / (double)a.P;
       const double mean_d = a.stats[c] * inv;
       mean = (float)mean_d;
-      const float var = fmaxf((float)(a.stats[a.C + c] * inv - mean_d * mean_d), 0.f);
+      const float var = fmaxf((float)(a.stats[a.sld + c] * inv - mean_d * mean_d), 0.f);
       rstd = rsqrtf(var + a.eps);
       if (blockIdx.x == 0 && pl == 0) {
         a.save[c] = mean; a.save[a.C + c] = rstd;
@@ -225,7 +232,26 @@ struct BnBwd {
   const float* save; const float* gamma; const float* beta;
   double* sums;           // (2, C): sum g, sum g * xhat   (zeroed by the caller before the reduce kernel)
   float* dgamma; float* dbeta;
+  // pre-activation BatchNorm of a dense block (jvae_bn_preact_bwd): dxf (fp32, row stride ld_dxf) += the data gradient
+  // instead of storing bf16 dy; eval != 0: running statistics, the gradient is the per-channel scale only (no reduction)
+  float* dxf; int ld_dxf, eval;
+  const float* rmean; const float* rvar; float eps;
 };
+
+// dst[0..V) += v (fp32 accumulator of a dense block's channel gradients)
+template <int V>
+__device__ __forceinline__ void acc_f32(float* dst, const float (&v)[V]) {
+  if constexpr (V == 8) {
+    float4* d = reinterpret_cast<float4*>(dst);
+    float4 x0 = d[0], x1 = d[1];
+    x0.x += v[0]; x0.y += v[1]; x0.z += v[2]; x0.w += v[3];
+    x1.x += v[4]; x1.y += v[5]; x1.z += v[6]; x1.w += v[7];
+    d[0] = x0; d[1] = x1;
+  } else {
+#pragma unroll
+    for (int j = 0; j < V; ++j) dst[j] += v[j];
+  }
+}
 
 template <int V>
 __global__ void __launch_bounds__(NORM_MAX_THREADS, BN_REDUCE_BLOCKS) bn_bwd_reduce_kernel(const BnBwd a) {
@@ -286,13 +312,21 @@ __global__ void __launch_bounds__(NORM_MAX_THREADS) bn_bwd_apply_kernel(const Bn
 #pragma unroll
   for (int j = 0; j < V; ++j) {
     const int c = chunk * V + j;
-    mean[j] = a.save[c]; rstd[j] = a.save[a.C + c];
+    if (a.eval) {
+      mean[j] = a.rmean[c]; rstd[j] = rsqrtf(a.rvar[c] + a.eps);
+    } else {
+      mean[j] = a.save[c]; rstd[j] = a.save[a.C + c];
+    }
     const float g = a.gamma ? a.gamma[c] : 1.f, b = a.beta ? a.beta[c] : 0.f;
     scale[j] = g * rstd[j]; shift[j] = b - mean[j] * scale[j];
-    k1[j] = (float)(a.sums[c] * (double)inv); k2[j] = (float)(a.sums[a.C + c] * (double)inv);
-    if (blockIdx.x == 0 && pl == 0) {
-      if (a.dbeta) a.dbeta[c] += (float)a.sums[c];   // accumulated: the caller passes a zeroed buffer or the live .grad
-      if (a.dgamma) a.dgamma[c] += (float)a.sums[a.C + c];
+    if (a.eval) {
+      k1[j] = k2[j] = 0.f;
+    } else {
+      k1[j] = (float)(a.sums[c] * (double)inv); k2[j] = (float)(a.sums[a.C + c] * (double)inv);
+      if (blockIdx.x == 0 && pl == 0) {
+        if (a.dbeta) a.dbeta[c] += (float)a.sums[c];   // accumulated: the caller passes a zeroed buffer or the live .grad
+        if (a.dgamma) a.dgamma[c] += (float)a.sums[a.C + c];
+      }
     }
   }
   constexpr int U = 2;        // rows per thread and round, the 2 U loads requested together
@@ -322,7 +356,8 @@ __global__ void __launch_bounds__(NORM_MAX_THREADS) bn_bwd_apply_kernel(const Bn
         const float xh = (y[j] - mean[j]) * rstd[j];
         g[j] = scale[j] * (gz - k1[j] - xh * k2[j]);
       }
-      Vec<V>::store(a.dy + p * a.ld_dy + chunk * V, g);
+      if (a.dxf) acc_f32<V>(a.dxf + p * a.ld_dxf + chunk * V, g);
+      else Vec<V>::store(a.dy + p * a.ld_dy + chunk * V, g);
     }
   }
 }
@@ -379,7 +414,7 @@ __global__ void __launch_bounds__(NORM_MAX_THREADS) bn_apply_fwd_narrow_kernel(c
       const double inv = 1.0 / (double)a.P;
       const double mean_d = a.stats[c] * inv;
       mean = (float)mean_d;
-      const float var = fmaxf((float)(a.stats[a.C + c] * inv - mean_d * mean_d), 0.f);
+      const float var = fmaxf((float)(a.stats[a.sld + c] * inv - mean_d * mean_d), 0.f);
       rstd = rsqrtf(var + a.eps);
       if (blockIdx.x == 0 && threadIdx.x == 0) {
         a.save[c] = mean; a.save[a.C + c] = rstd;
@@ -988,6 +1023,29 @@ __global__ void __launch_bounds__(256) vstack_rows_kernel(const __nv_bfloat16* _
   }
 }
 
+// ------------------------------------------------------------------------------------------------ fp32 -> bf16 channel slice
+// dst (P, C) bf16 = src (P, C) fp32, both with their own leading dimension: a completed slice of a dense block's gradient
+// accumulator becomes the bf16 operand of the convolutions' backward
+template <int V>
+__global__ void __launch_bounds__(NORM_MAX_THREADS) cast_slice_kernel(const float* __restrict__ src, int ld_src,
+                                                                      __nv_bfloat16* __restrict__ dst, int ld_dst, size_t P,
+                                                                      int nchunk, int ppb) {
+  const int chunk = threadIdx.x % nchunk, pl = threadIdx.x / nchunk;
+  const size_t step = (size_t)gridDim.x * ppb;
+  for (size_t p = (size_t)blockIdx.x * ppb + pl; p < P; p += step) {
+    float v[V];
+    const float* s = src + p * ld_src + chunk * V;
+    if constexpr (V == 8) {
+      const float4 x0 = reinterpret_cast<const float4*>(s)[0], x1 = reinterpret_cast<const float4*>(s)[1];
+      v[0] = x0.x; v[1] = x0.y; v[2] = x0.z; v[3] = x0.w; v[4] = x1.x; v[5] = x1.y; v[6] = x1.z; v[7] = x1.w;
+    } else {
+#pragma unroll
+      for (int j = 0; j < V; ++j) v[j] = s[j];
+    }
+    Vec<V>::store(dst + p * ld_dst + chunk * V, v);
+  }
+}
+
 static bool vec_ok(int C, std::initializer_list<int> lds, std::initializer_list<const void*> ptrs) {
   if (C % 8) return false;
   for (int l : lds) if (l % 8) return false;
@@ -1037,7 +1095,17 @@ int jvae_bn_stats(const void* y, size_t P, int C, int ld, double* stats, void* s
   JVAE_CHECK_ARG(vec ? C <= 8 * NORM_MAX_THREADS : C <= NORM_MAX_THREADS, "too many channels for this layout");
   const Geo g = make_geo(P, C, vec ? 8 : 1);
   NORM_DISPATCH(vec, bn_stats_kernel, g, 2 * C * sizeof(double), (cudaStream_t)stream,
-                reinterpret_cast<const __nv_bfloat16*>(y), P, C, ld, g.nchunk, g.ppb, stats);
+                reinterpret_cast<const __nv_bfloat16*>(y), P, C, ld, g.nchunk, g.ppb, stats, C);
+  return JVAE_OK;
+}
+
+int jvae_bn_stats_ld(const void* y, size_t P, int C, int ld, double* stats, int stats_ld, void* stream) {
+  JVAE_CHECK_ARG(y && stats && P > 0 && C > 0 && ld >= C && stats_ld >= C, "bad arguments");
+  const bool vec = vec_ok(C, {ld}, {y});
+  JVAE_CHECK_ARG(vec ? C <= 8 * NORM_MAX_THREADS : C <= NORM_MAX_THREADS, "too many channels for this layout");
+  const Geo g = make_geo(P, C, vec ? 8 : 1);
+  NORM_DISPATCH(vec, bn_stats_kernel, g, 2 * C * sizeof(double), (cudaStream_t)stream,
+                reinterpret_cast<const __nv_bfloat16*>(y), P, C, ld, g.nchunk, g.ppb, stats, stats_ld);
   return JVAE_OK;
 }
 
@@ -1056,7 +1124,7 @@ int jvae_bn_apply_fwd(const void* y, size_t P, int C, int ld_y, const double* st
   BnFwd a;
   a.y = reinterpret_cast<const __nv_bfloat16*>(y); a.out = reinterpret_cast<__nv_bfloat16*>(out);
   a.P = P; a.C = C; a.ld_y = ld_y; a.ld_out = ld_out; a.nchunk = g.nchunk; a.ppb = g.ppb; a.act = act; a.training = training;
-  a.stats = stats; a.gamma = gamma; a.beta = beta; a.running_mean = running_mean; a.running_var = running_var;
+  a.sld = C; a.stats = stats; a.gamma = gamma; a.beta = beta; a.running_mean = running_mean; a.running_var = running_var;
   a.num_batches = reinterpret_cast<long long*>(num_batches); a.save = save_mean_rstd; a.eps = eps; a.momentum = momentum;
   if (narrow) {      // a thread per pixel (the image head's BatchNorm)
     const int want = (int)((P + NORM_MAX_THREADS * 4 - 1) / (NORM_MAX_THREADS * 4));
@@ -1077,7 +1145,7 @@ int jvae_bn_bwd(const void* da, int ld_da, const void* y, int ld_y, size_t P, in
   const bool vec = vec_ok(C, {ld_da, ld_y, ld_dy}, {da, y, dy});
   JVAE_CHECK_ARG(vec ? C <= 8 * NORM_MAX_THREADS : C <= NORM_MAX_THREADS, "too many channels for this layout");
   const Geo g = make_geo(P, C, vec ? 8 : 1);
-  BnBwd a;
+  BnBwd a = {};
   a.da = reinterpret_cast<const __nv_bfloat16*>(da); a.y = reinterpret_cast<const __nv_bfloat16*>(y);
   a.dy = reinterpret_cast<__nv_bfloat16*>(dy);
   a.P = P; a.C = C; a.ld_da = ld_da; a.ld_y = ld_y; a.ld_dy = ld_dy; a.nchunk = g.nchunk; a.ppb = g.ppb; a.act = act;
@@ -1105,6 +1173,55 @@ int jvae_bn_bwd(const void* da, int ld_da, const void* y, int ld_y, size_t P, in
     NORM_DISPATCH(vec, bn_bwd_reduce_kernel, gr, 2 * C * sizeof(double), (cudaStream_t)stream, a);
   }
   NORM_DISPATCH(vec, bn_bwd_apply_kernel, g, 0, (cudaStream_t)stream, a);
+  return JVAE_OK;
+}
+
+int jvae_bn_preact_fwd(const void* y, size_t P, int C, int ld_y, const double* stats, int stats_ld, const float* gamma,
+                       const float* beta, float eps, float momentum, float* running_mean, float* running_var,
+                       int64_t* num_batches, int training, int act, void* out, int ld_out, float* save_mean_rstd, void* stream) {
+  JVAE_CHECK_ARG(y && out && P > 0 && C > 0 && ld_y >= C && ld_out >= C, "bad arguments");
+  JVAE_CHECK_ARG(training ? (stats && save_mean_rstd && stats_ld >= C) : (running_mean && running_var), "statistics missing");
+  JVAE_CHECK_ARG(vec_ok(C, {ld_y, ld_out}, {y, out}) && C <= 8 * NORM_MAX_THREADS,
+                 "pre-activation BatchNorm needs C, ld_y, ld_out multiples of 8 and 16-byte aligned rows");
+  const Geo g = make_geo(P, C, 8);
+  BnFwd a;
+  a.y = reinterpret_cast<const __nv_bfloat16*>(y); a.out = reinterpret_cast<__nv_bfloat16*>(out);
+  a.P = P; a.C = C; a.ld_y = ld_y; a.ld_out = ld_out; a.nchunk = g.nchunk; a.ppb = g.ppb; a.act = act; a.training = training;
+  a.sld = stats_ld; a.stats = stats; a.gamma = gamma; a.beta = beta; a.running_mean = running_mean; a.running_var = running_var;
+  a.num_batches = reinterpret_cast<long long*>(num_batches); a.save = save_mean_rstd; a.eps = eps; a.momentum = momentum;
+  NORM_DISPATCH(true, bn_apply_fwd_kernel, g, 0, (cudaStream_t)stream, a);
+  return JVAE_OK;
+}
+
+int jvae_bn_preact_bwd(const void* da, int ld_da, const void* y, int ld_y, size_t P, int C, const float* save_mean_rstd,
+                       const float* gamma, const float* beta, const float* running_mean, const float* running_var, float eps,
+                       int training, int act, double* sums, float* dx, int ld_dx, float* dgamma, float* dbeta, void* stream) {
+  JVAE_CHECK_ARG(da && y && dx && P > 0 && C > 0 && ld_da >= C && ld_y >= C && ld_dx >= C, "bad arguments");
+  JVAE_CHECK_ARG(training ? (sums && save_mean_rstd) : (running_mean && running_var), "statistics missing");
+  JVAE_CHECK_ARG(vec_ok(C, {ld_da, ld_y, ld_dx}, {da, y, dx}) && C <= 8 * NORM_MAX_THREADS,
+                 "pre-activation BatchNorm needs C and every ld multiples of 8 and 16-byte aligned rows");
+  const Geo g = make_geo(P, C, 8);
+  BnBwd a = {};
+  a.da = reinterpret_cast<const __nv_bfloat16*>(da); a.y = reinterpret_cast<const __nv_bfloat16*>(y);
+  a.P = P; a.C = C; a.ld_da = ld_da; a.ld_y = ld_y; a.nchunk = g.nchunk; a.ppb = g.ppb; a.act = act;
+  a.save = save_mean_rstd; a.gamma = gamma; a.beta = beta; a.sums = sums; a.dgamma = dgamma; a.dbeta = dbeta;
+  a.dxf = dx; a.ld_dxf = ld_dx; a.eval = !training; a.rmean = running_mean; a.rvar = running_var; a.eps = eps;
+  if (training) {
+    JVAE_CUDA(cudaMemsetAsync(sums, 0, 2 * (size_t)C * sizeof(double), (cudaStream_t)stream));
+    const Geo gr = make_geo(P, C, 8, BN_REDUCE_BLOCKS);
+    NORM_DISPATCH(true, bn_bwd_reduce_kernel, gr, 2 * C * sizeof(double), (cudaStream_t)stream, a);
+  }
+  NORM_DISPATCH(true, bn_bwd_apply_kernel, g, 0, (cudaStream_t)stream, a);
+  return JVAE_OK;
+}
+
+int jvae_cast_f32_bf16_ld(const float* src, int ld_src, void* dst, int ld_dst, size_t P, int C, void* stream) {
+  JVAE_CHECK_ARG(src && dst && P > 0 && C > 0 && ld_src >= C && ld_dst >= C, "bad arguments");
+  const bool vec = vec_ok(C, {ld_src, ld_dst}, {src, dst});
+  JVAE_CHECK_ARG(vec ? C <= 8 * NORM_MAX_THREADS : C <= NORM_MAX_THREADS, "too many channels for this layout");
+  const Geo g = make_geo(P, C, vec ? 8 : 1);
+  NORM_DISPATCH(vec, cast_slice_kernel, g, 0, (cudaStream_t)stream, src, ld_src, reinterpret_cast<__nv_bfloat16*>(dst), ld_dst,
+                P, g.nchunk, g.ppb);
   return JVAE_OK;
 }
 

@@ -139,10 +139,11 @@ _CONV_TYPES = (nn.Conv2d, nn.ConvTranspose2d, nn.BatchNorm2d, nn.MaxPool2d, nn.A
 
 
 def _is_conv_type(m):
-    """layers the native conv engine executes, including torchvision's residual blocks and Sequentials of them"""
-    from .conv_engine import is_residual_block
+    """layers the native conv engine executes, including torchvision's residual blocks and Sequentials of them, and the
+    `features` Sequential of torchvision's DenseNets (stem, dense blocks, transitions, norm5)"""
+    from .conv_engine import is_residual_block, is_densenet_features
     return isinstance(m, _CONV_TYPES) or is_residual_block(m) or \
-        (isinstance(m, nn.Sequential) and len(m) > 0 and all(is_residual_block(b) for b in m))
+        (isinstance(m, nn.Sequential) and len(m) > 0 and all(is_residual_block(b) for b in m)) or is_densenet_features(m)
 
 
 def run_sequential(seq, x, out_dtype=None, image_out=False):
@@ -189,7 +190,8 @@ def run_sequential(seq, x, out_dtype=None, image_out=False):
 
 def run_conv_stack(mods, x, image_out=False):
     """x NCHW through the tcgen05 implicit-GEMM kernels of csrc/conv.cu + csrc/norm.cu (conv_engine).  A layer type
-    without a native kernel (DenseNet blocks, MaxPool2d with ceil_mode, ...) raises NotImplementedError."""
+    without a native kernel (MaxPool2d with ceil_mode, DenseNets with dropout or channel offsets that are not multiples of
+    8, ...) raises NotImplementedError."""
     from . import conv_engine
     return conv_engine.run(mods, x, image_out=image_out)
 

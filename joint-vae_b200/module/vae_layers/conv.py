@@ -106,7 +106,7 @@ def build_de_conv_layers(input_shape, layers_name, batch_norm=False, where='inpu
                          output_activation='linear', output_distribution='gaussian', pretrained_dict=None):
     """conv.py:128-244: features (where='input') or upsampler (where='output') as an nn.Sequential with
     .name, .input_shape, .output_shape, .shapes."""
-    if where == 'input' and layers_name.startswith('resnet'):
+    if where == 'input' and layers_name.startswith(('resnet', 'densenet')):
         return ResOrDenseNetFeatures(model_name=layers_name, input_shape=input_shape)
     table = features_dict if where == 'input' else upsampler_dict
     name = layers_name if layers_name in table else None
