@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define JVAE_ABI_VERSION 16
+#define JVAE_ABI_VERSION 17
 
 enum jvae_status {
   JVAE_OK = 0,
@@ -185,12 +185,6 @@ int jvae_sample_bwd(int B, int L, int K, const float* head, const float* log_var
  * ------------------------------------------------------------------------------------------ */
 enum jvae_act { JVAE_ACT_NONE = 0, JVAE_ACT_RELU = 1, JVAE_ACT_SIGMOID = 2, JVAE_ACT_LEAKY = 3 };   /* leaky: slope 0.01 (nn.LeakyReLU default, misc.py:27) */
 #define JVAE_LEAKY_SLOPE 0.01f
-/* flags OR-ed into the `act` argument of the convolution / row kernels:
- *   JVAE_OUT_F32 (jvae_conv_gather_gemm): `out` holds fp32 and ld_out counts floats (no activation rounding at all: the 1 x k
- *   stage of the separable image head, whose vertical taps cancel -- rounding them to bf16 costs the head's gradients 10 x);
- *   JVAE_IN_F32 (jvae_vsum_rows): T holds fp32 */
-#define JVAE_OUT_F32 0x100
-#define JVAE_IN_F32 0x200
 enum jvae_gemm_mode {
   JVAE_GEMM_NT = 0,  /* D[M,N] = A[M,K] . B[N,K]^T   forward:  y = x W^T                       */
   JVAE_GEMM_NN = 1,  /* D[M,N] = A[M,K] . B[K,N]     dgrad:    dx = dy W                        */
@@ -231,23 +225,6 @@ int jvae_conv_gather_gemm(const void* in, int N, int H, int W, int Cin, int ld_i
                           int ntaps, const int16_t* tap_dy, const int16_t* tap_dx, int in_stride, int Hq, int Wq,
                           void* out, int Ho, int Wo, int Cout, int ld_out, int out_sy, int out_sx, int out_oy, int out_ox,
                           const float* bias, int act, double* stats, void* stream);
-/* Data-gradient launches can fold the reduction pass of the PREVIOUS layer's BatchNorm backward into their epilogue: the
- * output of the launch is dL/da of that layer (a = act(BN(y))), `bn` describes its BatchNorm, and `stats` (2,Cout)
- * receives += sum g*act'(z) and sum g*act'(z)*xhat (what jvae_bn_bwd's first kernel computes; zero it first).
- * *bn_fused (host int) is set to 1 when the kernel variant used supports the fusion, else 0: then call jvae_bn_bwd with
- * skip_reduce = 0 as usual. */
-typedef struct jvae_bn_reduce {
-  const void* y;                /* previous layer's pre-BN output (P,C) bf16 at the pixels this launch writes */
-  int32_t ld_y;
-  const float* save_mean_rstd;  /* (2,C) from jvae_bn_apply_fwd */
-  const float* gamma;           /* (C) or NULL */
-  const float* beta;            /* (C) or NULL */
-  int32_t act;                  /* jvae_act of that layer */
-} jvae_bn_reduce;
-int jvae_conv_gather_gemm_bn(const void* in, int N, int H, int W, int Cin, int ld_in, const void* wmat, int Cout_pad, int ldw,
-                             int ntaps, const int16_t* tap_dy, const int16_t* tap_dx, int in_stride, int Hq, int Wq,
-                             void* out, int Ho, int Wo, int Cout, int ld_out, int out_sy, int out_sx, int out_oy, int out_ox,
-                             const float* bias, int act, double* stats, const jvae_bn_reduce* bn, int* bn_fused, void* stream);
 /* ALL sub-pixel phases of a stride-`out_s` ConvTranspose2d (conv.py:189-219, the imager stacks of conv-models.ini:25) or of
  * the data gradient of a strided Conv2d in ONE launch: phase i owns phase_ntaps[i] consecutive entries of the tap table (and
  * of wmat's [tap] blocks, same row layout as jvae_conv_gather_gemm) and writes
@@ -255,7 +232,7 @@ int jvae_conv_gather_gemm_bn(const void* in, int N, int H, int W, int Cin, int l
  * for every q of the (N, Hq, Wq) grid all phases share (even output sizes).  The input box is read once for all phases and
  * the taps of different phases that read the same input shift are one MMA (their weights stacked along N).
  * Returns JVAE_NOT_COVERED (nothing launched, no error text) when the geometry is outside what the merged kernel handles
- * (wide layers, weights that do not fit in shared memory, JVAE_CONV_MERGE_PHASES=0): the caller then issues one
+ * (wide layers, weights that do not fit in shared memory): the caller then issues one
  * jvae_conv_gather_gemm per phase, which computes the same thing. */
 #define JVAE_NOT_COVERED 1
 int jvae_conv_subpixel_gemm(const void* in, int N, int H, int W, int Cin, int ld_in, const void* wmat, int Cout_pad, int ldw,
@@ -282,7 +259,7 @@ int jvae_conv_wgrad_emulate(const float* dy, int N, int Hq, int Wq, int Cout, in
 int jvae_conv_wgrad(const void* dy, int N, int Hq, int Wq, int Cout, int ld_dy, const void* x, int H, int W, int Cin, int ld_x,
                     int ntaps, const int16_t* tap_dy, const int16_t* tap_dx, int in_stride, float* dw, int dw_ld_tap,
                     int dw_ld_co, int dw_ld_ci, void* stream);
-/* which kernel the calling thread's last jvae_conv_gather_gemm[_bn] / jvae_conv_wgrad call launched (measurement aid:
+/* which kernel the calling thread's last jvae_conv_gather_gemm / jvae_conv_wgrad call launched (measurement aid:
  * bench.py attributes per-launch CUDA-event times to the dominant kernel of the step) */
 enum jvae_conv_kernel { JVAE_KERNEL_CONV_HALO = 1, JVAE_KERNEL_CONV_TAPBOX = 2, JVAE_KERNEL_WGRAD_HALO = 3, JVAE_KERNEL_WGRAD_TAPBOX = 4 };
 int jvae_last_conv_kernel(void);
@@ -301,10 +278,10 @@ int jvae_bn_apply_fwd(const void* y, size_t P, int C, int ld_y, const double* st
                       float eps, float momentum, float* running_mean, float* running_var, int64_t* num_batches, int training,
                       int act, void* out, int ld_out, float* save_mean_rstd, void* stream);
 /* backward of act(BN_train(y)) given da = dL/d(out): dy (P,C) bf16, dgamma, dbeta (C) f32 (+=, any may be NULL);
- * sums (2,C) f64 scratch; skip_reduce != 0: sums were already produced by jvae_conv_gather_gemm_bn */
+ * sums (2,C) f64 scratch */
 int jvae_bn_bwd(const void* da, int ld_da, const void* y, int ld_y, size_t P, int C, const float* save_mean_rstd,
                 const float* gamma, const float* beta, int act, double* sums, void* dy, int ld_dy, float* dgamma, float* dbeta,
-                int skip_reduce, void* stream);
+                void* stream);
 /* DenseNet blocks (torchvision _DenseBlock): every layer appends its channels to ONE (P, C_total) bf16 buffer, whose batch
  * statistics live in ONE (2, C_total) f64 array (row stride stats_ld = C_total) written once per channel and read by every
  * later pre-activation BatchNorm; the backward accumulates the channel gradients of all consumers in ONE fp32 buffer.
@@ -348,16 +325,11 @@ int jvae_maxpool_pad_bwd(const void* in, int N, int H, int W, int C, int ld_in, 
  * src (N,H/k,W/k,C) / k^2 spread over the windows */
 int jvae_avgpool(const void* src, int ld_src, void* dst, int ld_dst, int N, int H, int W, int C, int k, int backward,
                  void* stream);
-/* Separable form of a k x k stride-1 'same' convolution with few output channels (k * Co <= 16, Co <= 4: the image head 32 -> 3 of
- * the deconv presets, conv-models.ini:25): the tensor-core kernels run the 1 x k convolution to k * Co channels,
- * T[r][ty*Co + co] = sum_tx sum_ci x[r + (0, tx - pad)][ci] W[co][ci][ty][tx], and
- *   jvae_vsum_rows:   out[q][co] = act(bias[co] + sum_ty T[q + (ty - pad, 0)][ty*Co + co]); stats (2, Co) f64 (optional) +=
- *                     sum / sum of squares of the pre-activation (BatchNorm2d batch statistics);
- *   jvae_vstack_rows: U[r][ty*Co + co] = dy[r - (ty - pad, 0)][co], the gradient of T (zero outside the image, zero padding
- *                     channels up to ld_u): the 1 x k kernel's data / weight gradients then run on U.
- * k taps instead of k^2 in the three tensor-core passes. */
-int jvae_vsum_rows(const void* T, int ld_t, int N, int H, int W, int k, int pad, int Co, const float* bias, int act, double* stats,
-                   void* out, int ld_out, void* stream);
+/* Backward of a k x k stride-1 'same' convolution with few output channels (k * Co <= 16, Co <= 4: the image head 32 -> 3 of
+ * the deconv presets, conv-models.ini:25) in separable form: the gradient of the 1 x k convolution to k * Co channels,
+ * T[r][ty*Co + co] = sum_tx sum_ci x[r + (0, tx - pad)][ci] W[co][ci][ty][tx], whose vertical sum is the layer's output, is
+ *   jvae_vstack_rows: U[r][ty*Co + co] = dy[r - (ty - pad, 0)][co] (zero outside the image, zero padding channels up to ld_u):
+ *                     the 1 x k kernel's data / weight gradients then run on U, k taps instead of k^2. */
 int jvae_vstack_rows(const void* dy, int ld_dy, int N, int H, int W, int k, int pad, int Co, void* U, int ld_u, void* stream);
 /* out = act(a + b) over P pixels x C channels: the join of a residual block (out += identity; relu); act = NONE adds two
  * gradient branches */

@@ -16,7 +16,6 @@ F32, BF16 = 0, 1
 VAR_DIM = {'scalar': 0, 'diag': 1, 'full': 2}
 PRIOR_KIND = {'gaussian': 0, 'tilted': 1, 'uniform': 2}
 ACT = {'none': 0, 'linear': 0, 'relu': 1, 'sigmoid': 2, 'leaky': 3}
-OUT_F32, IN_F32 = 0x100, 0x200      # include/jvae_b200.h: JVAE_OUT_F32 / JVAE_IN_F32 flags of the `act` argument
 LEAKY_SLOPE = 0.01      # JVAE_LEAKY_SLOPE: nn.LeakyReLU() default, the only slope the reference builds (misc.py:27)
 NSCORES, NPRED = 16, 4
 SCORE_INDEX = {'elbo': 0, 'max': 0, 'sum': 1, 'mean': 2, 'iws': 3, 'soft': 4, 'softkl': 4, 'zdist': 5, 'kl': 6,
@@ -33,12 +32,6 @@ class ElboCfg(ctypes.Structure):
                  'has_xreco', 'has_logits', 'sigma_is_log', 'sigma_is_rmse')] + \
                [(n, ctypes.c_float) for n in ('beta', 'gamma_w', 'var_w', 'tau', 'alpha')] + \
                [(n, ctypes.c_int32) for n in ('prior_stats_ready', 'categorical', 'cat_group', 'sigma_per_sample')]
-
-
-class BnReduce(ctypes.Structure):
-    """include/jvae_b200.h: jvae_bn_reduce"""
-    _fields_ = [('y', ctypes.c_void_p), ('ld_y', ctypes.c_int32), ('save_mean_rstd', ctypes.c_void_p),
-                ('gamma', ctypes.c_void_p), ('beta', ctypes.c_void_p), ('act', ctypes.c_int32)]
 
 
 class BatchCfg(ctypes.Structure):          # include/jvae_b200.h: jvae_batch_cfg
@@ -102,9 +95,6 @@ def lib():
     L.jvae_conv_gather_gemm.argtypes = [P, c_int, c_int, c_int, c_int, c_int, P, c_int, c_int, c_int, I16P, I16P, c_int,
                                         c_int, c_int, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P, c_int,
                                         P, P]
-    L.jvae_conv_gather_gemm_bn.argtypes = [P, c_int, c_int, c_int, c_int, c_int, P, c_int, c_int, c_int, I16P, I16P, c_int,
-                                           c_int, c_int, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P,
-                                           c_int, P, ctypes.POINTER(BnReduce), ctypes.POINTER(c_int), P]
     L.jvae_conv_wgrad.argtypes = [P, c_int, c_int, c_int, c_int, c_int, P, c_int, c_int, c_int, c_int, c_int, I16P, I16P,
                                   c_int, P, c_int, c_int, c_int, P]
     L.jvae_conv_subpixel_gemm.argtypes = [P, c_int, c_int, c_int, c_int, c_int, P, c_int, c_int, c_int, I16P, I16P, I16P, I16P,
@@ -117,7 +107,7 @@ def lib():
     L.jvae_bn_stats.argtypes = [P, c_size_t, c_int, c_int, P, P]
     L.jvae_bn_apply_fwd.argtypes = [P, c_size_t, c_int, c_int, P, P, P, c_float, c_float, P, P, P, c_int, c_int, P, c_int,
                                     P, P]
-    L.jvae_bn_bwd.argtypes = [P, c_int, P, c_int, c_size_t, c_int, P, P, P, c_int, P, P, c_int, P, P, c_int, P]
+    L.jvae_bn_bwd.argtypes = [P, c_int, P, c_int, c_size_t, c_int, P, P, P, c_int, P, P, c_int, P, P, P]
     L.jvae_act_bwd.argtypes = [P, c_int, P, c_int, c_size_t, c_int, c_int, P, c_int, P, P]
     L.jvae_bn_stats_ld.argtypes = [P, c_size_t, c_int, c_int, P, c_int, P]
     L.jvae_bn_preact_fwd.argtypes = [P, c_size_t, c_int, c_int, P, c_int, P, P, c_float, c_float, P, P, P, c_int, c_int, P,
@@ -132,14 +122,13 @@ def lib():
     L.jvae_maxpool_pad_bwd.argtypes = [P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P, c_int, P, c_int, P]
     L.jvae_avgpool.argtypes = [P, c_int, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P]
     L.jvae_add_act.argtypes = [P, c_int, P, c_int, c_size_t, c_int, c_int, P, c_int, P]
-    L.jvae_vsum_rows.argtypes = [P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P, c_int, P, P, c_int, P]
     L.jvae_vstack_rows.argtypes = [P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P, c_int, P]
     L.jvae_elbo_prior_stats.argtypes = [ctypes.POINTER(ElboCfg), P, P, P, c_size_t, P]
     L.jvae_batch_u8_to_f32.argtypes = [ctypes.POINTER(BatchCfg), P, ctypes.c_longlong, P, c_int, P, P, P, P]
     L.jvae_last_conv_kernel.restype = c_int
     L.jvae_pack_job_blocks.argtypes = [ctypes.c_longlong, c_int, c_int]
     L.jvae_pack_weights.argtypes = [P, c_int, P, c_int, P]
-    if L.jvae_abi_version() != 16:
+    if L.jvae_abi_version() != 17:
         raise NativeError('ABI version mismatch between _native.py and libjvae_sm100.so')
     _lib = L
     return L
@@ -512,26 +501,12 @@ def taps_arg(taps):
 
 
 def conv_gather_gemm(inp, N, H, W, Cin, ld_in, wmat, Cout_pad, ldw, taps, in_stride, Hq, Wq, out, Ho, Wo, Cout, ld_out,
-                     out_s=(1, 1), out_o=(0, 0), bias=None, act=0, stats=None, bn=None):
-    """include/jvae_b200.h: jvae_conv_gather_gemm[_bn].  taps = (dy_array, dx_array) from taps_arg.
-    bn = dict(y, ld_y, save, gamma, beta, act): fold the previous layer's BatchNorm-backward reduction into this
-    data-gradient launch (sums go to `stats`); returns True when the launched kernel did it."""
-    if bn is None:
-        with _timed_conv(2.0 * N * Hq * Wq * len(taps[0]) * Cin * Cout):
-            check(lib().jvae_conv_gather_gemm(rawptr(inp), N, H, W, Cin, ld_in, rawptr(wmat), Cout_pad, ldw, len(taps[0]),
-                                              taps[0], taps[1], in_stride, Hq, Wq, rawptr(out), Ho, Wo, Cout, ld_out,
-                                              out_s[0], out_s[1], out_o[0], out_o[1], rawptr(bias), act, rawptr(stats),
-                                              stream()))
-        return False
-    d = BnReduce(y=bn['y'].data_ptr(), ld_y=bn['ld_y'], save_mean_rstd=bn['save'].data_ptr(),
-                 gamma=bn['gamma'].data_ptr() if bn['gamma'] is not None else None,
-                 beta=bn['beta'].data_ptr() if bn['beta'] is not None else None, act=bn['act'])
-    fused = c_int(0)
-    check(lib().jvae_conv_gather_gemm_bn(rawptr(inp), N, H, W, Cin, ld_in, rawptr(wmat), Cout_pad, ldw, len(taps[0]),
-                                         taps[0], taps[1], in_stride, Hq, Wq, rawptr(out), Ho, Wo, Cout, ld_out, out_s[0],
-                                         out_s[1], out_o[0], out_o[1], rawptr(bias), act, rawptr(stats), ctypes.byref(d),
-                                         ctypes.byref(fused), stream()))
-    return bool(fused.value)
+                     out_s=(1, 1), out_o=(0, 0), bias=None, act=0, stats=None):
+    """include/jvae_b200.h: jvae_conv_gather_gemm.  taps = (dy_array, dx_array) from taps_arg."""
+    with _timed_conv(2.0 * N * Hq * Wq * len(taps[0]) * Cin * Cout):
+        check(lib().jvae_conv_gather_gemm(rawptr(inp), N, H, W, Cin, ld_in, rawptr(wmat), Cout_pad, ldw, len(taps[0]),
+                                          taps[0], taps[1], in_stride, Hq, Wq, rawptr(out), Ho, Wo, Cout, ld_out,
+                                          out_s[0], out_s[1], out_o[0], out_o[1], rawptr(bias), act, rawptr(stats), stream()))
 
 
 NOT_COVERED = 1
@@ -624,9 +599,9 @@ def bn_apply_fwd(y, P, C, ld_y, stats, gamma, beta, eps, momentum, running_mean,
                                   int(training), act, rawptr(out), ld_out, rawptr(save), stream()))
 
 
-def bn_bwd(da, ld_da, y, ld_y, P, C, save, gamma, beta, act, sums, dy, ld_dy, dgamma, dbeta, skip_reduce=False):
+def bn_bwd(da, ld_da, y, ld_y, P, C, save, gamma, beta, act, sums, dy, ld_dy, dgamma, dbeta):
     check(lib().jvae_bn_bwd(rawptr(da), ld_da, rawptr(y), ld_y, P, C, rawptr(save), rawptr(gamma), rawptr(beta), act,
-                            rawptr(sums), rawptr(dy), ld_dy, rawptr(dgamma), rawptr(dbeta), int(skip_reduce), stream()))
+                            rawptr(sums), rawptr(dy), ld_dy, rawptr(dgamma), rawptr(dbeta), stream()))
 
 
 def bn_stats_ld(y, P, C, ld, stats, stats_ld):
@@ -680,11 +655,6 @@ def maxpool_pad_bwd(inp, N, H, W, C, ld_in, k, stride, pad, dout, ld_dout, din, 
 
 def avgpool(src, ld_src, dst, ld_dst, N, H, W, C, k, backward=False):
     check(lib().jvae_avgpool(rawptr(src), ld_src, rawptr(dst), ld_dst, N, H, W, C, k, int(backward), stream()))
-
-
-def vsum_rows(T, ld_t, N, H, W, k, pad, Co, bias, act, stats, out, ld_out):
-    check(lib().jvae_vsum_rows(rawptr(T), ld_t, N, H, W, k, pad, Co, rawptr(bias), act, rawptr(stats), rawptr(out), ld_out,
-                               stream()))
 
 
 def vstack_rows(dy, ld_dy, N, H, W, k, pad, Co, U, ld_u):

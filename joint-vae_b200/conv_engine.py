@@ -19,7 +19,6 @@ streaming pass (csrc/norm.cu), its backward two.
 `K` is the kernel backend: `NativeKernels` (ctypes -> CUDA) in the product.  tests/ substitute a torch emulation of the
 same entry points to check the tap tables / weight arrangements on machines without a GPU; the product never does.
 """
-import os
 
 import torch
 from torch import nn
@@ -42,24 +41,8 @@ def cout_pad_of(c):
 
 _ACT_CODE = {nn.ReLU: 1, nn.Sigmoid: 2, nn.Identity: 0, nn.LeakyReLU: 3}
 
-# Fold the BatchNorm-backward reduction of layer i-1 into the data-gradient kernel of layer i (jvae_conv_gather_gemm_bn).
-# Correct and covered by the GPU tests (run them with JVAE_FUSE_BN_REDUCE=1), but measured SLOWER on B200 at c2 even with the
-# saved pre-BN tile fed through its own TMA ring: +0.7 ms per fused 32-channel launch against 0.37 ms saved.  The N = 32
-# MMAs of these layers already saturate the shared-memory bandwidth (measured pacing, DESIGN.md section 3.2), so every
-# extra shared-memory read in the epilogue slows the MMAs themselves.  Opt-in until the per-channel constants move to
-# registers / the constant bank.
-import os as _os
-FUSE_BN_REDUCE = _os.environ.get('JVAE_FUSE_BN_REDUCE', '0') == '1'
-# opt-in, NOT yet measured on the GPU (DESIGN.md section 6, vgg19's 512-channel layers at 2x2): 'same' stride-1 convolutions on
-# maps of at most 2x2 pixels as ONE dense GEMM over (pixel, channel) pairs -- every (output pixel, input pixel) pair is exactly
-# one filter tap, so nothing is wasted on padding taps and the launch fills the machine (M = batch, N = K = pixels * channels)
-DENSE_SMALL = _os.environ.get('JVAE_CONV_DENSE_SMALL', '0') == '1'
-# the separable image head runs its FORWARD as the direct k x k convolution (tap-stacked halo kernel, one fp32 accumulation of all
-# k^2 taps, no fp32 intermediate of 16 channels per pixel): 336 us against 241 + 147 us at c2 since the second epilogue pass.  The
-# backward stays separable (data gradient 229 us against ~400 direct, weight gradient 184 against ~530).  0 restores the 1 x k pass.
-SEP_FWD_DIRECT = _os.environ.get('JVAE_HEAD_FWD_DIRECT', '1') != '0'
-# weight gradients on maps of at most this many pixels go through a patch matrix + one TN GEMM (0 disables)
-IM2COL_MAXPIX = int(_os.environ.get('JVAE_CONV_IM2COL_MAXPIX', '16'))
+# weight gradients on maps of at most this many pixels go through a patch matrix + one TN GEMM
+IM2COL_MAXPIX = 16
 
 
 # ------------------------------------------------------------------------------------------------ kernel backend
@@ -91,12 +74,12 @@ class NativeKernels:
         return nat.nhwc_bf16_to_nchw(t, C)
 
     @staticmethod
-    def gather(x, Cin, wmat, cout_pad, taps, in_stride, Hq, Wq, out, Cout, out_s, out_o, bias, act, stats, bn=None):
+    def gather(x, Cin, wmat, cout_pad, taps, in_stride, Hq, Wq, out, Cout, out_s, out_o, bias, act, stats):
         N, H, W, ld_in = x.shape
         _, Ho, Wo, _ = out.shape
         ld_out = out.stride(2)          # `out` may be a channel slice of a wider buffer (a dense block's new channels)
-        return nat.conv_gather_gemm(x, N, H, W, Cin, ld_in, wmat, cout_pad, wmat.shape[1], taps, in_stride, Hq, Wq, out, Ho,
-                                    Wo, Cout, ld_out, out_s, out_o, bias, act, stats, bn=bn)
+        nat.conv_gather_gemm(x, N, H, W, Cin, ld_in, wmat, cout_pad, wmat.shape[1], taps, in_stride, Hq, Wq, out, Ho, Wo, Cout,
+                             ld_out, out_s, out_o, bias, act, stats)
 
     @staticmethod
     def wgrad(g, Cg, x, Cx, taps, in_stride, dw, swapped=False):
@@ -156,7 +139,6 @@ class NativeKernels:
     maxpool_pad_bwd = staticmethod(nat.maxpool_pad_bwd)
     avgpool = staticmethod(nat.avgpool)
     add_act = staticmethod(nat.add_act)
-    vsum_rows = staticmethod(nat.vsum_rows)
     vstack_rows = staticmethod(nat.vstack_rows)
     taps_arg = staticmethod(nat.taps_arg)
 
@@ -339,12 +321,6 @@ class ConvStep:
         self.out_shape = (self.Co, self.Ho, self.Wo)
         self.gemm1x1 = (self.transposed and H == 1 and W == 1 and p == 0 and conv.output_padding[0] == 0
                         and self.Co % 8 == 0)
-        self.dense_small = DENSE_SMALL and (not self.transposed) and (not self.gemm1x1) and s == 1 and k > 1 and 2 * p == k - 1 \
-            and H * W <= 4 and Ci % 8 == 0 and self.Co % 8 == 0 and not final_dense
-        if self.dense_small:      # (output pixel q, input pixel r) -> filter tap (ry - qy + p, rx - qx + p) when inside the window
-            self.dense_pairs = [(qy * W + qx, ry * W + rx, ry - qy + p, rx - qx + p)
-                                for qy in range(H) for qx in range(W) for ry in range(H) for rx in range(W)
-                                if 0 <= ry - qy + p < k and 0 <= rx - qx + p < k]
         self.final_dense = final_dense
         self.ld_y = r8(self.Co) if (bn is not None or not final_dense) else self.Co
         self.ld_a = self.Co if final_dense else r8(self.Co)
@@ -374,12 +350,14 @@ class ConvStep:
         self.wgrad_swapped = (not self.transposed) and s == 1 and (self.Ho, self.Wo) == (H, W) and \
             cblk_of(min(self.Co, 64)) < cblk_of(min(Ci, 64))
         self.wgrad_taps_neg = [(-a, -b) for a, b in self.wgrad_taps]
-        # narrow image heads (32 -> 3, k5): the k x k 'same' convolution runs as a 1 x k convolution to k * Co channels on the
-        # tensor cores followed by a vertical shift-and-add (include/jvae_b200.h: jvae_vsum_rows / jvae_vstack_rows): k taps
-        # instead of k^2 in the forward, data-gradient and weight-gradient kernels
-        # k >= 5: with a 3 x 3 head (c4's ivgg) the 9 -> 3 tap reduction does not pay for the two row passes (measured: -0.24 ms)
+        # narrow image heads (32 -> 3, k5): the backward of the k x k 'same' convolution runs as the backward of a 1 x k
+        # convolution to k * Co channels whose vertical shift-and-add is the layer's output (include/jvae_b200.h:
+        # jvae_vstack_rows): k taps instead of k^2 in the data-gradient and weight-gradient kernels.  The forward runs direct
+        # (tap-stacked halo kernel, one fp32 accumulation of all k^2 taps): 336 us against 241 + 147 us at c2 for the
+        # separable forward, while the separable backward wins (data gradient 229 us against ~400 direct, weight gradient 184
+        # against ~530).  k >= 5: with a 3 x 3 head (c4's ivgg) the 9 -> 3 tap reduction does not pay (measured: -0.24 ms)
         self.separable = (not self.transposed) and (not self.gemm1x1) and s == 1 and k >= 5 and 2 * p == k - 1 and \
-            self.Co <= 4 and k * self.Co <= 16 and W >= 8 and os.environ.get('JVAE_CONV_SEPARABLE', '1') != '0'
+            self.Co <= 4 and k * self.Co <= 16 and W >= 8
         if self.separable:
             self.sep_C, self.sep_ld = k * self.Co, r8(k * self.Co)
             self.sep_fwd_taps = [(0, j - p) for j in range(k)]
@@ -402,9 +380,7 @@ class ConvStep:
 
     def pack_specs(self):
         """jobs of the native re-pack for the training-mode (unfolded) weights: the same arrangements _pack() builds with
-        torch ops (tests/test_conv_engine_cpu.py checks them against each other); [] when this layer keeps the torch path"""
-        if self.dense_small:
-            return []
+        torch ops (tests/test_conv_engine_cpu.py checks them against each other)"""
         kk, k, Co, Ci = self.k * self.k, self.k, self.Co, self.Ci
         if self.gemm1x1:      # W (Ci, Co, k, k): Bm[(yx, co)][ci] = W[ci][co][yx]; bias repeated per output pixel
             sp = [pack_spec('bm', 'w', kk * Co, Ci, [0], kk, Co * kk, R0=Co, s_r1=1, cols_pad=r8(Ci))]
@@ -417,10 +393,7 @@ class ConvStep:
         sp += [gather_spec('bwd', i, Ci, Co, op['idx'], s_ci, s_co) for i, op in enumerate(self.dgrad_ops)]
         if self.merged_fwd:
             sp.append(gather_spec('fwd_all', None, Co, Ci, self.fwd_all_idx, s_co, s_ci))
-        if self.separable:    # rows (ky, co) of the 1 x k kernel over kx taps; and [ci][kx][(ky, co)] for the data gradient
-            cb = cblk_of(Ci)
-            sp.append(pack_spec('sep_fwd', 'w', k * Co, Ci, range(k), s_co, s_ci, R0=Co, s_r1=k,
-                                rows_pad=cout_pad_of(k * Co), cols_pad=((Ci + cb - 1) // cb) * cb))
+        if self.separable:    # [ci][kx][(ky, co)]: the data gradient of the 1 x k kernel
             cb = cblk_of(k * Co)
             sp.append(pack_spec('sep_bwd', 'w', Ci, k * Co, range(k), s_ci, s_co, C0=Co, s_c1=k,
                                 rows_pad=cout_pad_of(Ci), cols_pad=((k * Co + cb - 1) // cb) * cb))
@@ -436,11 +409,11 @@ class ConvStep:
     def _pack(self, fold_bn=False, want_bwd=None):
         """bf16 weight arrangements, refreshed when the Parameter changes (optimizer step / load_state_dict / in-place
         writes).  Training-mode weights on the GPU come from the stack's PackPlan (one native launch per stack and step);
-        this torch formulation serves the BatchNorm-folded inference weights, the opt-in dense form and the CPU emulation.
+        this torch formulation serves the BatchNorm-folded inference weights and the CPU emulation.
         fold_bn (inference with running statistics): BatchNorm is folded into the weights and the bias, so the layer is
         ONE kernel: W' = W * gamma * rstd, b' = (b - mean) * gamma * rstd + beta."""
         w = self.conv.weight
-        if not fold_bn and K is NativeKernels and not self.dense_small:
+        if not fold_bn and K is NativeKernels:
             plan = getattr(self, 'plan', None)
             if plan is None:                      # a step used outside a ConvStack
                 plan = self.plan = PackPlan([self])
@@ -494,17 +467,8 @@ class ConvStep:
             d['fwd'] = [pack_gather_weights(g_f, op['idx'], self.Ci) for op in self.fwd_ops]
             if self.merged_fwd:
                 d['fwd_all'] = pack_gather_weights(g_f, self.fwd_all_idx, self.Ci)
-            if self.dense_small:     # W_eff[(q, co), (r, ci)] = W[co][ci][tap(q, r)]
-                hw = self.H * self.W
-                weff = torch.zeros((hw, self.Co, hw, self.Ci), dtype=torch.float32, device=w.device)
-                for q, r, ty, tx in self.dense_pairs:
-                    weff[q, :, r, :] = wd[:, :, ty, tx]
-                d['dense'] = weff.view(hw * self.Co, hw * self.Ci).to(torch.bfloat16).contiguous()
-                d['dense_bias'] = b0.repeat(hw).contiguous() if b0 is not None else None
-            if self.separable:      # wd (Co, Ci, ky, kx): rows (ky, co) of the 1 x k kernel, and its transpose for the data gradient
+            if self.separable:      # wd (Co, Ci, ky, kx): the transpose of the 1 x k kernel for the data gradient
                 kq = self.k
-                d['sep_fwd'] = pack_gather_weights(wd.permute(2, 0, 3, 1).reshape(kq * self.Co, kq, self.Ci),
-                                                   list(range(kq)), self.Ci)
                 d['sep_bwd'] = pack_gather_weights(wd.permute(1, 3, 2, 0).reshape(self.Ci, kq, kq * self.Co),
                                                    list(range(kq)), kq * self.Co)
             if want_bwd:
@@ -526,7 +490,7 @@ class ConvStep:
         if y is None:
             y = K.empty((N, self.Ho, self.Wo, self.ld_y), x)
         else:
-            assert bn is None and not (self.gemm1x1 or self.dense_small or self.separable or self.merged_fwd)
+            assert bn is None and not (self.gemm1x1 or self.separable or self.merged_fwd)
         stats = (st.pop('stats_buf', None) if bn_train else None)
         if bn_train and stats is None:
             stats = K.zeros((2, self.Co), x, torch.float64)
@@ -537,14 +501,6 @@ class ConvStep:
                    out_bf16=y.view(N, kk * self.Co))
             if bn_train:
                 K.bn_stats(y, N * kk, self.Co, self.ld_y, stats)
-        elif self.dense_small:
-            hw = self.H * self.W
-            K.gemm(nat.GEMM_NT, N, hw * self.Co, hw * self.Ci, x.view(N, hw * self.Ci), pk['dense'], bias=pk['dense_bias'],
-                   act=fused_act, out_bf16=y.view(N, hw * self.Co))
-            if bn_train:
-                K.bn_stats(y, N * hw, self.Co, self.ld_y, stats)
-        elif self.separable and not SEP_FWD_DIRECT:
-            self._sep_forward(x, pk, bias, fused_act, stats, y)
         elif not self._merged_forward(x, pk, y, bias, fused_act, stats):
             for i, (op, wm) in enumerate(zip(self.fwd_ops, pk['fwd'])):
                 K.gather(x, self.Ci, wm, wm.shape[0], self._taps(('f', i), op['taps']), op['in_stride'], op['Hq'], op['Wq'],
@@ -577,18 +533,6 @@ class ConvStep:
         op = self.fwd_ops[0]
         return K.subpixel(x, self.Ci, wm, wm.shape[0], ph, op['Hq'], op['Wq'], out, self.Co, self.s, bias, act, stats)
 
-    def _sep_forward(self, x, pk, bias, act, stats, out):
-        """1 x k convolution to k * Co channels (tensor cores), then the vertical shift-and-add with bias / activation / stats.
-        T stays fp32: the k vertical taps of an output pixel cancel, and rounding them to bf16 first costs the gradients of the
-        head and of the layer under it an order of magnitude (measured: 25 % instead of 1.8 % on the head's weight gradient)."""
-        N = x.shape[0]
-        T = K.empty((N, self.H, self.W, self.sep_ld), x, torch.float32)
-        wm = pk['sep_fwd']
-        K.gather(x, self.Ci, wm, wm.shape[0], self._taps('sf', self.sep_fwd_taps), 1, self.H, self.W, T, self.sep_C, (1, 1),
-                 (0, 0), None, nat.OUT_F32, None)
-        K.vsum_rows(T, self.sep_ld, N, self.H, self.W, self.k, self.p, self.Co, bias, act | nat.IN_F32, stats, out,
-                    out.shape[-1])
-
     def _forward_folded(self, x, st):
         """inference: conv + folded BatchNorm + activation in one kernel, no intermediate tensor"""
         N = x.shape[0]
@@ -598,12 +542,6 @@ class ConvStep:
             kk = self.k * self.k
             K.gemm(nat.GEMM_NT, N, kk * self.Co, self.Ci, x.view(N, x.shape[-1]), pk['bm'], bias=pk['bias'], act=self.act,
                    out_bf16=a.view(N, kk * self.Co))
-        elif self.dense_small:
-            hw = self.H * self.W
-            K.gemm(nat.GEMM_NT, N, hw * self.Co, hw * self.Ci, x.view(N, hw * self.Ci), pk['dense'], bias=pk['dense_bias'],
-                   act=self.act, out_bf16=a.view(N, hw * self.Co))
-        elif self.separable and not SEP_FWD_DIRECT:
-            self._sep_forward(x, pk, pk['b'], self.act, None, a)
         elif not self._merged_forward(x, pk, a, pk['b'], self.act, None):
             for i, (op, wm) in enumerate(zip(self.fwd_ops, pk['fwd'])):
                 K.gather(x, self.Ci, wm, wm.shape[0], self._taps(('f', i), op['taps']), op['in_stride'], op['Hq'], op['Wq'],
@@ -612,10 +550,7 @@ class ConvStep:
         return a
 
     # ---- backward: da = dL/d(output) NHWC bf16 -> (dx or None, [param grads])
-    def backward(self, da, st, need_dx, prev_bn=None):
-        """prev_bn: dict describing the previous layer's train-mode BatchNorm (y, ld_y, save, gamma, beta, act, sums): its
-        backward reduction is folded into this layer's data-gradient kernel when the kernel supports it; prev_bn['done']
-        then tells that layer to skip its own reduction pass."""
+    def backward(self, da, st, need_dx):
         x = st['x']
         N = x.shape[0]
         P = N * self.Ho * self.Wo
@@ -635,16 +570,14 @@ class ConvStep:
         elif bn is not None:
             y = st['y']
             dy = K.empty(y.shape, x)
-            pre = st.get('bn_sums')            # produced by the next layer's data-gradient kernel
-            sums = pre if pre is not None else K.empty((2, self.Co), x, torch.float64)
+            sums = K.empty((2, self.Co), x, torch.float64)
             dg = db = lg = lb = None
             if bn.affine:
                 lg, lb = _live_grad(bn.weight, x), _live_grad(bn.bias, x)
                 dg = lg if lg is not None else K.zeros((self.Co,), x)
                 db = lb if lb is not None else K.zeros((self.Co,), x)
             K.bn_bwd(da, da.shape[-1], y, self.ld_y, P, self.Co, st['save'], bn.weight.detach() if bn.affine else None,
-                     bn.bias.detach() if bn.affine else None, self.act, sums, dy, self.ld_y, dg, db,
-                     **({'skip_reduce': True} if pre is not None else {}))
+                     bn.bias.detach() if bn.affine else None, self.act, sums, dy, self.ld_y, dg, db)
             grads['bn_w'], grads['bn_b'] = (None if lg is not None else dg), (None if lb is not None else db)
             # the bias of a convolution followed by train-mode BatchNorm has an exactly zero gradient
             # (BN subtracts the batch mean); the reference's autograd returns rounding noise here
@@ -685,22 +618,6 @@ class ConvStep:
                     K.gemm(nat.GEMM_NN, N, self.Ci, kk * self.Co, dy2, pk['bm'], out_f32=tmp)
                     dx = K.zeros(x.shape, x, torch.bfloat16)
                     dx.view(N, ldx)[:, :self.Ci] = tmp
-        elif self.dense_small:
-            hw = self.H * self.W
-            dy2, x2 = dy.view(N, hw * self.Co), x.view(N, hw * self.Ci)
-            if not folded:
-                dweff = K.empty((hw * self.Co, hw * self.Ci), x, torch.float32)
-                K.gemm(nat.GEMM_TN, hw * self.Co, hw * self.Ci, N, dy2, x2, out_f32=dweff)
-                dw4 = dweff.view(hw, self.Co, hw, self.Ci)
-                w = self.conv.weight
-                live = _live_grad(w, x)
-                dw = live if live is not None else K.zeros(tuple(w.shape), x)
-                for q, r, ty, tx in self.dense_pairs:          # fold the (pixel, pixel) blocks back onto their taps
-                    dw[:, :, ty, tx] += dw4[q, :, r, :]
-                grads['w'] = None if live is not None else dw
-            if need_dx:
-                dx = K.empty(x.shape, x)
-                K.gemm(nat.GEMM_NN, N, hw * self.Ci, hw * self.Co, dy2, pk['dense'], out_bf16=dx.view(N, hw * self.Ci))
         elif self.separable:
             kq = self.k
             U = K.empty((N, self.H, self.W, self.sep_ld), x)      # gradient of the 1 x k stage's output
@@ -738,17 +655,9 @@ class ConvStep:
                 grads['w'] = None if live is not None else dw
             if need_dx:
                 dx = K.zeros(x.shape, x, torch.bfloat16) if self.dgrad_sparse else K.empty(x.shape, x)
-                fuse = FUSE_BN_REDUCE and prev_bn is not None and K is NativeKernels and \
-                    prev_bn['y'].shape[:3] == dx.shape[:3]
-                sums_prev = K.zeros((2, self.Ci), x, torch.float64) if fuse else None
-                done = fuse
                 for i, (op, wm) in enumerate(zip(self.dgrad_ops, pk['bwd'])):
-                    r = K.gather(dy, self.Co, wm, wm.shape[0], self._taps(('b', i), op['taps']), op['in_stride'], op['Hq'],
-                                 op['Wq'], dx, self.Ci, op['out_s'], op['out_o'], None, 0, sums_prev,
-                                 **({'bn': prev_bn} if fuse else {}))
-                    done = done and bool(r)
-                if fuse and done:
-                    prev_bn['sums'] = sums_prev
+                    K.gather(dy, self.Co, wm, wm.shape[0], self._taps(('b', i), op['taps']), op['in_stride'], op['Hq'],
+                             op['Wq'], dx, self.Ci, op['out_s'], op['out_o'], None, 0, None)
         out = [grads['w'], grads['b']]
         if bn is not None:
             out += [grads['bn_w'], grads['bn_b']]
@@ -1262,18 +1171,7 @@ class ConvStack:
             g = K.to_nhwc(dout, ld_last)
         grads = []
         for idx in range(len(self.steps) - 1, -1, -1):
-            s = self.steps[idx]
-            kw = {}
-            prev = self.steps[idx - 1] if idx > 0 else None
-            if isinstance(s, ConvStep) and isinstance(prev, ConvStep) and prev.bn is not None and \
-                    state[idx - 1].get('bn_train') and not s.gemm1x1:
-                pb = prev.bn
-                kw['prev_bn'] = dict(y=state[idx - 1]['y'], ld_y=prev.ld_y, save=state[idx - 1]['save'],
-                                     gamma=pb.weight.detach() if pb.affine else None,
-                                     beta=pb.bias.detach() if pb.affine else None, act=prev.act)
-            g, pg = s.backward(g, state[idx], need_dx or idx > 0, **kw)
-            if 'prev_bn' in kw and kw['prev_bn'].get('sums') is not None:
-                state[idx - 1]['bn_sums'] = kw['prev_bn']['sums']
+            g, pg = self.steps[idx].backward(g, state[idx], need_dx or idx > 0)
             grads = pg + grads
             if g is None:
                 break

@@ -14,7 +14,6 @@
 #include "tc_common.cuh"
 #include <vector>
 #include <algorithm>
-#include <stdlib.h>
 
 namespace jvae {
 
@@ -38,7 +37,6 @@ struct ConvParams {
   int Ho, Wo, Cout, ldc;       // output tensor (N, Ho, Wo, ldc channels); Cout real channels written
   int out_sy, out_sx, out_oy, out_ox;   // output pixel = q * out_s + out_o
   int act;
-  int out_f32;                 // 1: `out` holds fp32 (ldc counts floats): JVAE_OUT_F32
   const float* bias;
   __nv_bfloat16* out;
   double* stats;               // (2, Cout) per-channel sum / sum of squares of the pre-activation, += (or null)
@@ -243,11 +241,7 @@ conv_gather_gemm_kernel(const __grid_constant__ CUtensorMap tmap_in, const __gri
 #pragma unroll
             for (int j = 0; j < 16; ++j) v[j] = v[j] > 0.f ? v[j] : JVAE_LEAKY_SLOPE * v[j];
           }
-          if (p.out_f32) {
-            float* of = reinterpret_cast<float*>(p.out) + (((size_t)n * p.Ho + oy) * p.Wo + ox) * p.ldc + (size_t)nt * p.BN + c0;
-            for (int j = 0; j < 16; ++j)
-              if (ch0 + c0 + j < p.ldc) of[j] = v[j];
-          } else if (ch0 + c0 + 16 <= p.ldc && (p.ldc & 15) == 0 && (reinterpret_cast<uintptr_t>(p.out) & 31) == 0) {
+          if (ch0 + c0 + 16 <= p.ldc && (p.ldc & 15) == 0 && (reinterpret_cast<uintptr_t>(p.out) & 31) == 0) {
             st_global_v8(orow + c0, pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7]),
                          pack_bf16(v[8], v[9]), pack_bf16(v[10], v[11]), pack_bf16(v[12], v[13]), pack_bf16(v[14], v[15]));
           } else if (ch0 + c0 + 16 <= p.ldc && (p.ldc & 7) == 0) {
@@ -298,7 +292,7 @@ struct HaloParams {
   int RT, NBt, HHs, HWp, MT;            // rows / images per box, slots per image, halo width (pixels), M-tiles per box
   int strips_x, blocks_y, blocks_n, num_boxes, n_tiles_n;
   int Cblk, ntaps, BN;
-  int nkc;                               // input-channel chunks of Cblk (wide layers: Cin > 64); 1 otherwise
+  int nkc;                               // input-channel chunks of Cblk (2: a 33..64-channel input in 32-channel chunks); 1 otherwise
   int dymin, dxmin;                      // smallest tap offset in PLANE coordinates (e = (d - r) / in_stride)
   int in_stride, nplanes;                // input stride s: the input is read as up to s*s parity planes P_r[j] = in[s*j + r]
   short plane_ry[4], plane_rx[4];
@@ -306,17 +300,10 @@ struct HaloParams {
   short dy[CONV_MAX_TAPS], dx[CONV_MAX_TAPS];
   uint32_t tap_off16[CONV_MAX_TAPS];     // (plane * plane_bytes + ((ey-eymin)*HWp + (ex-exmin)) * row bytes) / 16
   int Ho, Wo, Cout, ldc, out_sy, out_sx, out_oy, out_ox, act;
-  int out_f32;                           // 1: `out` holds fp32 (ldc counts floats): JVAE_OUT_F32
   const float* bias;
   __nv_bfloat16* out;
   double* stats;
   int cout_pad;
-  // fused BatchNorm-backward reduction (data-gradient launches): this launch's output is dL/da of the PREVIOUS layer,
-  // bn_y that layer's pre-BN output at the same pixels (read by the epilogue threads straight from global memory); stats then
-  // receives sum g*act'(z) and sum g*act'(z)*xhat
-  const __nv_bfloat16* bn_y;
-  const float* bn_save; const float* bn_gamma; const float* bn_beta;
-  int bn_ld, bn_act;
   uint32_t stage_bytes, box_bytes, w_tap_bytes, w_bytes, tmem_cols, acc_stride;
   int stages, resident, wstages;
   // Vertical tap stacking (G > 1): one M row stands for G consecutive output rows (slots) of one pixel column; the N side of an
@@ -414,16 +401,11 @@ __device__ __forceinline__ void halo_mma_box_g(const HaloParams& p, uint32_t d0,
 //   * two warps per TMEM lane quarter (set = 0 / 1): a set takes every other 16-channel chunk of each block (every other block
 //     for 16-channel tiles), so a scheduler interleaves two independent drains and a thread keeps statistics for at most 32
 //     channels.
-// MODE 0: plain; 1: BatchNorm batch statistics of the output (sum y, sum y^2); 2: BatchNorm-BACKWARD sums of the previous layer
-// (data-gradient launches whose output is dL/da of a conv-BN-activation layer): with y that layer's saved pre-BN output at the
-// same pixel (two 16-byte global loads per chunk, requested before the accumulator is read), g' = g * act'(scale y + shift),
-// the thread accumulates sum g' and sum g' y; the CTA turns them into sum g' and sum g' xhat = rstd (sum g' y - mean sum g').
-template <int NCH, int MODE>
+// STATS: BatchNorm batch statistics of the output (sum y, sum y^2).
+template <int NCH, bool STATS>
 __device__ __forceinline__ void halo_epilogue_fast(const HaloParams& p, uint32_t tmem_base, uint64_t* tfull_bar, uint64_t* tempty_bar,
-                                                   double* s_stats, const float* s_bias, const float* s_bn, int2* s_tab, int warp,
-                                                   int lane, int nt, int box0, int box_step) {
-  constexpr bool STATS = MODE != 0;
-  constexpr bool BNRED = MODE == 2;
+                                                   double* s_stats, const float* s_bias, int2* s_tab, int warp, int lane, int nt,
+                                                   int box0, int box_step) {
   constexpr int LC = (NCH + 1) / 2;              // chunks a thread handles at most
   const int set = (warp - 2) >> 2;               // warps 2..5: set 0, warps 6..9: set 1
   const int q = warp & 3;
@@ -452,11 +434,11 @@ __device__ __forceinline__ void halo_epilogue_fast(const HaloParams& p, uint32_t
   const bool has_bias = p.bias != nullptr;
   const uint32_t sb = smem_u32(s_bias);
   const uint32_t stab = smem_u32(s_tab) + 8u * (uint32_t)(mrow >> 3);      // this thread's entry of block 0
-  const bool vec_bf16 = (p.ldc & 7) == 0, vec_f32 = (p.ldc & 3) == 0;
+  const bool vec_bf16 = (p.ldc & 7) == 0;
   // 32-byte stores (st.global.v8.b32) when the thread's 16 channels start on a 32-byte boundary: one full sector per instruction
   // instead of two half sectors (the scattered 16-byte stores of the sub-pixel / narrow layers kept L1TEX 67 % busy)
   const bool al32 = (reinterpret_cast<uintptr_t>(p.out) & 31) == 0;
-  const bool v8_bf16 = al32 && (p.ldc & 15) == 0, v8_f32 = al32 && (p.ldc & 7) == 0;
+  const bool v8_bf16 = al32 && (p.ldc & 15) == 0;
   uint32_t it = 0;
   // (strip, row block, image block) of the box, advanced by the decomposition of box_step with carries: the two runtime
   // divisions per box were a fifth of the epilogue's stall samples on launches with few blocks per box (ncu source view)
@@ -496,16 +478,6 @@ __device__ __forceinline__ void halo_epilogue_fast(const HaloParams& p, uint32_t
       if (!__any_sync(0xffffffffu, ok)) continue;
       const uint32_t t_addr = tmem_base + acc * p.acc_stride + (uint32_t)(blk * p.BN) + ((uint32_t)(q * 32) << 16);
       const size_t pix = pix0 + (size_t)(ok ? e.x : 0);
-      uint4 yq[BNRED ? LC : 1][2];
-      if (BNRED && ok) {
-#pragma unroll
-        for (int lc = 0; lc < LC; ++lc)
-          if (c_first + 2 * lc < NCH && ch0 + (c_first + 2 * lc) * 16 < p.Cout) {
-            const __nv_bfloat16* yp = p.bn_y + pix * (size_t)p.bn_ld + (size_t)(ch0 + (c_first + 2 * lc) * 16);
-            yq[lc][0] = ld_stream16(yp);
-            yq[lc][1] = ld_stream16(yp + 8);
-          }
-      }
       // the bias of the thread's channels is requested BEFORE the accumulator (its latency hides under the TMEM load, and the
       // sum lands in the accumulator's own registers: with the loads after the wait the compiler copied all 16 values away
       // and back, 32 of ~145 instructions per block)
@@ -538,33 +510,7 @@ __device__ __forceinline__ void halo_epilogue_fast(const HaloParams& p, uint32_t
 #pragma unroll
           for (int j = 0; j < 16; ++j) v[j] += bq[lc][j];
         }
-        if (BNRED) {
-          float y[16];
-          {
-            const uint4 u0 = yq[BNRED ? lc : 0][0], u1 = yq[BNRED ? lc : 0][1];
-            y[0] = bf16_lo(u0.x); y[1] = bf16_hi(u0.x); y[2] = bf16_lo(u0.y); y[3] = bf16_hi(u0.y);
-            y[4] = bf16_lo(u0.z); y[5] = bf16_hi(u0.z); y[6] = bf16_lo(u0.w); y[7] = bf16_hi(u0.w);
-            y[8] = bf16_lo(u1.x); y[9] = bf16_hi(u1.x); y[10] = bf16_lo(u1.y); y[11] = bf16_hi(u1.y);
-            y[12] = bf16_lo(u1.z); y[13] = bf16_hi(u1.z); y[14] = bf16_lo(u1.w); y[15] = bf16_hi(u1.w);
-          }
-          const uint32_t sbn = smem_u32(s_bn);
-#pragma unroll
-          for (int j = 0; j < 16; j += 4) {
-            float sc[4], sh[4];
-            asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(sc[0]), "=f"(sc[1]), "=f"(sc[2]), "=f"(sc[3]) : "r"(sbn + 4u * (128 + c * 16 + j)));
-            asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(sh[0]), "=f"(sh[1]), "=f"(sh[2]), "=f"(sh[3]) : "r"(sbn + 4u * (192 + c * 16 + j)));
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              const float z = fmaf(y[j + i], sc[i], sh[i]);
-              float gz = v[j + i];
-              if (p.bn_act == JVAE_ACT_RELU) gz = z > 0.f ? gz : 0.f;
-              else if (p.bn_act == JVAE_ACT_LEAKY) gz = z > 0.f ? gz : JVAE_LEAKY_SLOPE * gz;
-              else if (p.bn_act == JVAE_ACT_SIGMOID) { const float sg = 1.f / (1.f + __expf(-z)); gz *= sg * (1.f - sg); }
-              s1[lc * 16 + j + i] += gz;
-              s2[lc * 16 + j + i] = fmaf(gz, y[j + i], s2[lc * 16 + j + i]);
-            }
-          }
-        } else if (STATS) {
+        if (STATS) {
 #pragma unroll
           for (int j = 0; j < 16; ++j) { s1[lc * 16 + j] += v[j]; s2[lc * 16 + j] = fmaf(v[j], v[j], s2[lc * 16 + j]); }
           // keeps the sums ahead of the activation: sunk below it they needed a second copy of the 16 values (32 moves per block)
@@ -584,38 +530,20 @@ __device__ __forceinline__ void halo_epilogue_fast(const HaloParams& p, uint32_t
           }
         }
         const int c0 = c * 16;
-        const size_t off = pix * (size_t)p.ldc + (size_t)(ch0 + c0);
-        if (p.out_f32) {
-          float* o = reinterpret_cast<float*>(p.out) + off;
-          if (ch0 + c0 + 16 <= p.ldc && v8_f32) {
-            st_global_v8(o, __float_as_uint(v[0]), __float_as_uint(v[1]), __float_as_uint(v[2]), __float_as_uint(v[3]),
-                         __float_as_uint(v[4]), __float_as_uint(v[5]), __float_as_uint(v[6]), __float_as_uint(v[7]));
-            st_global_v8(o + 8, __float_as_uint(v[8]), __float_as_uint(v[9]), __float_as_uint(v[10]), __float_as_uint(v[11]),
-                         __float_as_uint(v[12]), __float_as_uint(v[13]), __float_as_uint(v[14]), __float_as_uint(v[15]));
-          } else if (ch0 + c0 + 16 <= p.ldc && vec_f32) {
-#pragma unroll
-            for (int j = 0; j < 16; j += 4) *reinterpret_cast<float4*>(o + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
-          } else {
-#pragma unroll
-            for (int j = 0; j < 16; ++j)
-              if (ch0 + c0 + j < p.ldc) o[j] = ch0 + c0 + j < p.Cout ? v[j] : 0.f;
-          }
+        __nv_bfloat16* o = p.out + pix * (size_t)p.ldc + (size_t)(ch0 + c0);
+        if (ch0 + c0 + 16 <= p.ldc && v8_bf16) {
+          st_global_v8(o, pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7]),
+                       pack_bf16(v[8], v[9]), pack_bf16(v[10], v[11]), pack_bf16(v[12], v[13]), pack_bf16(v[14], v[15]));
+        } else if (ch0 + c0 + 16 <= p.ldc && vec_bf16) {
+          uint4 o0, o1;
+          o0.x = pack_bf16(v[0], v[1]); o0.y = pack_bf16(v[2], v[3]); o0.z = pack_bf16(v[4], v[5]); o0.w = pack_bf16(v[6], v[7]);
+          o1.x = pack_bf16(v[8], v[9]); o1.y = pack_bf16(v[10], v[11]); o1.z = pack_bf16(v[12], v[13]); o1.w = pack_bf16(v[14], v[15]);
+          *reinterpret_cast<uint4*>(o) = o0;
+          *reinterpret_cast<uint4*>(o + 8) = o1;
         } else {
-          __nv_bfloat16* o = p.out + off;
-          if (ch0 + c0 + 16 <= p.ldc && v8_bf16) {
-            st_global_v8(o, pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7]),
-                         pack_bf16(v[8], v[9]), pack_bf16(v[10], v[11]), pack_bf16(v[12], v[13]), pack_bf16(v[14], v[15]));
-          } else if (ch0 + c0 + 16 <= p.ldc && vec_bf16) {
-            uint4 o0, o1;
-            o0.x = pack_bf16(v[0], v[1]); o0.y = pack_bf16(v[2], v[3]); o0.z = pack_bf16(v[4], v[5]); o0.w = pack_bf16(v[6], v[7]);
-            o1.x = pack_bf16(v[8], v[9]); o1.y = pack_bf16(v[10], v[11]); o1.z = pack_bf16(v[12], v[13]); o1.w = pack_bf16(v[14], v[15]);
-            *reinterpret_cast<uint4*>(o) = o0;
-            *reinterpret_cast<uint4*>(o + 8) = o1;
-          } else {
 #pragma unroll
-            for (int j = 0; j < 16; ++j)
-              if (ch0 + c0 + j < p.ldc) o[j] = __float2bfloat16(ch0 + c0 + j < p.Cout ? v[j] : 0.f);
-          }
+          for (int j = 0; j < 16; ++j)
+            if (ch0 + c0 + j < p.ldc) o[j] = __float2bfloat16(ch0 + c0 + j < p.Cout ? v[j] : 0.f);
         }
       }
     }
@@ -643,9 +571,7 @@ __device__ __forceinline__ void halo_epilogue_fast(const HaloParams& p, uint32_t
     const int t = threadIdx.x - 64;
     for (int i = t; i < 2 * p.cout_pad; i += 256) {
       const int ch = i % p.cout_pad;
-      double val = s_stats[i];
-      if (BNRED && i >= p.cout_pad && ch - ch0 >= 0 && ch - ch0 < p.BN)      // sum g' xhat = rstd (sum g' y - mean sum g')
-        val = (double)s_bn[64 + ch - ch0] * (val - (double)s_bn[ch - ch0] * s_stats[ch]);
+      const double val = s_stats[i];
       if (ch < p.Cout && val != 0.0) atomicAdd(&p.stats[(i / p.cout_pad) * p.Cout + ch], val);
     }
   }
@@ -670,17 +596,10 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmap_in, const __grid_const
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int nt = (int)blockIdx.x % p.n_tiles_n;
-  float* s_bn = s_bias + 64;                                               // [4][64]: mean, rstd, scale, shift (bn_y launches)
-  int2* s_tab = reinterpret_cast<int2*>(s_bn + 256);                       // [MT * G][16]: block table of the fast epilogue
+  int2* s_tab = reinterpret_cast<int2*>(s_bias + 64);                      // [MT * G][16]: block table of the fast epilogue
   for (int i = threadIdx.x; i < p.BN; i += HALO_THREADS) {
     const int ch = nt * p.BN + i;
     s_bias[i] = (p.bias && ch < p.Cout) ? p.bias[ch] : 0.f;
-    if (p.bn_y) {
-      const bool live = ch < p.Cout;
-      const float mean = live ? p.bn_save[ch] : 0.f, rstd = live ? p.bn_save[p.Cout + ch] : 0.f;
-      const float g = (live && p.bn_gamma) ? p.bn_gamma[ch] : 1.f, b = (live && p.bn_beta) ? p.bn_beta[ch] : 0.f;
-      s_bn[i] = mean; s_bn[64 + i] = rstd; s_bn[128 + i] = live ? g * rstd : 0.f; s_bn[192 + i] = live ? b - mean * g * rstd : 0.f;
-    }
   }
   const int box0 = (int)blockIdx.x / p.n_tiles_n, box_step = (int)gridDim.x / p.n_tiles_n;
   const uint32_t rb = (uint32_t)p.Cblk * 2u;
@@ -792,10 +711,9 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmap_in, const __grid_const
     }
   } else {
     // ================= epilogue =================
-#define HALO_EPI_FAST(NCH_)                                                                                                            \
-    if (p.bn_y) halo_epilogue_fast<NCH_, 2>(p, tmem_base, tfull_bar, tempty_bar, s_stats, s_bias, s_bn, s_tab, warp, lane, nt, box0, box_step);    \
-    else if (p.stats) halo_epilogue_fast<NCH_, 1>(p, tmem_base, tfull_bar, tempty_bar, s_stats, s_bias, s_bn, s_tab, warp, lane, nt, box0, box_step); \
-    else halo_epilogue_fast<NCH_, 0>(p, tmem_base, tfull_bar, tempty_bar, s_stats, s_bias, s_bn, s_tab, warp, lane, nt, box0, box_step)
+#define HALO_EPI_FAST(NCH_)                                                                                                      \
+    if (p.stats) halo_epilogue_fast<NCH_, true>(p, tmem_base, tfull_bar, tempty_bar, s_stats, s_bias, s_tab, warp, lane, nt, box0, box_step); \
+    else halo_epilogue_fast<NCH_, false>(p, tmem_base, tfull_bar, tempty_bar, s_stats, s_bias, s_tab, warp, lane, nt, box0, box_step)
     switch (p.BN >> 4) {
       case 1: HALO_EPI_FAST(1); break;
       case 2: HALO_EPI_FAST(2); break;
@@ -1138,40 +1056,28 @@ struct PhaseSpec { int n; const int16_t* ntaps; const int16_t* oy; const int16_t
 static int try_launch_halo(const void* in, int N, int H, int W, int Cin, int ld_in, const void* wmat, int Cout_pad, int ldw,
                            int ntaps, const int16_t* tap_dy, const int16_t* tap_dx, int in_stride, int Hq, int Wq, void* out,
                            int Ho, int Wo, int Cout, int ld_out, int out_sy, int out_sx, int out_oy, int out_ox,
-                           const float* bias, int act, double* stats, const jvae_bn_reduce* bn, int* bn_fused,
-                           cudaStream_t stream, const PhaseSpec* phs = nullptr, HaloParams* plan_out = nullptr,
-                           int force_cblk = 0, double* score_out = nullptr) {
+                           const float* bias, int act, double* stats, cudaStream_t stream, const PhaseSpec* phs = nullptr,
+                           HaloParams* plan_out = nullptr, int force_cblk = 0, double* score_out = nullptr) {
   if (Wq < 6) return 1;
-  // wide layers (Cin > 64 or more than 64 output channels): 64-channel output tiles (the epilogue keeps per-thread statistics
-  // for at most 32 channels per warp set), the input channels in chunks of 64, weights streamed per (tap, chunk); the input
-  // box is read once per (box, chunk) instead of once per tap as in the tap-box kernel.  Opt-in (JVAE_CONV_WIDE=1, read per call
-  // so a test can switch it): measured on B200 it moves 0.71 ms of the c2 step out of the tap-box kernel and costs 0.87 ms here
-  // (N = 64 MMAs at 48 cycles against N = 256 at 128, the box re-read by each of the 2-8 channel tiles, 2.3 waves of work
-  // items on the 8 x 8 maps), so the vgg19 / ResNet bodies stay on the tap-box kernels by default.
-  const bool wide = Cin > 64 || Cout_pad > 64;
-  if (phs && (wide || in_stride != 1 || phs->n < 2 || phs->n > 4 || bn)) return 1;
-  if (wide) {
-    const bool wide_on = getenv("JVAE_CONV_WIDE") && atoi(getenv("JVAE_CONV_WIDE")) != 0;
-    if (!wide_on || (Cout_pad > 64 && (Cout_pad % 64) != 0) || bn) return 1;
-  }
-  if (bn && !(out_sy == 1 && out_sx == 1 && out_oy == 0 && out_ox == 0 && Ho == Hq && Wo == Wq)) {
-    bn = nullptr; stats = nullptr;                        // phase launches: the caller runs the separate reduction
-  }
+  // wide layers (Cin > 64 or more than 64 output channels) run on the tap-box kernel: a halo form with 64-channel output tiles
+  // and weights streamed per (tap, chunk) measured slower on B200 (DESIGN.md section 6)
+  if (Cin > 64 || Cout_pad > 64) return 1;
+  if (phs && (in_stride != 1 || phs->n < 2 || phs->n > 4)) return 1;
   // 33..64 input channels, narrow output: either ONE 64-channel chunk (128-byte rows; the resident weights then leave no room for
   // tap stacking: N = BN MMAs bound by the A-operand fetch) or TWO 32-channel chunks per box (64-byte rows, half-size stages, the
   // weights of both chunks resident) with tap stacking.  Both are planned, the better modelled one runs.
-  if (!phs && !wide && force_cblk == 0 && Cin > 32 && !(getenv("JVAE_CONV_KSPLIT") && atoi(getenv("JVAE_CONV_KSPLIT")) == 0)) {
+  if (!phs && force_cblk == 0 && Cin > 32) {
     HaloParams pa, pb;
     double sa = 0.0, sb = 0.0;
     const int ra = try_launch_halo(in, N, H, W, Cin, ld_in, wmat, Cout_pad, ldw, ntaps, tap_dy, tap_dx, in_stride, Hq, Wq, out, Ho, Wo,
-                                   Cout, ld_out, out_sy, out_sx, out_oy, out_ox, bias, act, stats, bn, nullptr, stream, nullptr, &pa, 64, &sa);
+                                   Cout, ld_out, out_sy, out_sx, out_oy, out_ox, bias, act, stats, stream, nullptr, &pa, 64, &sa);
     const int rb2 = try_launch_halo(in, N, H, W, Cin, ld_in, wmat, Cout_pad, ldw, ntaps, tap_dy, tap_dx, in_stride, Hq, Wq, out, Ho, Wo,
-                                    Cout, ld_out, out_sy, out_sx, out_oy, out_ox, bias, act, stats, bn, nullptr, stream, nullptr, &pb, 32, &sb);
+                                    Cout, ld_out, out_sy, out_sx, out_oy, out_ox, bias, act, stats, stream, nullptr, &pb, 32, &sb);
     if (ra < 0) return ra;
     const int pick = (rb2 == 0 && (ra != 0 || sb > 1.15 * sa)) ? 32 : 64;
     if (score_out) *score_out = pick == 32 ? sb : sa;
     return try_launch_halo(in, N, H, W, Cin, ld_in, wmat, Cout_pad, ldw, ntaps, tap_dy, tap_dx, in_stride, Hq, Wq, out, Ho, Wo, Cout,
-                           ld_out, out_sy, out_sx, out_oy, out_ox, bias, act, stats, bn, bn_fused, stream, nullptr, plan_out, pick, nullptr);
+                           ld_out, out_sy, out_sx, out_oy, out_ox, bias, act, stats, stream, nullptr, plan_out, pick, nullptr);
   }
   HaloParams p;
   memset(&p, 0, sizeof(p));
@@ -1196,9 +1102,9 @@ static int try_launch_halo(const void* in, int N, int H, int W, int Cin, int ld_
   const int ey = dymax - dymin, ex = dxmax - dxmin;
   if (ey > 16 || ex > 16) return 1;
   p.N = N; p.Hq = Hq; p.Wq = Wq; p.dymin = dymin; p.dxmin = dxmin;
-  p.Cblk = force_cblk ? force_cblk : cblk_of(Cin > 64 ? 64 : Cin); p.ntaps = ntaps;
+  p.Cblk = force_cblk ? force_cblk : cblk_of(Cin); p.ntaps = ntaps;
   p.nkc = (Cin + p.Cblk - 1) / p.Cblk;
-  p.BN = Cout_pad > 64 ? 64 : Cout_pad; p.n_tiles_n = Cout_pad / p.BN;
+  p.BN = Cout_pad; p.n_tiles_n = 1;
   const uint32_t rb = (uint32_t)p.Cblk * 2u;
   p.HWp = 8 + ex;
   p.RT = Hq <= 32 ? Hq : 32;
@@ -1206,8 +1112,8 @@ static int try_launch_halo(const void* in, int N, int H, int W, int Cin, int ld_
   p.w_tap_bytes = (uint32_t)p.BN * rb;
   const uint32_t budget = 200u * 1024u;
   const uint32_t stats_bytes = stats ? 2u * (uint32_t)Cout_pad * 8u : 0u;
-  const uint32_t w_res = (uint32_t)ntaps * p.w_tap_bytes * (uint32_t)(wide ? 1 : p.nkc);      // every chunk's weights resident
-  const bool ksplit = !wide && p.nkc > 1;
+  const uint32_t w_res = (uint32_t)ntaps * p.w_tap_bytes * (uint32_t)p.nkc;      // every chunk's weights resident
+  const bool ksplit = p.nkc > 1;
   const int ksteps = p.Cblk >> 4;
   // modelled cycles of one 128 x n x 16 MMA with both operands in shared memory (measured: profiles/r01_umma_rate_probe.txt):
   // the tensor pipe needs n / 2, the operand fetch (4 KB of A + 32 n bytes of B at 128 B / cycle) 32 + n / 4
@@ -1216,7 +1122,7 @@ static int try_launch_halo(const void* in, int N, int H, int W, int Cin, int ld_
   // ---- tap rectangles per parity plane (vertical stacking needs, for every tap column, a contiguous run of tap rows)
   struct Col { int pl, x, e_lo, e_hi; };
   std::vector<Col> cols;
-  bool stackable = !wide && getenv("JVAE_CONV_NOSTACK") == nullptr;
+  bool stackable = true;
   for (int t = 0; t < ntaps && stackable; ++t) {
     const int x = tex[t] - dxmin, e = tey[t] - dymin;
     Col* c = nullptr;
@@ -1319,7 +1225,6 @@ static int try_launch_halo(const void* in, int N, int H, int W, int Cin, int ld_
     if (G > 1 && (!stackable || G * p.BN > 256)) break;
     for (int resident = 1; resident >= 0; --resident) {
       if (G > 1 && !resident) continue;
-      if (wide && resident) continue;                      // wide layers stream their weights per (tap, chunk)
       if (ksplit && (G == 1 || !resident)) continue;       // two resident chunks: only the stacked form is built
       const uint32_t wb = resident ? w_res : 4u * p.w_tap_bytes;
       bool found = false;
@@ -1433,16 +1338,10 @@ static int try_launch_halo(const void* in, int N, int H, int W, int Cin, int ld_
   p.num_boxes = p.strips_x * p.blocks_y * p.blocks_n;
   p.Ho = Ho; p.Wo = Wo; p.Cout = Cout; p.ldc = ld_out;
   p.out_sy = out_sy; p.out_sx = out_sx; p.out_oy = out_oy; p.out_ox = out_ox;
-  p.act = act & 0xff; p.out_f32 = (act & JVAE_OUT_F32) ? 1 : 0;
+  p.act = act & 0xff;
   p.bias = bias; p.out = reinterpret_cast<__nv_bfloat16*>(out); p.stats = stats; p.cout_pad = Cout_pad;
   if (plan_out) { *plan_out = p; return JVAE_OK; }      // jvae_conv_halo_emulate: the plan only, nothing touches the device
   CUtensorMap tin, tw;
-  if (bn) {
-    p.bn_y = reinterpret_cast<const __nv_bfloat16*>(bn->y); p.bn_ld = bn->ld_y; p.bn_save = bn->save_mean_rstd;
-    p.bn_gamma = bn->gamma; p.bn_beta = bn->beta; p.bn_act = bn->act;
-    if ((bn->ld_y % 8) != 0) { set_error("jvae_conv_gather_gemm_bn: bn.ld_y must be a multiple of 8"); return JVAE_ERR_INVALID; }
-    if (!stats) { set_error("jvae_conv_gather_gemm_bn: the sums need the stats buffer"); return JVAE_ERR_INVALID; }
-  }
   {
     uint64_t dims[4] = {(uint64_t)Cin, (uint64_t)W, (uint64_t)H, (uint64_t)N};
     uint64_t strides[3] = {(uint64_t)ld_in * 2, (uint64_t)W * ld_in * 2, (uint64_t)H * W * ld_in * 2};
@@ -1460,8 +1359,7 @@ static int try_launch_halo(const void* in, int N, int H, int W, int Cin, int ld_
     if (rc) return rc;
   }
   const size_t tab_bytes = (size_t)p.MT * p.G * p.PH * 16 * sizeof(int2);       // block table of the fast epilogue
-  const size_t smem = (size_t)p.stages * p.stage_bytes + p.w_bytes + 512 + stats_bytes +
-                      256 + 1024 + 1024 + tab_bytes;
+  const size_t smem = (size_t)p.stages * p.stage_bytes + p.w_bytes + 512 + stats_bytes + 256 + 1024 + tab_bytes;
   if (smem > 227u * 1024u) return 1;
   static bool attr = false;
   if (!attr) {
@@ -1475,7 +1373,6 @@ static int try_launch_halo(const void* in, int N, int H, int W, int Cin, int ld_
   prof_end(prof, stream);
   JVAE_LAUNCH_CHECK();
   g_last_conv_kernel = JVAE_KERNEL_CONV_HALO;
-  if (bn && bn_fused) *bn_fused = 1;
   return JVAE_OK;
 }
 
@@ -1523,10 +1420,8 @@ static int try_launch_wgrad_halo(const void* g, int N, int Hq, int Wq, int Cg, i
   // Measured on B200 (tools/bench_layers.py, old form / stacked form): 32 -> 32 k5 at 32 x 32: 850 / 600 us; 256-channel k3 layers at
   // 8 x 8: 142 / 117 us; but 64-channel tiles on 16 x 16 and 32 x 32 maps and the 64 -> 64 k5 layer at 8 x 8 lose (a stacked B
   // fetch costs ~1.5x per MMA, so the form pays only when it removes most of the MMAs): enabled for 32-channel gradient tiles
-  // with at least four tap rows, and for 3 x 3 windows on maps of at most 8 x 8 with >= 128 channels.  JVAE_WGRAD_VSTACK = 0 / 1
-  // forces it off / on.
-  bool want = (cblk_of(Cg > 64 ? 64 : Cg) == 32 && ey + 1 >= 4) || (ey + 1 == 3 && Hq * Wq <= 64 && Cg >= 128);
-  if (const char* e = getenv("JVAE_WGRAD_VSTACK")) want = atoi(e) != 0;
+  // with at least four tap rows, and for 3 x 3 windows on maps of at most 8 x 8 with >= 128 channels.
+  const bool want = (cblk_of(Cg > 64 ? 64 : Cg) == 32 && ey + 1 >= 4) || (ey + 1 == 3 && Hq * Wq <= 64 && Cg >= 128);
   bool full = want && st == 1 && p.nplanes == 1 && ntaps == (ey + 1) * (ex + 1);
   for (int t = 0; t < ntaps && full; ++t) {
     int& slot = tap_at[(size_t)(tey[t] - dymin) * (ex + 1) + (tex[t] - dxmin)];
@@ -1538,8 +1433,7 @@ static int try_launch_wgrad_halo(const void* g, int N, int Hq, int Wq, int Cg, i
   const uint32_t gslot16 = (8u * rbg) >> 4;               // one slot of the gradient tile (8 pixels), 16-byte units
   const int E = ey;
   if (full) {
-    int nvmax = min(ey + 1, 256 / p.Cblk_g);
-    if (const char* e = getenv("JVAE_WGRAD_NVMAX")) nvmax = max(1, min(nvmax, atoi(e)));
+    const int nvmax = min(ey + 1, 256 / p.Cblk_g);
     const int nsets = (ey + 1 + nvmax - 1) / nvmax;
     for (int x0 = 0; x0 <= ex; x0 += min(tpm, 8)) {
       const int n = min(min(tpm, 8), ex + 1 - x0);
@@ -1755,17 +1649,7 @@ int jvae_conv_gather_gemm(const void* in, int N, int H, int W, int Cin, int ld_i
                           int ntaps, const int16_t* tap_dy, const int16_t* tap_dx, int in_stride, int Hq, int Wq,
                           void* out, int Ho, int Wo, int Cout, int ld_out, int out_sy, int out_sx, int out_oy, int out_ox,
                           const float* bias, int act, double* stats, void* stream) {
-  return jvae_conv_gather_gemm_bn(in, N, H, W, Cin, ld_in, wmat, Cout_pad, ldw, ntaps, tap_dy, tap_dx, in_stride, Hq, Wq, out, Ho,
-                                  Wo, Cout, ld_out, out_sy, out_sx, out_oy, out_ox, bias, act, stats, nullptr, nullptr, stream);
-}
-
-int jvae_conv_gather_gemm_bn(const void* in, int N, int H, int W, int Cin, int ld_in, const void* wmat, int Cout_pad, int ldw,
-                             int ntaps, const int16_t* tap_dy, const int16_t* tap_dx, int in_stride, int Hq, int Wq,
-                             void* out, int Ho, int Wo, int Cout, int ld_out, int out_sy, int out_sx, int out_oy, int out_ox,
-                             const float* bias, int act, double* stats, const jvae_bn_reduce* bn, int* bn_fused, void* stream) {
   JVAE_CHECK_ARG(in && wmat && out && tap_dy && tap_dx, "null pointer");
-  JVAE_CHECK_ARG(!bn || (bn->y && bn->save_mean_rstd && stats && bn->ld_y >= Cout), "bn reduce needs y, save_mean_rstd and the sums buffer");
-  if (bn_fused) *bn_fused = 0;
   JVAE_CHECK_ARG(ntaps >= 1 && ntaps <= CONV_MAX_TAPS, "1..64 taps");
   JVAE_CHECK_ARG((ld_in % 8) == 0 && (ldw % 8) == 0, "input / weight channel strides must be multiples of 8");
   JVAE_CHECK_ARG(ld_out >= Cout, "ld_out < Cout");
@@ -1773,14 +1657,9 @@ int jvae_conv_gather_gemm_bn(const void* in, int N, int H, int W, int Cin, int l
   JVAE_CHECK_ARG(!stats || Cout_pad <= 2048, "statistics epilogue supports up to 2048 channels");
   JVAE_CHECK_ARG(in_stride == 1 || in_stride == 2, "input stride 1 or 2");
   JVAE_CHECK_ARG((((uintptr_t)in | (uintptr_t)wmat | (uintptr_t)out) & 15) == 0, "16-byte alignment");
-  static const bool force_v1 = getenv("JVAE_CONV_V1") != nullptr;
-  if (!force_v1) {
-    const int rc = try_launch_halo(in, N, H, W, Cin, ld_in, wmat, Cout_pad, ldw, ntaps, tap_dy, tap_dx, in_stride, Hq, Wq, out,
-                                   Ho, Wo, Cout, ld_out, out_sy, out_sx, out_oy, out_ox, bias, act, stats, bn, bn_fused,
-                                   (cudaStream_t)stream);
-    if (rc <= 0) return rc;      // launched (0) or failed (< 0); 1 = geometry not covered, use the tap-box kernel
-  }
-  if (bn) stats = nullptr;       // the tap-box kernel has no fused BatchNorm-backward reduction: the caller runs jvae_bn_bwd
+  int rc = try_launch_halo(in, N, H, W, Cin, ld_in, wmat, Cout_pad, ldw, ntaps, tap_dy, tap_dx, in_stride, Hq, Wq, out, Ho, Wo,
+                           Cout, ld_out, out_sy, out_sx, out_oy, out_ox, bias, act, stats, (cudaStream_t)stream);
+  if (rc <= 0) return rc;      // launched (0) or failed (< 0); 1 = geometry not covered, use the tap-box kernel
   ConvParams p;
   memset(&p, 0, sizeof(p));
   p.N = N; p.Hq = Hq; p.Wq = Wq;
@@ -1789,15 +1668,14 @@ int jvae_conv_gather_gemm_bn(const void* in, int N, int H, int W, int Cin, int l
   p.BN = Cout_pad > 256 ? 256 : Cout_pad;
   if (Cout_pad > 256) JVAE_CHECK_ARG((Cout_pad % 256) == 0, "Cout_pad > 256 must be a multiple of 256");
   // small maps (vgg19's 512-channel layers at 2x2: 16 pixel tiles): narrower channel tiles until the CTAs cover the SMs
-  static const bool narrow = !(getenv("JVAE_CONV_NARROW") && atoi(getenv("JVAE_CONV_NARROW")) == 0);
-  while (narrow && p.BN > 64 && (p.BN % 32) == 0 && 2 * p.tiles_x * p.tiles_y * p.tiles_n * (Cout_pad / p.BN) <= sm_count()) p.BN /= 2;
+  while (p.BN > 64 && (p.BN % 32) == 0 && 2 * p.tiles_x * p.tiles_y * p.tiles_n * (Cout_pad / p.BN) <= sm_count()) p.BN /= 2;
   p.n_tiles_n = Cout_pad / p.BN;
   p.num_tiles = p.tiles_x * p.tiles_y * p.tiles_n * p.n_tiles_n;
   p.Cblk = cblk_of(Cin); p.nCk = (Cin + p.Cblk - 1) / p.Cblk; p.ntaps = ntaps; p.in_stride = in_stride;
   for (int t = 0; t < ntaps; ++t) { p.dy[t] = tap_dy[t]; p.dx[t] = tap_dx[t]; }
   p.Ho = Ho; p.Wo = Wo; p.Cout = Cout; p.ldc = ld_out;
   p.out_sy = out_sy; p.out_sx = out_sx; p.out_oy = out_oy; p.out_ox = out_ox;
-  p.act = act & 0xff; p.out_f32 = (act & JVAE_OUT_F32) ? 1 : 0;
+  p.act = act & 0xff;
   p.bias = bias; p.out = reinterpret_cast<__nv_bfloat16*>(out);
   p.stats = stats; p.cout_pad = Cout_pad;
   const uint32_t stats_bytes = stats ? 2u * (uint32_t)Cout_pad * 8u : 0u;
@@ -1809,7 +1687,7 @@ int jvae_conv_gather_gemm_bn(const void* in, int N, int H, int W, int Cin, int l
   JVAE_CHECK_ARG(p.stages >= 2, "tile too large for shared memory");
   p.tmem_cols = (uint32_t)pow2_ceil(2 * p.BN < 32 ? 32 : 2 * p.BN);
   CUtensorMap tin, tw;
-  int rc = act_tmap(&tin, in, N, H, W, Cin, ld_in, p.Cblk, p.TW, p.TH, p.NB, in_stride);
+  rc = act_tmap(&tin, in, N, H, W, Cin, ld_in, p.Cblk, p.TW, p.TH, p.NB, in_stride);
   if (rc) return rc;
   {
     const int Ktot = ntaps * p.nCk * p.Cblk;
@@ -1854,11 +1732,9 @@ int jvae_conv_subpixel_gemm(const void* in, int N, int H, int W, int Cin, int ld
   JVAE_CHECK_ARG((Cout_pad % 16) == 0 && Cout_pad >= 16 && Cout_pad >= Cout, "Cout_pad must be a multiple of 16, >= Cout");
   JVAE_CHECK_ARG((((uintptr_t)in | (uintptr_t)wmat | (uintptr_t)out) & 15) == 0, "16-byte alignment");
   JVAE_CHECK_ARG(out_s >= 1 && (Hq - 1) * out_s + out_s <= Ho && (Wq - 1) * out_s + out_s <= Wo, "phase grid larger than the output");
-  static const bool off = (getenv("JVAE_CONV_V1") != nullptr) || (getenv("JVAE_CONV_MERGE_PHASES") && atoi(getenv("JVAE_CONV_MERGE_PHASES")) == 0);
-  if (off) return JVAE_NOT_COVERED;
   PhaseSpec ps = {nphases, phase_ntaps, phase_oy, phase_ox};
   const int rc = try_launch_halo(in, N, H, W, Cin, ld_in, wmat, Cout_pad, ldw, ntaps, tap_dy, tap_dx, 1, Hq, Wq, out, Ho, Wo, Cout,
-                                 ld_out, out_s, out_s, 0, 0, bias, act, stats, nullptr, nullptr, (cudaStream_t)stream, &ps);
+                                 ld_out, out_s, out_s, 0, 0, bias, act, stats, (cudaStream_t)stream, &ps);
   return rc > 0 ? JVAE_NOT_COVERED : rc;
 }
 
@@ -1869,34 +1745,30 @@ int jvae_conv_wgrad(const void* dy, int N, int Hq, int Wq, int Cout, int ld_dy, 
   JVAE_CHECK_ARG(ntaps >= 1 && ntaps <= CONV_MAX_TAPS, "1..64 taps");
   JVAE_CHECK_ARG((ld_dy % 8) == 0 && (ld_x % 8) == 0, "channel strides must be multiples of 8");
   JVAE_CHECK_ARG(in_stride == 1 || in_stride == 2, "input stride 1 or 2");
-  static const bool force_v1 = getenv("JVAE_CONV_V1") != nullptr;
-  if (!force_v1) {
-    const int rc = try_launch_wgrad_halo(dy, N, Hq, Wq, Cout, ld_dy, x, H, W, Cin, ld_x, ntaps, tap_dy, tap_dx, in_stride, dw,
-                                         dw_ld_tap, dw_ld_co, dw_ld_ci, (cudaStream_t)stream);
-    if (rc <= 0) return rc;
-    // Stride 2 with wide rows (the 64-channel stride-2 layers): the four parity planes of the gathered tensor do not fit one
-    // stage together, but each plane alone does -- one launch per plane with that plane's taps (a tap belongs to exactly one
-    // plane, so the launches add into disjoint slices of dW).  Tap-box kernel before: 375 us for the 8 -> 16 layer of c2.
-    static const bool split_off = getenv("JVAE_WGRAD_PLANE_SPLIT") && atoi(getenv("JVAE_WGRAD_PLANE_SPLIT")) == 0;
-    if (in_stride == 2 && !split_off) {
-      std::vector<int16_t> sdy[4], sdx[4];
-      std::vector<int> ids[4];
-      for (int t = 0; t < ntaps; ++t) {
-        const int pl = (((tap_dy[t] % 2) + 2) % 2) * 2 + (((tap_dx[t] % 2) + 2) % 2);
-        sdy[pl].push_back(tap_dy[t]); sdx[pl].push_back(tap_dx[t]); ids[pl].push_back(t);
-      }
-      bool covered = true;
-      for (int pass = 0; pass < 2 && covered; ++pass)      // first pass: plans only, so that either every plane launches or none
-        for (int pl = 0; pl < 4; ++pl) {
-          if (ids[pl].empty()) continue;
-          const int r2 = try_launch_wgrad_halo(dy, N, Hq, Wq, Cout, ld_dy, x, H, W, Cin, ld_x, (int)ids[pl].size(), sdy[pl].data(),
-                                               sdx[pl].data(), 2, dw, dw_ld_tap, dw_ld_co, dw_ld_ci, (cudaStream_t)stream,
-                                               ids[pl].data(), pass == 0);
-          if (r2 < 0) return r2;
-          if (r2 > 0) { covered = false; break; }
-        }
-      if (covered) return JVAE_OK;
+  int rc = try_launch_wgrad_halo(dy, N, Hq, Wq, Cout, ld_dy, x, H, W, Cin, ld_x, ntaps, tap_dy, tap_dx, in_stride, dw,
+                                 dw_ld_tap, dw_ld_co, dw_ld_ci, (cudaStream_t)stream);
+  if (rc <= 0) return rc;
+  // Stride 2 with wide rows (the 64-channel stride-2 layers): the four parity planes of the gathered tensor do not fit one
+  // stage together, but each plane alone does -- one launch per plane with that plane's taps (a tap belongs to exactly one
+  // plane, so the launches add into disjoint slices of dW).  Tap-box kernel before: 375 us for the 8 -> 16 layer of c2.
+  if (in_stride == 2) {
+    std::vector<int16_t> sdy[4], sdx[4];
+    std::vector<int> ids[4];
+    for (int t = 0; t < ntaps; ++t) {
+      const int pl = (((tap_dy[t] % 2) + 2) % 2) * 2 + (((tap_dx[t] % 2) + 2) % 2);
+      sdy[pl].push_back(tap_dy[t]); sdx[pl].push_back(tap_dx[t]); ids[pl].push_back(t);
     }
+    bool covered = true;
+    for (int pass = 0; pass < 2 && covered; ++pass)      // first pass: plans only, so that either every plane launches or none
+      for (int pl = 0; pl < 4; ++pl) {
+        if (ids[pl].empty()) continue;
+        const int r2 = try_launch_wgrad_halo(dy, N, Hq, Wq, Cout, ld_dy, x, H, W, Cin, ld_x, (int)ids[pl].size(), sdy[pl].data(),
+                                             sdx[pl].data(), 2, dw, dw_ld_tap, dw_ld_co, dw_ld_ci, (cudaStream_t)stream,
+                                             ids[pl].data(), pass == 0);
+        if (r2 < 0) return r2;
+        if (r2 > 0) { covered = false; break; }
+      }
+    if (covered) return JVAE_OK;
   }
   WgradParams p;
   memset(&p, 0, sizeof(p));
@@ -1935,7 +1807,7 @@ int jvae_conv_wgrad(const void* dy, int N, int Hq, int Wq, int Cout, int ld_dy, 
   int gx = (2 * sm_count() + tap_groups * nz - 1) / (tap_groups * nz);
   if (gx < 1) gx = 1;
   if (gx > p.num_tiles) gx = p.num_tiles;
-  int rc = act_tmap(&tdy, dy, N, Hq, Wq, Cout, ld_dy, p.Cblk_y, p.TW, p.TH, p.NB, 1);
+  rc = act_tmap(&tdy, dy, N, Hq, Wq, Cout, ld_dy, p.Cblk_y, p.TW, p.TH, p.NB, 1);
   if (rc) return rc;
   rc = act_tmap(&tx, x, N, H, W, Cin, ld_x, p.Cblk_x, p.TW, p.TH, p.NB, in_stride);
   if (rc) return rc;
@@ -2010,7 +1882,7 @@ int jvae_conv_halo_emulate(const float* in, int N, int H, int W, int Cin, int ld
   HaloParams p;
   PhaseSpec ps = {nphases, phase_ntaps, phase_oy, phase_ox};
   const int rc = try_launch_halo(in, N, H, W, Cin, ld_in, wmat, Cout_pad, ldw, ntaps, tap_dy, tap_dx, in_stride, Hq, Wq, out, Ho, Wo,
-                                 Cout, ld_out, out_sy, out_sx, out_oy, out_ox, bias, act, nullptr, nullptr, nullptr, nullptr,
+                                 Cout, ld_out, out_sy, out_sx, out_oy, out_ox, bias, act, nullptr, nullptr,
                                  nphases > 0 ? &ps : nullptr, &p);
   if (rc != 0) return rc > 0 ? JVAE_NOT_COVERED : rc;
   if (info) { info[0] = p.G; info[1] = p.PH; info[2] = p.MT; info[3] = p.NBt; info[4] = p.BN; info[5] = p.nck; info[6] = p.resident; info[7] = p.stages; }
@@ -2382,13 +2254,11 @@ int conv_selftest(int verbose) {
     fails += conv_case(c, verbose);
     if (fails > 4) { printf("[selftest] conv: too many failures, stopping\n"); break; }
   }
-  if (!(getenv("JVAE_CONV_V1") || (getenv("JVAE_CONV_MERGE_PHASES") && atoi(getenv("JVAE_CONV_MERGE_PHASES")) == 0))) {
-    fails += subpixel_case(5, 16, 16, 32, 32, 5, 2, 0, verbose);      // c2 imager 16 -> 32: one image per box, 4 x 32 columns
-    fails += subpixel_case(7, 8, 8, 64, 64, 5, 2, 0, verbose);        // c2 imager 8 -> 16: channel tile halved, 3 images per box
-    fails += subpixel_case(3, 16, 16, 32, 16, 4, 1, 1, verbose);      // k = 4 (two taps per axis and phase), relu
-    fails += subpixel_case(2, 40, 24, 16, 24, 3, 1, 0, verbose);      // two row blocks per image, ragged channel count
-    fails += subpixel_case(150, 8, 8, 16, 16, 5, 2, 0, verbose);      // more boxes than SMs
-  }
+  fails += subpixel_case(5, 16, 16, 32, 32, 5, 2, 0, verbose);      // c2 imager 16 -> 32: one image per box, 4 x 32 columns
+  fails += subpixel_case(7, 8, 8, 64, 64, 5, 2, 0, verbose);        // c2 imager 8 -> 16: channel tile halved, 3 images per box
+  fails += subpixel_case(3, 16, 16, 32, 16, 4, 1, 1, verbose);      // k = 4 (two taps per axis and phase), relu
+  fails += subpixel_case(2, 40, 24, 16, 24, 3, 1, 0, verbose);      // two row blocks per image, ragged channel count
+  fails += subpixel_case(150, 8, 8, 16, 16, 5, 2, 0, verbose);      // more boxes than SMs
   return fails;
 }
 }  // namespace jvae

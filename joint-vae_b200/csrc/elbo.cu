@@ -12,7 +12,6 @@
 // exactly once.
 #include "tc_common.cuh"
 #include <math_constants.h>
-#include <stdlib.h>
 
 namespace jvae {
 
@@ -67,23 +66,16 @@ struct ElboArgs {
   const float* cross;
   const float* mnorm;       // (Cp) ||m_c||^2
   int cross_ld;
-  // TMA-staged train forward
-  int tma_lg, tma_stages;
-  unsigned int tma_stage_bytes;
 };
 
 struct WsLayout {
   size_t counters, dnv, zero_bytes, mse, dict_mean, logdet, lat, ce, tdiag, full_dist, tc_a, tc_b, tc_cross, tc_mnorm, total;
   int tc_ld, tc_cpad;
 };
-// classes from which the eval kernel takes its distances from the tensor-core cross-term GEMM (JVAE_ELBO_TC_MINC overrides)
-static int tc_min_classes() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("JVAE_ELBO_TC_MINC"); v = e ? atoi(e) : 32; if (v < 1) v = 1; }
-  return v;
-}
+// classes from which the eval kernel takes its distances from the tensor-core cross-term GEMM
+constexpr int ELBO_TC_MIN_CLASSES = 32;
 static bool tc_eligible(int K, int Cp, int var_dim, int prior_kind, int conditional) {
-  return conditional && var_dim == JVAE_VAR_SCALAR && prior_kind == JVAE_PRIOR_GAUSSIAN && (K % 8) == 0 && Cp >= tc_min_classes();
+  return conditional && var_dim == JVAE_VAR_SCALAR && prior_kind == JVAE_PRIOR_GAUSSIAN && (K % 8) == 0 && Cp >= ELBO_TC_MIN_CLASSES;
 }
 static inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 static WsLayout ws_layout(int B, int L, int K, int Cp, bool full = false, bool tc = false) {
@@ -725,136 +717,6 @@ __global__ void __launch_bounds__(ELBO_THREADS, MINB) elbo_train_fwd_v2_kernel(E
       a.counters[b] = 0;
       train_finalize(a, b);
     }
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// TMA-staged persistent variant of the train forward (opt-in, JVAE_ELBO_TMA=1; rows must be 16-byte aligned): one CTA per SM;
-// a producer thread streams work items (sample b, group of tma_lg draws) = the x row + tma_lg x_reco rows as 1-D bulk
-// copies into a ring of shared-memory stages (up to ~180 KB in flight per SM, full-row DRAM bursts); 12 consumer warps
-// reduce sum (x_reco - x)^2 out of shared memory.  Per item the warp partials meet in shared memory and the LAST warp
-// adds them in a fixed order (deterministic), publishes ws_mse and counts the sample's arrival; the latent warps run
-// first, while the pipeline fills.  No CTA waves, no tail of half-empty SMs.
-// ------------------------------------------------------------------------------------------------
-constexpr int ELBO_TMA_CWARPS = 12;
-constexpr int ELBO_TMA_FWARPS = 8;                               // finisher warps: one global round trip each in flight
-constexpr int ELBO_TMA_LWARPS = 4;                               // latent warps (one sample at a time each)
-constexpr int ELBO_TMA_THREADS = (ELBO_TMA_CWARPS + 1 + ELBO_TMA_LWARPS + ELBO_TMA_FWARPS) * 32;
-constexpr int ELBO_TMA_MAXLG = 4;
-
-template <bool XR_BF16>
-__global__ void __launch_bounds__(ELBO_TMA_THREADS, 1) elbo_train_fwd_tma_kernel(ElboArgs a) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 127) & ~(uintptr_t)127);
-  __shared__ uint64_t full_bar[8], empty_bar[8], pfull_bar[8];
-  __shared__ float s_part[8][ELBO_TMA_CWARPS][ELBO_TMA_MAXLG];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int LG = a.tma_lg, G = a.G, D = a.D;
-  const int nitems = a.B * G;
-  const uint32_t x_bytes = (uint32_t)D * 4u, r_bytes = (uint32_t)D * (XR_BF16 ? 2u : 4u);
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < a.tma_stages; ++s) {
-      mbar_init(&full_bar[s], 1);
-      mbar_init(&empty_bar[s], ELBO_TMA_CWARPS + 1);     // 12 consumer warps + the finisher lane that read the partials
-      mbar_init(&pfull_bar[s], ELBO_TMA_CWARPS);
-    }
-    fence_barrier_init();
-    fence_proxy_async();
-  }
-  __syncthreads();
-  if (warp == ELBO_TMA_CWARPS) {
-    // ---------------- producer: one thread streams the work items into the stage ring
-    if (lane == 0) {
-      uint32_t s = 0, ph = 0;
-      for (int item = blockIdx.x; item < nitems; item += gridDim.x) {
-        const int b = item / G, g = item - b * G;
-        const int l0 = 1 + g * LG, nl = min(LG, a.L + 1 - l0);
-        mbar_wait(&empty_bar[s], ph ^ 1);
-        uint8_t* st = smem + (size_t)s * a.tma_stage_bytes;
-        mbar_arrive_expect_tx(&full_bar[s], x_bytes + (uint32_t)nl * r_bytes);
-        tma_bulk_load(st, a.x + (size_t)b * D, x_bytes, &full_bar[s]);
-        const uint8_t* r0 = reinterpret_cast<const uint8_t*>(a.xr) + ((size_t)l0 * a.B + b) * r_bytes;
-        for (int j = 0; j < nl; ++j)
-          tma_bulk_load(st + x_bytes + (size_t)j * r_bytes, r0 + (size_t)j * a.B * r_bytes, r_bytes, &full_bar[s]);
-        if (++s == (uint32_t)a.tma_stages) { s = 0; ph ^= 1; }
-      }
-    }
-    return;
-  }
-  if (warp > ELBO_TMA_CWARPS && warp <= ELBO_TMA_CWARPS + ELBO_TMA_LWARPS) {
-    // ---------------- latent warps: KL / cross-entropy of this CTA's share of the samples, beside the stream
-    const int q = (int)blockIdx.x * ELBO_TMA_LWARPS + (warp - ELBO_TMA_CWARPS - 1);
-    for (int b = q; b < a.B; b += (int)gridDim.x * ELBO_TMA_LWARPS) train_latent_warp(a, b, lane);
-    return;
-  }
-  if (warp > ELBO_TMA_CWARPS + ELBO_TMA_LWARPS) {
-    // ---------------- finisher warps: warp f owns STAGE f (every use of it, in order, so its phase parity never runs
-    // ahead): adds the 12 warp partials in a fixed order, publishes ws_mse and counts the sample's arrival with ONE
-    // acq_rel atomic (a single global round trip per item; one per stage in flight), then finalises the sample if it
-    // was the last arrival
-    const int f = warp - (ELBO_TMA_CWARPS + 1 + ELBO_TMA_LWARPS);
-    if (lane != 0 || f >= a.tma_stages) return;
-    const int s = f;
-    uint32_t fph = 0;
-    for (int item = (int)blockIdx.x + f * (int)gridDim.x; item < nitems; item += a.tma_stages * (int)gridDim.x, fph ^= 1) {
-      const int b = item / G, g = item - b * G;
-      const int l0 = 1 + g * LG, nl = min(LG, a.L + 1 - l0);
-      mbar_wait(&pfull_bar[s], fph);
-      float t[ELBO_TMA_MAXLG];
-#pragma unroll
-      for (int j = 0; j < ELBO_TMA_MAXLG; ++j) {
-        t[j] = 0.f;
-#pragma unroll
-        for (int w = 0; w < ELBO_TMA_CWARPS; ++w) t[j] += reinterpret_cast<volatile float*>(&s_part[s][w][0])[j];
-      }
-      mbar_arrive(&empty_bar[s]);                 // partials are in registers: the stage may be refilled
-#pragma unroll
-      for (int j = 0; j < ELBO_TMA_MAXLG; ++j)
-        if (j < nl) a.ws_mse[(size_t)(l0 - 1 + j) * a.B + b] = t[j];
-      unsigned int gold;
-      asm volatile("atom.acq_rel.gpu.global.add.u32 %0, [%1], 1;" : "=r"(gold) : "l"(&a.counters[b]) : "memory");
-      if (gold == (unsigned int)G) {              // G streaming items + the latent warp: this one is last
-        a.counters[b] = 0;
-        train_finalize(a, b);
-      }
-    }
-    return;
-  }
-  // ---------------- consumers (12 warps)
-  const int ctid = threadIdx.x;                       // 0 .. 383
-  const int nvec = XR_BF16 ? (D >> 3) : (D >> 2);
-  uint32_t s = 0, ph = 0;
-  for (int item = blockIdx.x; item < nitems; item += gridDim.x) {
-    const int g = item % G;
-    const int l0 = 1 + g * LG, nl = min(LG, a.L + 1 - l0);
-    mbar_wait(&full_bar[s], ph);
-    const uint8_t* st = smem + (size_t)s * a.tma_stage_bytes;
-    float acc[ELBO_TMA_MAXLG];
-#pragma unroll
-    for (int j = 0; j < ELBO_TMA_MAXLG; ++j) acc[j] = 0.f;
-    for (int v = ctid; v < nvec; v += ELBO_TMA_CWARPS * 32) {
-      if (XR_BF16) {
-        const float4 x0 = reinterpret_cast<const float4*>(st)[2 * v], x1 = reinterpret_cast<const float4*>(st)[2 * v + 1];
-#pragma unroll
-        for (int j = 0; j < ELBO_TMA_MAXLG; ++j)
-          if (j < nl) sq_acc8(acc[j], x0, x1, reinterpret_cast<const uint4*>(st + x_bytes + (size_t)j * r_bytes)[v]);
-      } else {
-        const float4 x0 = reinterpret_cast<const float4*>(st)[v];
-#pragma unroll
-        for (int j = 0; j < ELBO_TMA_MAXLG; ++j)
-          if (j < nl) sq_acc4(acc[j], x0, reinterpret_cast<const uint4*>(st + x_bytes + (size_t)j * r_bytes)[v]);
-      }
-    }
-#pragma unroll
-    for (int j = 0; j < ELBO_TMA_MAXLG; ++j) acc[j] = warp_sum(acc[j]);
-    if (lane == 0) {
-#pragma unroll
-      for (int j = 0; j < ELBO_TMA_MAXLG; ++j) s_part[s][warp][j] = acc[j];
-      mbar_arrive(&pfull_bar[s]);                 // release: the finisher lane that waits on it sees the partials
-      mbar_arrive(&empty_bar[s]);
-    }
-    __syncwarp();
-    if (++s == (uint32_t)a.tma_stages) { s = 0; ph ^= 1; }
   }
 }
 
@@ -1568,23 +1430,15 @@ static int check_cfg(const jvae_elbo_cfg* cfg, const char* fn) {
   return JVAE_OK;
 }
 
-// latent draws streamed per CTA (1, 2, 4 or 8); JVAE_ELBO_LG overrides the default for tuning runs
-static int elbo_lg() {
-  static int lg = 0;
-  if (lg == 0) {
-    const char* e = getenv("JVAE_ELBO_LG");
-    int v = e ? atoi(e) : 4;
-    lg = (v == 1 || v == 2 || v == 4 || v == 8) ? v : 4;
-  }
-  return lg;
-}
+// latent draws streamed per CTA by the train forward / backward and eval kernels
+constexpr int ELBO_LG = 4;
 
 static void fill_args(ElboArgs& a, const jvae_elbo_cfg* cfg, void* workspace) {
   memset(&a, 0, sizeof(a));
   a.B = cfg->B; a.L = cfg->L; a.K = cfg->K; a.C = cfg->C; a.D = cfg->D;
   a.Cp = cfg->conditional ? cfg->C : 1;
   a.nkb = (cfg->K + 31) / 32;
-  a.G = cfg->has_xreco ? (cfg->L + elbo_lg() - 1) / elbo_lg() : 1;
+  a.G = cfg->has_xreco ? (cfg->L + ELBO_LG - 1) / ELBO_LG : 1;
   a.xr_bf16 = cfg->xreco_dtype == JVAE_BF16;
   a.lg_bf16 = cfg->logits_dtype == JVAE_BF16;
   a.var_dim = cfg->var_dim; a.prior_kind = cfg->prior_kind; a.conditional = cfg->conditional;
@@ -1695,56 +1549,14 @@ int jvae_elbo_train_fwd(const jvae_elbo_cfg* cfg, const float* x, const void* x_
     rc = categorical_prepass(a, st);
     if (rc) return rc;
   }
-  // TMA-staged persistent variant (JVAE_ELBO_TMA=1): measured on B200 at c2 it takes 19.7 us against 17.9 us for the
-  // many-CTA kernel below (both are bound by launch ramp + the arrival/finalise tail at 57 MB per launch, not by the
-  // stream), so it is opt-in; see DESIGN.md section 6
-  static const bool use_tma = getenv("JVAE_ELBO_TMA") != nullptr;
-  if (a.has_xreco && use_tma) {
-    const size_t esz = a.xr_bf16 ? 2 : 4;
-    const bool aligned = (((size_t)a.D * esz) % 16 == 0) && (((size_t)a.D * 4) % 16 == 0);
-    int lg = 0, stages = 0;
-    size_t stage = 0;
-    for (int cand : {4, 2, 1}) {
-      const size_t sb = (((size_t)a.D * 4 + (size_t)cand * a.D * esz) + 127) & ~(size_t)127;
-      const int st_ = (int)((200u * 1024u) / sb);
-      if (st_ >= 3 || (cand == 1 && st_ >= 2)) { lg = cand; stages = st_ > 8 ? 8 : st_; stage = sb; break; }
-    }
-    if (aligned && lg > 0) {
-      a.tma_lg = lg; a.tma_stages = stages; a.tma_stage_bytes = (unsigned int)stage;
-      a.G = (a.L + lg - 1) / lg;
-      const size_t smem = (size_t)stages * stage + 256;
-      const int nitems = a.B * a.G;
-      const int grid_t = nitems < sm_count() ? nitems : sm_count();
-      static bool attr = false;
-      if (!attr) {
-        JVAE_CUDA(cudaFuncSetAttribute(elbo_train_fwd_tma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-        JVAE_CUDA(cudaFuncSetAttribute(elbo_train_fwd_tma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-        attr = true;
-      }
-      if (a.xr_bf16) elbo_train_fwd_tma_kernel<true><<<grid_t, ELBO_TMA_THREADS, smem, st>>>(a);
-      else elbo_train_fwd_tma_kernel<false><<<grid_t, ELBO_TMA_THREADS, smem, st>>>(a);
-      JVAE_LAUNCH_CHECK();
-      return JVAE_OK;
-    }
-  }
-  // register-staged variant (bf16 reconstructions, vector-aligned rows); JVAE_ELBO_V2 = 0 disables, 1..5 picks the shape
-  static const int v2 = getenv("JVAE_ELBO_V2") ? atoi(getenv("JVAE_ELBO_V2")) : 1;
-  if (a.has_xreco && a.xr_bf16 && (a.D & 7) == 0 && v2 > 0) {
+  // register-staged variant (bf16 reconstructions, vector-aligned rows): 2 draws per CTA, 3 vector rounds in flight, 6 resident
+  // CTAs per SM, measured best at B = 512 and B = 2048 (tools/elbo_tune.py)
+  if (a.has_xreco && a.xr_bf16 && (a.D & 7) == 0) {
     const int nlat = (a.B + ELBO_THREADS / 32 - 1) / (ELBO_THREADS / 32);
-#define JVAE_ELBO_V2_LAUNCH(LG_, U_, MINB_)                                                   \
-    do {                                                                                      \
-      a.G = (a.L + LG_ - 1) / LG_;                                                            \
-      elbo_train_fwd_v2_kernel<LG_, U_, MINB_><<<nlat + a.B * a.G, ELBO_THREADS, 0, st>>>(a); \
-    } while (0)
+    constexpr int LG = 2, U = 3, MINB = 6;
+    a.G = (a.L + LG - 1) / LG;
     void* prof = prof_begin(JVAE_PROF_ELBO_TRAIN_FWD, st);
-    switch (v2) {
-      case 2: JVAE_ELBO_V2_LAUNCH(4, 3, 4); break;
-      case 3: JVAE_ELBO_V2_LAUNCH(4, 2, 6); break;
-      case 4: JVAE_ELBO_V2_LAUNCH(2, 2, 8); break;
-      case 5: JVAE_ELBO_V2_LAUNCH(1, 3, 7); break;
-      default: JVAE_ELBO_V2_LAUNCH(2, 3, 6); break;      // measured best at B = 512 and B = 2048 (tools/elbo_tune.py)
-    }
-#undef JVAE_ELBO_V2_LAUNCH
+    elbo_train_fwd_v2_kernel<LG, U, MINB><<<nlat + a.B * a.G, ELBO_THREADS, 0, st>>>(a);
     prof_end(prof, st);
     JVAE_LAUNCH_CHECK();
     return JVAE_OK;
@@ -1753,27 +1565,16 @@ int jvae_elbo_train_fwd(const jvae_elbo_cfg* cfg, const float* x, const void* x_
   int grid = (a.B + ELBO_THREADS / 32 - 1) / (ELBO_THREADS / 32);
   if (a.has_xreco) {
     const int items = a.B * a.G;
-    static const int wave_env = getenv("JVAE_ELBO_WAVE") ? atoi(getenv("JVAE_ELBO_WAVE")) : 12;   // resident CTAs per SM; 0: one CTA per item
-    const int wave = wave_env * sm_count() - grid;
+    const int wave = 12 * sm_count() - grid;      // 12 resident CTAs per SM
     // between one and two waves (c2: 2048 items, 1648 slots) a partial second wave costs ~1.2 us of a 17 us launch: two items
     // per CTA instead.  With several waves the hardware scheduler's refill beats a static split (measured at B = 2048).
-    const int per_cta = (wave_env > 0 && wave > 0 && items > wave && items <= 2 * wave) ? 2 : 1;
+    const int per_cta = (wave > 0 && items > wave && items <= 2 * wave) ? 2 : 1;
     grid += (items + per_cta - 1) / per_cta;
   }
-#define JVAE_ELBO_LAUNCH(kern, smem_)                                                              \
-  do {                                                                                           \
-    const int lg_ = elbo_lg();                                                                   \
-    if (a.xr_bf16) {                                                                             \
-      if (lg_ == 1) kern<true, 1><<<grid, ELBO_THREADS, smem_, st>>>(a);                         \
-      else if (lg_ == 2) kern<true, 2><<<grid, ELBO_THREADS, smem_, st>>>(a);                    \
-      else if (lg_ == 4) kern<true, 4><<<grid, ELBO_THREADS, smem_, st>>>(a);                    \
-      else kern<true, 8><<<grid, ELBO_THREADS, smem_, st>>>(a);                                  \
-    } else {                                                                                     \
-      if (lg_ == 1) kern<false, 1><<<grid, ELBO_THREADS, smem_, st>>>(a);                        \
-      else if (lg_ == 2) kern<false, 2><<<grid, ELBO_THREADS, smem_, st>>>(a);                   \
-      else if (lg_ == 4) kern<false, 4><<<grid, ELBO_THREADS, smem_, st>>>(a);                   \
-      else kern<false, 8><<<grid, ELBO_THREADS, smem_, st>>>(a);                                 \
-    }                                                                                            \
+#define JVAE_ELBO_LAUNCH(kern, smem_)                                           \
+  do {                                                                        \
+    if (a.xr_bf16) kern<true, ELBO_LG><<<grid, ELBO_THREADS, smem_, st>>>(a);  \
+    else kern<false, ELBO_LG><<<grid, ELBO_THREADS, smem_, st>>>(a);           \
   } while (0)
   void* prof = prof_begin(JVAE_PROF_ELBO_TRAIN_FWD, st);
   JVAE_ELBO_LAUNCH(elbo_train_fwd_kernel, 0);
@@ -1911,10 +1712,8 @@ int jvae_elbo_eval_fwd(const jvae_elbo_cfg* cfg, const float* x, const void* x_r
   }
   const int grid = a.B * a.G;
   if (smem > 48 * 1024) {
-#define JVAE_EVAL_ATTR(bf, lg) JVAE_CUDA(cudaFuncSetAttribute(elbo_eval_fwd_kernel<bf, lg>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem))
-    JVAE_EVAL_ATTR(true, 1); JVAE_EVAL_ATTR(true, 2); JVAE_EVAL_ATTR(true, 4); JVAE_EVAL_ATTR(true, 8);
-    JVAE_EVAL_ATTR(false, 1); JVAE_EVAL_ATTR(false, 2); JVAE_EVAL_ATTR(false, 4); JVAE_EVAL_ATTR(false, 8);
-#undef JVAE_EVAL_ATTR
+    JVAE_CUDA(cudaFuncSetAttribute(elbo_eval_fwd_kernel<true, ELBO_LG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    JVAE_CUDA(cudaFuncSetAttribute(elbo_eval_fwd_kernel<false, ELBO_LG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   }
   JVAE_ELBO_LAUNCH(elbo_eval_fwd_kernel, smem);
   prof_end(prof, st);

@@ -803,82 +803,13 @@ __global__ void __launch_bounds__(NORM_MAX_THREADS) add_act_kernel(const __nv_bf
 }
 
 // ------------------------------------------------------------------------------------------------ separable narrow-output convolution
-// A k x k convolution with few output channels (the image head 32 -> 3, k5: k * Co = 15 <= 16) is run as a 1 x k convolution
-// to k * Co channels, T[r][(ty, co)] = sum_tx sum_ci x[r + (0, tx - p)][ci] W[co][ci][ty][tx] (tensor cores, k taps instead of
-// k^2), followed by this vertical shift-and-add:  out[q][co] = bias[co] + sum_ty T[q + (ty - p, 0)][ty * Co + co].
-// One thread per output pixel; optional activation; optional BatchNorm statistics (sum, sum of squares of the pre-activation).
-constexpr int VS_MAXC = 16;
+// The backward of a k x k convolution with few output channels (the image head 32 -> 3, k5: k * Co = 15 <= 16) runs as the
+// backward of a 1 x k convolution to k * Co channels, T[r][(ty, co)] = sum_tx sum_ci x[r + (0, tx - p)][ci] W[co][ci][ty][tx]
+// (tensor cores, k taps instead of k^2), whose vertical shift-and-add out[q][co] = sum_ty T[q + (ty - p, 0)][ty * Co + co] is
+// the layer's output.  The kernels below are the adjoint of that sum: the gradient of T from the gradient of the output.
 
-__device__ __forceinline__ float bf16_pick(const uint32_t (&w)[8], int ch) {      // ch is a compile-time constant after unrolling
-  return (ch & 1) ? bf16_hi(w[ch >> 1]) : bf16_lo(w[ch >> 1]);
-}
-
-// compile-time (k, Co) with the vector layouts (T / U rows of 16 channels, dy / out rows of 8): every channel pick is a fixed
-// register, the kernels stream at memory speed.  KK * CO <= 16.
-template <int KK, int CO, bool TF>
-__global__ void __launch_bounds__(256) vsum_rows_fixed_kernel(const void* __restrict__ Tv, int N, int H, int W,
-                                                              const float* __restrict__ bias, int act, double* stats,
-                                                              __nv_bfloat16* __restrict__ out) {
-  __shared__ double s_st[2 * CO];
-  if (threadIdx.x < 2 * CO) s_st[threadIdx.x] = 0.0;
-  __syncthreads();
-  constexpr int PAD = (KK - 1) / 2;
-  const size_t P = (size_t)N * H * W;
-  float s1[CO], s2[CO], bv[CO];
-#pragma unroll
-  for (int c = 0; c < CO; ++c) { s1[c] = 0.f; s2[c] = 0.f; bv[c] = bias ? bias[c] : 0.f; }
-  for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < P; q += (size_t)gridDim.x * blockDim.x) {
-    const int y = (int)((q / W) % H);
-    float acc[CO];
-#pragma unroll
-    for (int c = 0; c < CO; ++c) acc[c] = bv[c];
-#pragma unroll
-    for (int ty = 0; ty < KK; ++ty) {
-      const int yy = y + ty - PAD;
-      if (yy < 0 || yy >= H) continue;
-      if constexpr (TF) {     // fp32 rows of 16 channels: the float4 vectors that hold channels [ty*CO, ty*CO + CO)
-        const float4* row = reinterpret_cast<const float4*>(reinterpret_cast<const float*>(Tv) + (q + (size_t)(ty - PAD) * W) * 16);
-        float f[16];
-#pragma unroll
-        for (int v4 = 0; v4 < 4; ++v4)
-          if (v4 * 4 < ty * CO + CO && v4 * 4 + 4 > ty * CO) {
-            const float4 t4 = row[v4];
-            f[v4 * 4] = t4.x; f[v4 * 4 + 1] = t4.y; f[v4 * 4 + 2] = t4.z; f[v4 * 4 + 3] = t4.w;
-          }
-#pragma unroll
-        for (int c = 0; c < CO; ++c) acc[c] += f[ty * CO + c];
-      } else {
-        const uint4* row = reinterpret_cast<const uint4*>(reinterpret_cast<const __nv_bfloat16*>(Tv) + (q + (size_t)(ty - PAD) * W) * 16);
-        // channels [ty*CO, ty*CO + CO) live in the first vector, the second, or straddle both
-        uint32_t w[8];
-        if (ty * CO < 8) { const uint4 lo = row[0]; w[0] = lo.x; w[1] = lo.y; w[2] = lo.z; w[3] = lo.w; }
-        if (ty * CO + CO > 8) { const uint4 hi = row[1]; w[4] = hi.x; w[5] = hi.y; w[6] = hi.z; w[7] = hi.w; }
-#pragma unroll
-        for (int c = 0; c < CO; ++c) acc[c] += bf16_pick(w, ty * CO + c);
-      }
-    }
-    float v[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-    for (int c = 0; c < CO; ++c) {
-      s1[c] += acc[c]; s2[c] = fmaf(acc[c], acc[c], s2[c]);
-      v[c] = act_fwd(acc[c], act);
-    }
-    uint4 o4;
-    o4.x = pack_bf16(v[0], v[1]); o4.y = pack_bf16(v[2], v[3]); o4.z = 0u; o4.w = 0u;
-    *reinterpret_cast<uint4*>(out + q * 8) = o4;
-  }
-  if (stats) {
-#pragma unroll
-    for (int c = 0; c < CO; ++c) {
-      float a = s1[c], b = s2[c];
-      for (int off = 16; off > 0; off >>= 1) { a += __shfl_xor_sync(0xffffffffu, a, off); b += __shfl_xor_sync(0xffffffffu, b, off); }
-      if ((threadIdx.x & 31) == 0) { atomicAdd(&s_st[c], (double)a); atomicAdd(&s_st[CO + c], (double)b); }
-    }
-    __syncthreads();
-    if (threadIdx.x < 2 * CO) atomicAdd(&stats[threadIdx.x], s_st[threadIdx.x]);
-  }
-}
-
+// compile-time (k, Co) with the vector layouts (U rows of 16 channels, dy rows of 8): every channel pick is a fixed register,
+// the kernel streams at memory speed.  KK * CO <= 16.
 template <int KK, int CO>
 __global__ void __launch_bounds__(256) vstack_rows_fixed_kernel(const __nv_bfloat16* __restrict__ dy, int N, int H, int W,
                                                                 __nv_bfloat16* __restrict__ U) {
@@ -903,80 +834,6 @@ __global__ void __launch_bounds__(256) vstack_rows_fixed_kernel(const __nv_bfloa
     b.x = pack_bf16(vals[8], vals[9]); b.y = pack_bf16(vals[10], vals[11]); b.z = pack_bf16(vals[12], vals[13]); b.w = pack_bf16(vals[14], vals[15]);
     uint4* u4 = reinterpret_cast<uint4*>(U + r * 16);
     u4[0] = a; u4[1] = b;
-  }
-}
-
-__global__ void __launch_bounds__(256) vsum_rows_kernel(const __nv_bfloat16* __restrict__ T, int ld_t, int N, int H, int W, int k, int p,
-                                                        int Co, const float* __restrict__ bias, int act, double* stats,
-                                                        __nv_bfloat16* __restrict__ out, int ld_out, int t_f32) {
-  __shared__ double s_st[2 * VS_MAXC];
-  if (threadIdx.x < 2 * VS_MAXC) s_st[threadIdx.x] = 0.0;
-  __syncthreads();
-  const size_t P = (size_t)N * H * W;
-  const bool vec = !t_f32 && ld_t == 16 && (reinterpret_cast<uintptr_t>(T) & 15) == 0;
-  const bool vec_out = ld_out == 8 && (reinterpret_cast<uintptr_t>(out) & 15) == 0;
-  float s1[4] = {0.f, 0.f, 0.f, 0.f}, s2[4] = {0.f, 0.f, 0.f, 0.f};      // statistics: Co <= 4 per thread registers
-  for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < P; q += (size_t)gridDim.x * blockDim.x) {
-    const int x = (int)(q % W), y = (int)((q / W) % H);
-    float acc[4] = {0.f, 0.f, 0.f, 0.f};
-    (void)x;
-    if (vec) {      // T rows are 16 channels = two 16-byte vectors; pick channels [ty * Co, ty * Co + Co) out of registers
-      for (int ty = 0; ty < k; ++ty) {
-        const int yy = y + ty - p;
-        if (yy < 0 || yy >= H) continue;
-        const uint4* row = reinterpret_cast<const uint4*>(T + (q + (size_t)(ty - p) * W) * 16);
-        const uint4 lo = row[0], hi = row[1];
-        const uint32_t w[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
-#pragma unroll
-        for (int c = 0; c < 4; ++c)
-          if (c < Co) {
-            const int ch = ty * Co + c;
-            uint32_t u = 0;
-#pragma unroll
-            for (int i = 0; i < 8; ++i) u = (ch >> 1) == i ? w[i] : u;
-            acc[c] += (ch & 1) ? bf16_hi(u) : bf16_lo(u);
-          }
-      }
-    } else {
-      for (int ty = 0; ty < k; ++ty) {
-        const int yy = y + ty - p;
-        if (yy < 0 || yy >= H) continue;
-        const size_t off = (q + (size_t)(ty - p) * W) * ld_t + ty * Co;
-#pragma unroll
-        for (int c = 0; c < 4; ++c)
-          if (c < Co) acc[c] += t_f32 ? reinterpret_cast<const float*>(T)[off + c] : __bfloat162float(T[off + c]);
-      }
-    }
-    float v[4];
-#pragma unroll
-    for (int c = 0; c < 4; ++c) {
-      v[c] = (c < Co) ? acc[c] + (bias ? bias[c] : 0.f) : 0.f;
-      if (c < Co) { s1[c] += v[c]; s2[c] = fmaf(v[c], v[c], s2[c]); }
-      v[c] = (c < Co) ? act_fwd(v[c], act) : 0.f;
-    }
-    if (vec_out) {      // 8-channel rows: one 16-byte store, padding channels zero
-      uint4 o4;
-      o4.x = pack_bf16(v[0], v[1]); o4.y = pack_bf16(v[2], v[3]); o4.z = 0u; o4.w = 0u;
-      *reinterpret_cast<uint4*>(out + q * 8) = o4;
-    } else {
-      __nv_bfloat16* o = out + q * ld_out;
-#pragma unroll
-      for (int c = 0; c < 4; ++c)
-        if (c < Co) o[c] = __float2bfloat16(v[c]);
-    }
-  }
-  if (stats) {
-#pragma unroll
-    for (int c = 0; c < 4; ++c) {
-      float a = s1[c], b = s2[c];
-      for (int off = 16; off > 0; off >>= 1) { a += __shfl_xor_sync(0xffffffffu, a, off); b += __shfl_xor_sync(0xffffffffu, b, off); }
-      if ((threadIdx.x & 31) == 0 && c < Co) { atomicAdd(&s_st[c], (double)a); atomicAdd(&s_st[VS_MAXC + c], (double)b); }
-    }
-    __syncthreads();
-    if (threadIdx.x < Co) {
-      atomicAdd(&stats[threadIdx.x], s_st[threadIdx.x]);
-      atomicAdd(&stats[Co + threadIdx.x], s_st[VS_MAXC + threadIdx.x]);
-    }
   }
 }
 
@@ -1139,7 +996,7 @@ int jvae_bn_apply_fwd(const void* y, size_t P, int C, int ld_y, const double* st
 
 int jvae_bn_bwd(const void* da, int ld_da, const void* y, int ld_y, size_t P, int C, const float* save_mean_rstd,
                 const float* gamma, const float* beta, int act, double* sums, void* dy, int ld_dy, float* dgamma, float* dbeta,
-                int skip_reduce, void* stream) {
+                void* stream) {
   JVAE_CHECK_ARG(da && y && dy && sums && save_mean_rstd && P > 0 && C > 0, "bad arguments");
   JVAE_CHECK_ARG(ld_da >= C && ld_y >= C && ld_dy >= C, "leading dimension < C");
   const bool vec = vec_ok(C, {ld_da, ld_y, ld_dy}, {da, y, dy});
@@ -1156,22 +1013,18 @@ int jvae_bn_bwd(const void* da, int ld_da, const void* y, int ld_y, size_t P, in
   if (narrow) {      // a thread per pixel (the image head's BatchNorm)
     const int want_r = (int)((P + NORM_MAX_THREADS * 4 - 1) / (NORM_MAX_THREADS * 4));
     const int want_a = (int)((P + NORM_MAX_THREADS * 2 - 1) / (NORM_MAX_THREADS * 2));
-    if (!skip_reduce) {
-      JVAE_CUDA(cudaMemsetAsync(sums, 0, 2 * (size_t)C * sizeof(double), (cudaStream_t)stream));
-      const int cap = sm_count() * BN_REDUCE_BLOCKS;
-      bn_bwd_reduce_narrow_kernel<<<want_r < cap ? (want_r ? want_r : 1) : cap, NORM_MAX_THREADS, 0, (cudaStream_t)stream>>>(a);
-      JVAE_LAUNCH_CHECK();
-    }
+    JVAE_CUDA(cudaMemsetAsync(sums, 0, 2 * (size_t)C * sizeof(double), (cudaStream_t)stream));
+    const int cap_r = sm_count() * BN_REDUCE_BLOCKS;
+    bn_bwd_reduce_narrow_kernel<<<want_r < cap_r ? (want_r ? want_r : 1) : cap_r, NORM_MAX_THREADS, 0, (cudaStream_t)stream>>>(a);
+    JVAE_LAUNCH_CHECK();
     const int cap = sm_count() * 8;
     bn_bwd_apply_narrow_kernel<<<want_a < cap ? (want_a ? want_a : 1) : cap, NORM_MAX_THREADS, 0, (cudaStream_t)stream>>>(a);
     JVAE_LAUNCH_CHECK();
     return JVAE_OK;
   }
-  if (!skip_reduce) {
-    JVAE_CUDA(cudaMemsetAsync(sums, 0, 2 * (size_t)C * sizeof(double), (cudaStream_t)stream));
-    const Geo gr = make_geo(P, C, vec ? 8 : 1, BN_REDUCE_BLOCKS);     // one resident wave: the per-block reduction tail runs once
-    NORM_DISPATCH(vec, bn_bwd_reduce_kernel, gr, 2 * C * sizeof(double), (cudaStream_t)stream, a);
-  }
+  JVAE_CUDA(cudaMemsetAsync(sums, 0, 2 * (size_t)C * sizeof(double), (cudaStream_t)stream));
+  const Geo gr = make_geo(P, C, vec ? 8 : 1, BN_REDUCE_BLOCKS);     // one resident wave: the per-block reduction tail runs once
+  NORM_DISPATCH(vec, bn_bwd_reduce_kernel, gr, 2 * C * sizeof(double), (cudaStream_t)stream, a);
   NORM_DISPATCH(vec, bn_bwd_apply_kernel, g, 0, (cudaStream_t)stream, a);
   return JVAE_OK;
 }
@@ -1321,34 +1174,6 @@ int jvae_avgpool(const void* src, int ld_src, void* dst, int ld_dst, int N, int 
   const Geo g = make_geo(Ps, C, vec ? 8 : 1);
   NORM_DISPATCH(vec, avgpool_kernel, g, 0, (cudaStream_t)stream, reinterpret_cast<const __nv_bfloat16*>(src), ld_src,
                 reinterpret_cast<__nv_bfloat16*>(dst), ld_dst, H, W, k, Ps, g.nchunk, g.ppb, backward);
-  return JVAE_OK;
-}
-
-int jvae_vsum_rows(const void* T, int ld_t, int N, int H, int W, int k, int pad, int Co, const float* bias, int act, double* stats,
-                   void* out, int ld_out, void* stream) {
-  JVAE_CHECK_ARG(T && out && N > 0 && H > 0 && W > 0, "bad arguments");
-  JVAE_CHECK_ARG(k >= 1 && pad >= 0 && Co >= 1 && Co <= 4 && k * Co <= VS_MAXC && ld_t >= k * Co && ld_out >= Co, "k * Co must be <= 16, Co <= 4");
-  const size_t P = (size_t)N * H * W;
-  size_t blocks = (P + 255) / 256;
-  const size_t cap = (size_t)sm_count() * 8;
-  if (blocks > cap) blocks = cap;
-  const bool fixed = ld_t == 16 && ld_out == 8 && pad == (k - 1) / 2 && (k & 1) &&
-                     ((reinterpret_cast<uintptr_t>(T) | reinterpret_cast<uintptr_t>(out)) & 15) == 0;
-  const int tf = (act & JVAE_IN_F32) ? 1 : 0;
-  act &= 0xff;
-  const __nv_bfloat16* Tp = reinterpret_cast<const __nv_bfloat16*>(T);
-  __nv_bfloat16* op = reinterpret_cast<__nv_bfloat16*>(out);
-  cudaStream_t st = (cudaStream_t)stream;
-#define VSUM_FIXED(KK, CO)                                                                                                   \
-  if (tf) vsum_rows_fixed_kernel<KK, CO, true><<<resident_grid(vsum_rows_fixed_kernel<KK, CO, true>, 256, 0, (int)blocks), 256, 0, st>>>(T, N, H, W, bias, act, stats, op); \
-  else vsum_rows_fixed_kernel<KK, CO, false><<<resident_grid(vsum_rows_fixed_kernel<KK, CO, false>, 256, 0, (int)blocks), 256, 0, st>>>(T, N, H, W, bias, act, stats, op)
-  if (fixed && k == 5 && Co == 3) { VSUM_FIXED(5, 3); }
-  else if (fixed && k == 3 && Co == 3) { VSUM_FIXED(3, 3); }
-  else if (fixed && k == 5 && Co == 1) { VSUM_FIXED(5, 1); }
-  else if (fixed && k == 3 && Co == 1) { VSUM_FIXED(3, 1); }
-  else vsum_rows_kernel<<<(int)blocks, 256, 0, st>>>(Tp, ld_t, N, H, W, k, pad, Co, bias, act, stats, op, ld_out, tf);
-#undef VSUM_FIXED
-  JVAE_LAUNCH_CHECK();
   return JVAE_OK;
 }
 

@@ -2,7 +2,6 @@
 ONE all-reduce per step on the flat gradient bucket the optimizer already owns (bf16 by default), averaged, followed by
 the global-norm clip and Adam on the reduced bucket (identical on every rank).  BatchNorm statistics stay per rank, as
 in the reference at the per-GPU batch size.  Scoring shards by sample with a single final gather (gather_scores)."""
-import os
 
 import torch
 import torch.distributed as dist
@@ -34,7 +33,7 @@ def attach(net, bf16_bucket=True, group=None):
 
     opt.allreduce = allreduce
     # NCCL collectives can be recorded into a CUDA graph (train_step(graph=True) replays the whole data-parallel step)
-    opt.allreduce_capturable = dist.get_backend(group) == 'nccl' and os.environ.get('JVAE_DP_GRAPH', '1') != '0'
+    opt.allreduce_capturable = dist.get_backend(group) == 'nccl'
     return net
 
 

@@ -86,8 +86,7 @@ class EmuKernels:
         acc = _act(acc, act & 0xff)
         view = out[:, out_o[0]::out_s[0], out_o[1]::out_s[1]]
         assert view.shape[1] == Hq and view.shape[2] == Wq, (view.shape, Hq, Wq)
-        assert bool(act & 0x100) == (out.dtype == torch.float32 and EmuKernels.store != torch.float32) or EmuKernels.store == torch.float32
-        view[..., :Cout] = acc if (act & 0x100) else acc.to(EmuKernels.store)      # JVAE_OUT_F32: no rounding of the result
+        view[..., :Cout] = acc.to(EmuKernels.store)
         view[..., Cout:] = 0
 
     @staticmethod
@@ -248,25 +247,6 @@ class EmuKernels:
             dst[..., :C] = s.view(N, H // k, k, W // k, k, C).mean((2, 4)).to(EmuKernels.store)
         else:
             dst[..., :C] = (s / (k * k)).repeat_interleave(k, 1).repeat_interleave(k, 2).to(EmuKernels.store)
-
-    @classmethod
-    def vsum_rows(cls, T, ld_t, N, H, W, k, pad, Co, bias, act, stats, out, ld_out):
-        cls.launches += 1
-        assert bool(act & 0x200) == (T.dtype == torch.float32) or EmuKernels.store == torch.float32      # JVAE_IN_F32
-        act &= 0xff
-        t = torch.nan_to_num(T.float())
-        acc = torch.zeros(N, H, W, Co)
-        for ty in range(k):
-            sh = ty - pad                           # out[y] += T[y + sh][ty*Co : ty*Co + Co]
-            lo, hi = max(0, -sh), min(H, H - sh)
-            if hi > lo:
-                acc[:, lo:hi] += t[:, lo + sh:hi + sh, :, ty * Co:(ty + 1) * Co]
-        if bias is not None:
-            acc = acc + bias.float()
-        if stats is not None:
-            stats[0] += acc.sum((0, 1, 2)).double()
-            stats[1] += (acc * acc).sum((0, 1, 2)).double()
-        out[..., :Co] = _act(acc, act).to(EmuKernels.store)
 
     @classmethod
     def vstack_rows(cls, dy, ld_dy, N, H, W, k, pad, Co, U, ld_u):

@@ -283,10 +283,9 @@ def test_residual_blocks_exact(pkg, ce, monkeypatch, kind):
 
 
 @pytest.mark.parametrize('shape,spec', [((16, 2, 2), '[x3+1]16-24'), ((8, 1, 2), '[x3+1]16'), ((16, 2, 1), '[x5+2]8-8')])
-def test_dense_small_map_form(pkg, ce, monkeypatch, shape, spec):
-    """opt-in JVAE_CONV_DENSE_SMALL: 'same' convolutions on maps of at most 2x2 pixels as one dense GEMM over (pixel, channel)
-    pairs (the vgg19 tail); forward, input gradient and parameter gradients equal torch's with fp32 storage"""
-    monkeypatch.setattr(ce, 'DENSE_SMALL', True)
+def test_small_map_same_convolutions(pkg, ce, monkeypatch, shape, spec):
+    """'same' convolutions on maps of at most 2x2 pixels (the vgg19 tail), where most taps read padding: forward, input
+    gradient and parameter gradients equal torch's with fp32 storage, in train and eval mode"""
     monkeypatch.setattr(EmuKernels, 'store', torch.float32)
     monkeypatch.setattr(EmuKernels, 'act_dtype', torch.float32)
     torch.manual_seed(0)
@@ -308,8 +307,6 @@ def test_dense_small_map_form(pkg, ce, monkeypatch, shape, spec):
         xin = x.clone().requires_grad_(True)
         ce._stacks.clear()
         got = ce.run(list(seq), xin)
-        stack = next(iter(ce._stacks.values()))
-        assert all(s.dense_small for s in stack.steps if isinstance(s, ce.ConvStep))
         tol = 1e-4 if mode == 'train' else 2e-2        # eval folds BatchNorm into bf16 weights
         assert _rel(got, want) < tol
         for p in seq.parameters():
@@ -333,11 +330,10 @@ def test_c2_stack_plan(pkg, ce):
     st = ce.ConvStack(list(imager), (128, 1, 1), True)
     convs = [s for s in st.steps if isinstance(s, ce.ConvStep)]
     assert [s.gemm1x1 for s in convs] == [True] + [False] * 6             # ConvTranspose2d on the 1x1 latent map is a plain GEMM
-    assert [s.separable for s in convs] == [False] * 6 + [True]           # 32 -> 3 k5 head: 1 x 5 pass + row kernels
+    assert [s.separable for s in convs] == [False] * 6 + [True]           # 32 -> 3 k5 head: separable backward
     assert convs[-1].wgrad_swapped and not any(s.wgrad_swapped for s in convs[:-1])
     assert [len(s.fwd_ops) if s.fwd_ops else 0 for s in convs] == [0, 1, 4, 1, 4, 1, 1]      # stride-2 deconvs: 4 sub-pixel phases
     assert [s.merged_fwd for s in convs] == [False, False, True, False, True, False, False]    # ... issued as ONE merged launch
-    assert not any(s.dense_small for s in convs)                          # opt-in only
     assert st.out_shape == (3, 32, 32)
     feats = build((3, 32, 32), 'vgg19', batch_norm=True, where='input')
     sf = ce.ConvStack(list(feats), (3, 32, 32), False)

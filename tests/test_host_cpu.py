@@ -21,7 +21,7 @@ def test_library_exports_every_declared_symbol(pkg):
     lib = ctypes.CDLL(pkg._native.LIB_PATH)
     missing = [s for s in declared if not hasattr(lib, s)]
     assert not missing, missing
-    assert lib.jvae_abi_version() == 16
+    assert lib.jvae_abi_version() == 17
 
 
 def test_elbo_cfg_struct_matches_header(pkg):

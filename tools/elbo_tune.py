@@ -1,5 +1,5 @@
 """Times the fused ELBO kernels alone (CUDA events, L2 flushed between launches) at the c2 / c5 shapes.
-Usage: JVAE_ELBO_LG={1,2,4,8} python tools/elbo_tune.py"""
+Usage: python tools/elbo_tune.py"""
 import os
 import sys
 
@@ -86,6 +86,6 @@ for (B, L, K, C, D) in [(512, 16, 128, 10, 3072), (512, 16, 256, 100, 3072), (51
     g_e = bench_graph(lambda i: (lambda: nat.elbo_eval_fwd(cfg, x, xrs[i], mu, lv, z, en, None, means, T, sig)))
     print(f'   graph-replayed, rotating buffers: fwd {g_f:.2f} us = {bytes_fwd / g_f / 1e3:.0f} GB/s | eval {g_e:.2f} us = '
           f'{(bytes_fwd + B * L * K * 4) / g_e / 1e3:.0f} GB/s', flush=True)
-    print(f'LG={os.environ.get("JVAE_ELBO_LG", "4")} B={B} L={L} K={K} C={C}: fwd {t_f[0]:.1f} us (min {t_f[1]:.1f}) = '
+    print(f'B={B} L={L} K={K} C={C}: fwd {t_f[0]:.1f} us (min {t_f[1]:.1f}) = '
           f'{bytes_fwd / t_f[0] / 1e3:.0f} GB/s | bwd {t_b[0]:.1f} us = {(bytes_fwd + B * L * D * 2) / t_b[0] / 1e3:.0f} GB/s | '
           f'eval {t_e[0]:.1f} us = {(bytes_fwd + B * L * K * 4) / t_e[0] / 1e3:.0f} GB/s', flush=True)
