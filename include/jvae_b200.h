@@ -402,7 +402,7 @@ int jvae_batch_u8_to_f32(const jvae_batch_cfg* cfg, const void* src, long long n
                          const unsigned char* flip, const int* crop_ij, float* out, void* stream);
 
 /* ------------------------------------------------------------------------------------------
- * Optimizer (module/optimizers.py:79-81,120-121: clip_grad_norm_ then Adam with L2 weight decay)
+ * Optimizer (module/optimizers.py:79-81,120-121: clip_grad_norm_ then Adam / AMSGrad / SGD with L2 weight decay)
  * on one flat f32 parameter / gradient buffer.  grad may be the bf16 all-reduced bucket.
  * ------------------------------------------------------------------------------------------ */
 /* The flat buffers hold the trainable parameters back to back, each starting on a multiple of JVAE_OPT_CHUNK elements;
@@ -422,6 +422,21 @@ int jvae_adam_step(float* p, float* m, float* v, const void* grad, int grad_dtyp
                    const float* norm2, float max_norm, float lr, float beta1, float beta2, float eps,
                    float weight_decay, int nseg, const int32_t* chunk_seg, const int32_t* seg_active, int32_t* seg_step,
                    float* seg_bc, float grad_scale, void* stream);
+/* jvae_adam_step with AMSGrad (torch.optim.Adam(amsgrad=True)): vmax (n) f32, zero-initialised, holds the running maximum
+ * of v; vmax = max(vmax, v) after the v update and denom = sqrt(vmax) / sqrt(1 - beta2^t) + eps. */
+int jvae_adam_amsgrad_step(float* p, float* m, float* v, float* vmax, const void* grad, int grad_dtype, size_t n,
+                           const float* norm2, float max_norm, float lr, float beta1, float beta2, float eps,
+                           float weight_decay, int nseg, const int32_t* chunk_seg, const int32_t* seg_active, int32_t* seg_step,
+                           float* seg_bc, float grad_scale, void* stream);
+/* torch.optim.SGD on the same flat buffers and parameter table: d = clip_coef * grad_scale * g + weight_decay * p; with
+ * momentum != 0, buf = d on a parameter's first update (its seg_step becomes 1 in this call), else
+ * buf = momentum * buf + (1 - dampening) * d, then d = nesterov ? d + momentum * buf : buf; p -= lr * d.
+ * buf (n) f32 is required iff momentum != 0 (with momentum == 0 only p and g are touched).  As for Adam, a parameter whose
+ * gradient slice is all zero counts as having no gradient: it is neither updated nor counted.  Two launches: per-parameter
+ * step counts, then the update. */
+int jvae_sgd_step(float* p, float* buf, const void* grad, int grad_dtype, size_t n, const float* norm2, float max_norm,
+                  float lr, float momentum, float dampening, int nesterov, float weight_decay, int nseg,
+                  const int32_t* chunk_seg, const int32_t* seg_active, int32_t* seg_step, float grad_scale, void* stream);
 
 /* Per-launch profile: while enabled, the fused ELBO and convolution entry points bracket their main kernel launch with CUDA events recorded
  * on the launching stream inside the library (tags below); jvae_profile_drain waits for them, returns (tag, milliseconds)

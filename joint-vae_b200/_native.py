@@ -81,6 +81,10 @@ def lib():
     L.jvae_grad_sqnorm.argtypes = [P, c_int, c_size_t, P, P, P, P]
     L.jvae_adam_step.argtypes = [P, P, P, P, c_int, c_size_t, P, c_float, c_float, c_float, c_float, c_float,
                                  c_float, c_int, P, P, P, P, c_float, P]
+    L.jvae_adam_amsgrad_step.argtypes = [P, P, P, P, P, c_int, c_size_t, P, c_float, c_float, c_float, c_float, c_float,
+                                         c_float, c_int, P, P, P, P, c_float, P]
+    L.jvae_sgd_step.argtypes = [P, P, P, c_int, c_size_t, P, c_float, c_float, c_float, c_float, c_int, c_float, c_int,
+                                P, P, P, c_float, P]
     for name in ('jvae_gemm_bf16', 'jvae_selftest'):
         if not hasattr(L, name):
             raise NativeError(f'{LIB_PATH} does not export {name}: stale build')
@@ -457,6 +461,23 @@ def adam_step(p, m, v, grad, norm2, *, max_norm, lr, beta1, beta2, eps, weight_d
     check(lib().jvae_adam_step(ptr(p), ptr(m), ptr(v), ptr(grad), dtype_code(grad), p.numel(), ptr(norm2),
                                float(max_norm or 0.0), lr, beta1, beta2, eps, weight_decay, seg_active.numel(), ptr(chunk_seg),
                                ptr(seg_active), ptr(seg_step), ptr(seg_bc), grad_scale, stream()))
+
+
+def adam_amsgrad_step(p, m, v, vmax, grad, norm2, *, max_norm, lr, beta1, beta2, eps, weight_decay, chunk_seg, seg_active,
+                      seg_step, seg_bc, grad_scale=1.0):
+    """include/jvae_b200.h: jvae_adam_amsgrad_step (adam_step that normalises by the running maximum vmax of v)"""
+    check(lib().jvae_adam_amsgrad_step(ptr(p), ptr(m), ptr(v), ptr(vmax), ptr(grad), dtype_code(grad), p.numel(), ptr(norm2),
+                                       float(max_norm or 0.0), lr, beta1, beta2, eps, weight_decay, seg_active.numel(),
+                                       ptr(chunk_seg), ptr(seg_active), ptr(seg_step), ptr(seg_bc), grad_scale, stream()))
+
+
+def sgd_step(p, buf, grad, norm2, *, max_norm, lr, momentum, dampening, nesterov, weight_decay, chunk_seg, seg_active, seg_step,
+             grad_scale=1.0):
+    """include/jvae_b200.h: jvae_sgd_step (buf: the momentum buffer, None iff momentum == 0; the per-parameter step counts
+    tell each parameter's first update)"""
+    check(lib().jvae_sgd_step(ptr(p), ptr(buf), ptr(grad), dtype_code(grad), p.numel(), ptr(norm2), float(max_norm or 0.0),
+                              lr, momentum, dampening, int(bool(nesterov)), weight_decay, seg_active.numel(), ptr(chunk_seg),
+                              ptr(seg_active), ptr(seg_step), grad_scale, stream()))
 
 
 GEMM_NT, GEMM_NN, GEMM_TN = 0, 1, 2

@@ -1,6 +1,6 @@
 """Batch-sharded data parallelism for the train step: one process per GPU (torch.distributed, NCCL over NVLink),
 ONE all-reduce per step on the flat gradient bucket the optimizer already owns (bf16 by default), averaged, followed by
-the global-norm clip and Adam on the reduced bucket (identical on every rank).  BatchNorm statistics stay per rank, as
+the global-norm clip and the Adam or SGD update on the reduced bucket (identical on every rank).  BatchNorm statistics stay per rank, as
 in the reference at the per-GPU batch size.  Scoring shards by sample with a single final gather (gather_scores)."""
 
 import torch
