@@ -207,9 +207,11 @@ int jvae_gemm_bf16(int mode, int M, int N, int K, const void* a, int lda, const 
  * jvae_conv_gather_gemm: for every position q = (n, qy, qx) of an (N, Hq, Wq) grid
  *     out[n, qy*out_sy + out_oy, qx*out_sx + out_ox, co] =
  *         act( bias[co] + sum_t sum_ci in[n, qy*in_stride + tap_dy[t], qx*in_stride + tap_dx[t], ci] * W[co][t][ci] )
- *   with out-of-image reads equal to zero.  One call is a Conv2d (stride 1 or 2), a ConvTranspose2d of stride 1
- *   (flipped taps), ONE sub-pixel phase of a stride-2 ConvTranspose2d (out_s = 2, out_o = phase), or the data
- *   gradient of any of them, depending on the tap table and weight arrangement the host passes.
+ *   with out-of-image reads equal to zero.  One call is a Conv2d (stride 1..8), a ConvTranspose2d of stride 1
+ *   (flipped taps), ONE sub-pixel phase of a stride-s ConvTranspose2d (out_s = s <= 8, out_o = phase), or the data
+ *   gradient of any of them, depending on the tap table and weight arrangement the host passes.  in_stride is 1..8
+ *   (the 'x4+0:4' / ':8' tokens of the spec grammar, conv.py:20-84): strides 1 and 2 run on the halo kernel where it
+ *   takes the geometry, strides 3..8 always on the tap-box kernel.
  *   in  (N,H,W,ld_in) bf16, Cin real channels; wmat (Cout_pad, ldw) bf16 with row co = [tap][chunk][Cblk] where
  *   Cblk = 16/32/64 for Cin <= 16 / <= 32 / > 32 and chunk = ceil(Cin/Cblk) (zero padded); Cout_pad a multiple of 16
  *   (of 256 above 256); out (N,Ho,Wo,ld_out) bf16, channels >= Cout up to ld_out are written as zeros.
@@ -217,6 +219,7 @@ int jvae_gemm_bf16(int mode, int M, int N, int K, const void* a, int lda, const 
  *   call writes, taken from the fp32 accumulators (BatchNorm2d batch statistics, conv.py:216-217); fp64 so that the
  *   arrival order of warps / CTAs does not change the result (run-to-run reproducible).
  * jvae_conv_wgrad: dw[t][co][ci] += sum_q dy[n,qy,qx,co] * x[n, qy*in_stride + tap_dy[t], qx*in_stride + tap_dx[t], ci]
+ *   (in_stride 1..8)
  *   (fp32, atomically accumulated into dw: the caller zeroes it, or passes the live .grad buffer to accumulate into);
  *   element (t, co, ci) lives at dw[t*dw_ld_tap + co*dw_ld_co + ci*dw_ld_ci], so the torch (Cout,Cin,kh,kw) layout is
  *   (1, Cin*kh*kw, kh*kw).
@@ -244,7 +247,7 @@ int jvae_conv_subpixel_gemm(const void* in, int N, int H, int W, int Cin, int ld
  * so the planner is testable without a device.  nphases = 0: the plan of jvae_conv_gather_gemm (ntaps / in_stride / out_o as
  * there); nphases >= 2: the plan of jvae_conv_subpixel_gemm (out_sy = out_sx = out_s, out_o = 0).  info (8 ints, may be NULL)
  * receives {G, phases, M-tiles per box, images per box, channel tile, chunk records, resident weights, stages}.
- * Returns JVAE_NOT_COVERED when the halo kernel does not take the geometry. */
+ * Returns JVAE_NOT_COVERED when the halo kernel does not take the geometry (always for in_stride 3..8). */
 int jvae_conv_halo_emulate(const float* in, int N, int H, int W, int Cin, int ld_in, const float* wmat, int Cout_pad, int ldw,
                            int nphases, const int16_t* phase_ntaps, const int16_t* phase_oy, const int16_t* phase_ox, int ntaps,
                            const int16_t* tap_dy, const int16_t* tap_dx, int in_stride, int Hq, int Wq, float* out, int Ho, int Wo,
@@ -268,7 +271,7 @@ int jvae_last_conv_kernel(void);
 /* ------------------------------------------------------------------------------------------
  * Layers between the convolutions, NHWC bf16, P = N*H*W pixels (module/vae_layers/conv.py:189-227):
  * BatchNorm2d (torch semantics: biased variance to normalise, unbiased for running_var, momentum 0.1),
- * activation backward + bias gradient, MaxPool2d(2), UpsamplingNearest2d(2).
+ * activation backward + bias gradient, MaxPool2d, AvgPool2d, UpsamplingNearest2d.
  * ------------------------------------------------------------------------------------------ */
 /* stats (2,C) f64 += per-channel sum / sum of squares of y (P,C) with leading dimension ld (zero stats first) */
 int jvae_bn_stats(const void* y, size_t P, int C, int ld, double* stats, void* stream);
@@ -337,6 +340,20 @@ int jvae_add_act(const void* a, int ld_a, const void* b, int ld_b, size_t P, int
                  void* stream);
 /* backward == 0: dst (N,2H,2W,C) = nearest up-sampling of src (N,H,W,C); backward != 0: dst (N,H,W,C) = 2x2 block sums of src */
 int jvae_upsample2(const void* src, int ld_src, void* dst, int ld_dst, int N, int H, int W, int C, int backward, void* stream);
+/* UpsamplingNearest2d(scale_factor=s) for an integer s >= 1 (the 'U:s' tokens of the spec grammar, conv.py:20-84, 149-151):
+ * backward == 0: dst (N,sH,sW,C) = nearest up-sampling of src (N,H,W,C); backward != 0: dst (N,H,W,C) = s x s block sums of
+ * src (N,sH,sW,C), summed in fp32 in a fixed order per pixel (gather form, no atomics: bit-reproducible).  Channel strides
+ * ld_src / ld_dst as for jvae_upsample2, which stays the s = 2 kernel. */
+int jvae_upsample_nearest(const void* src, int ld_src, void* dst, int ld_dst, int N, int H, int W, int C, int s, int backward,
+                          void* stream);
+/* AvgPool2d(kernel (kh,kw), stride (sh,sw), padding (ph,pw)) with torch's defaults ceil_mode=False, count_include_pad=True
+ * (the 'A' tokens of the spec grammar that overlap, pad or do not tile the map, conv.py:144-148; with (kh,kw) = (sh,sw) =
+ * (H,W) also AdaptiveAvgPool2d(1) on a non-square map).  Output (N, (H+2ph-kh)/sh+1, (W+2pw-kw)/sw+1, C); the divisor is
+ * always kh*kw.  Padding at most half the kernel.  backward == 0: dst = pooled src; backward != 0: src is the output gradient
+ * and dst (N,H,W,C) the input gradient, each input pixel summing dout / (kh*kw) over the windows that cover it (gather form,
+ * no atomics, deterministic; pixels no window covers get zero). */
+int jvae_avgpool_pad(const void* src, int ld_src, void* dst, int ld_dst, int N, int H, int W, int C, int kh, int kw, int sh, int sw,
+                     int ph, int pw, int backward, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Small data-movement / elementwise kernels of the step

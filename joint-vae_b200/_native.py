@@ -125,6 +125,8 @@ def lib():
     L.jvae_maxpool_pad_fwd.argtypes = [P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P, c_int, P]
     L.jvae_maxpool_pad_bwd.argtypes = [P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P, c_int, P, c_int, P]
     L.jvae_avgpool.argtypes = [P, c_int, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P]
+    L.jvae_upsample_nearest.argtypes = [P, c_int, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P]
+    L.jvae_avgpool_pad.argtypes = [P, c_int, P, c_int] + [c_int] * 11 + [P]
     L.jvae_add_act.argtypes = [P, c_int, P, c_int, c_size_t, c_int, c_int, P, c_int, P]
     L.jvae_vstack_rows.argtypes = [P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P, c_int, P]
     L.jvae_elbo_prior_stats.argtypes = [ctypes.POINTER(ElboCfg), P, P, P, c_size_t, P]
@@ -676,6 +678,15 @@ def maxpool_pad_bwd(inp, N, H, W, C, ld_in, k, stride, pad, dout, ld_dout, din, 
 
 def avgpool(src, ld_src, dst, ld_dst, N, H, W, C, k, backward=False):
     check(lib().jvae_avgpool(rawptr(src), ld_src, rawptr(dst), ld_dst, N, H, W, C, k, int(backward), stream()))
+
+
+def upsample_nearest(src, ld_src, dst, ld_dst, N, H, W, C, s, backward=False):
+    check(lib().jvae_upsample_nearest(rawptr(src), ld_src, rawptr(dst), ld_dst, N, H, W, C, s, int(backward), stream()))
+
+
+def avgpool_pad(src, ld_src, dst, ld_dst, N, H, W, C, kh, kw, sh, sw, ph, pw, backward=False):
+    check(lib().jvae_avgpool_pad(rawptr(src), ld_src, rawptr(dst), ld_dst, N, H, W, C, kh, kw, sh, sw, ph, pw, int(backward),
+                                 stream()))
 
 
 def vstack_rows(dy, ld_dy, N, H, W, k, pad, Co, U, ld_u):

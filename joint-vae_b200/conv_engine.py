@@ -7,9 +7,9 @@ hand-written backward.  Activations live in HBM as NHWC bf16 (channel stride pad
 are re-packed to the kernels' bf16 [Cout][tap][Cin-chunk] arrangement whenever their version changes.
 
 Every convolution flavour is one or several launches of the same tcgen05 "gather GEMM" (csrc/conv.cu):
-  Conv2d stride 1/2            taps (i-p, j-p), input stride s
+  Conv2d stride 1..8           taps (i-p, j-p), input stride s
   ConvTranspose2d stride 1     taps (p-i, p-j)
-  ConvTranspose2d stride s>1   s*s sub-pixel phases, each a small stride-1 gather written with output stride s
+  ConvTranspose2d stride 2..8  s*s sub-pixel phases, each a small stride-1 gather written with output stride s
   data gradients               the same two forms with the roles of Conv / ConvTranspose exchanged
   ConvTranspose2d on 1x1 input a plain GEMM (csrc/gemm.cu)
 Weight gradients use csrc/conv.cu's wgrad kernel (MN-major operands straight from the NHWC tensors).
@@ -138,6 +138,8 @@ class NativeKernels:
     maxpool_pad_fwd = staticmethod(nat.maxpool_pad_fwd)
     maxpool_pad_bwd = staticmethod(nat.maxpool_pad_bwd)
     avgpool = staticmethod(nat.avgpool)
+    avgpool_pad = staticmethod(nat.avgpool_pad)
+    upsample_nearest = staticmethod(nat.upsample_nearest)
     add_act = staticmethod(nat.add_act)
     vstack_rows = staticmethod(nat.vstack_rows)
     taps_arg = staticmethod(nat.taps_arg)
@@ -307,6 +309,8 @@ class ConvStep:
             raise NotImplementedError('dilated / grouped convolutions')
         if k * k > 64:
             raise NotImplementedError('kernels larger than 8x8')
+        if s > 8:
+            raise NotImplementedError('convolution stride > 8')
         self.k, self.p, self.s = k, p, s
         Ci, H, W = in_shape
         self.Ci, self.H, self.W = Ci, H, W
@@ -315,8 +319,6 @@ class ConvStep:
             op = conv.output_padding[0]
             self.Ho, self.Wo = (H - 1) * s - 2 * p + k + op, (W - 1) * s - 2 * p + k + op
         else:
-            if s > 2:
-                raise NotImplementedError('convolution stride > 2')
             self.Ho, self.Wo = (H + 2 * p - k) // s + 1, (W + 2 * p - k) // s + 1
         self.out_shape = (self.Co, self.Ho, self.Wo)
         self.gemm1x1 = (self.transposed and H == 1 and W == 1 and p == 0 and conv.output_padding[0] == 0
@@ -327,8 +329,6 @@ class ConvStep:
         if self.gemm1x1:
             self.fwd_ops = self.dgrad_ops = None
         elif self.transposed:
-            if s > 2:
-                raise NotImplementedError('transposed convolution stride > 2 (weight gradient kernel)')
             self.fwd_ops = deconv_form(k, p, s, self.Ho, self.Wo)
             self.dgrad_ops = conv_form(k, p, s, H, W)
         else:
@@ -709,23 +709,30 @@ class PoolStep:
 
 
 class AvgStep:
-    """AvgPool2d(k) with stride k, or AdaptiveAvgPool2d(1) (k = H = W: the last layer of torchvision's ResNet features)"""
+    """AvgPool2d (floor mode, count_include_pad=True) and AdaptiveAvgPool2d(1).  Windows that tile the map (stride = kernel,
+    no padding; k = H = W for the last layer of torchvision's ResNet features) run on jvae_avgpool; overlapping, padded or
+    non-tiling windows ('A3+1:2', 'A2' on an odd map) and the global pool of a non-square map on jvae_avgpool_pad."""
 
     def __init__(self, mod, in_shape):
         self.C, self.H, self.W = in_shape
+        pair = lambda v: tuple(v) if isinstance(v, (tuple, list)) else (v, v)
         if isinstance(mod, nn.AdaptiveAvgPool2d):
-            o = mod.output_size if isinstance(mod.output_size, (tuple, list)) else (mod.output_size, mod.output_size)
-            if tuple(o) != (1, 1) or self.H != self.W:
-                raise NotImplementedError('AdaptiveAvgPool2d other than (1, 1) on a square map has no native kernel')
-            k = self.H
+            if pair(mod.output_size) != (1, 1):
+                raise NotImplementedError('AdaptiveAvgPool2d with an output size other than (1, 1) has no native kernel')
+            (kh, kw), (sh, sw), (ph, pw) = (self.H, self.W), (self.H, self.W), (0, 0)
         else:
-            k = mod.kernel_size if isinstance(mod.kernel_size, int) else mod.kernel_size[0]
-            stv = mod.stride if isinstance(mod.stride, int) else mod.stride[0]
-            pad = mod.padding if isinstance(mod.padding, int) else mod.padding[0]
-            if stv != k or pad != 0 or self.H % k or self.W % k or mod.ceil_mode:
-                raise NotImplementedError('AvgPool2d must tile the map (stride = kernel, no padding)')
-        self.k = k
-        self.out_shape = (self.C, self.H // k, self.W // k)
+            (kh, kw), (sh, sw), (ph, pw) = pair(mod.kernel_size), pair(mod.stride), pair(mod.padding)
+            if mod.ceil_mode:
+                raise NotImplementedError('AvgPool2d with ceil_mode=True has no native kernel')
+            if mod.divisor_override or (not mod.count_include_pad and (ph or pw)):
+                raise NotImplementedError('AvgPool2d with count_include_pad=False or a divisor_override has no native kernel')
+            if 2 * ph > kh or 2 * pw > kw:
+                raise NotImplementedError('AvgPool2d with padding larger than half the kernel')
+        self.win = (kh, kw, sh, sw, ph, pw)
+        self.tiling = kh == kw == sh == sw and ph == pw == 0 and self.H % kh == 0 and self.W % kw == 0
+        self.k = kh
+        self.Ho, self.Wo = (self.H + 2 * ph - kh) // sh + 1, (self.W + 2 * pw - kw) // sw + 1
+        self.out_shape = (self.C, self.Ho, self.Wo)
 
     def params(self):
         return []
@@ -734,8 +741,11 @@ class AvgStep:
         N, _, _, ld = x.shape
         out = st.pop('out', None)        # the first channels of a dense block's buffer (DenseBlockStep)
         if out is None:
-            out = K.empty((N, self.H // self.k, self.W // self.k, ld), x)
-        K.avgpool(x, ld, out, out.stride(2), N, self.H, self.W, ld, self.k, False)
+            out = K.empty((N, self.Ho, self.Wo, ld), x)
+        if self.tiling:
+            K.avgpool(x, ld, out, out.stride(2), N, self.H, self.W, ld, self.k, False)
+        else:
+            K.avgpool_pad(x, ld, out, out.stride(2), N, self.H, self.W, ld, *self.win, False)
         st['ld'] = ld
         return out
 
@@ -744,7 +754,10 @@ class AvgStep:
             return None, []
         N, ld = da.shape[0], st['ld']
         dx = K.empty((N, self.H, self.W, ld), da)
-        K.avgpool(da, da.shape[-1], dx, ld, N, self.H, self.W, ld, self.k, True)
+        if self.tiling:
+            K.avgpool(da, da.shape[-1], dx, ld, N, self.H, self.W, ld, self.k, True)
+        else:
+            K.avgpool_pad(da, da.shape[-1], dx, ld, N, self.H, self.W, ld, *self.win, True)
         return dx, []
 
 
@@ -999,21 +1012,28 @@ class DenseBlockStep:
 
 
 class UpStep:
-    """UpsamplingNearest2d(scale_factor=2)"""
+    """UpsamplingNearest2d(scale_factor=s) for an integer s >= 1: jvae_upsample2 for s = 2, jvae_upsample_nearest otherwise"""
 
     def __init__(self, mod, in_shape):
-        if int(mod.scale_factor) != 2:
-            raise NotImplementedError('only 2x nearest up-sampling has a native kernel')
+        sf = mod.scale_factor
+        sf = tuple(sf) if isinstance(sf, (tuple, list)) else (sf, sf)
+        if mod.size is not None or sf[0] is None or sf[0] != sf[1] or float(sf[0]) != int(sf[0]) or int(sf[0]) < 1:
+            raise NotImplementedError('nearest up-sampling by an output size or a non-integer / non-uniform scale factor '
+                                      'has no native kernel')
+        self.s = int(sf[0])
         self.C, self.H, self.W = in_shape
-        self.out_shape = (self.C, 2 * self.H, 2 * self.W)
+        self.out_shape = (self.C, self.s * self.H, self.s * self.W)
 
     def params(self):
         return []
 
     def forward(self, x, st, training):
         N, _, _, ld = x.shape
-        out = K.empty((N, 2 * self.H, 2 * self.W, ld), x)
-        K.upsample2(x, ld, out, ld, N, self.H, self.W, ld, False)
+        out = K.empty((N, self.s * self.H, self.s * self.W, ld), x)
+        if self.s == 2:
+            K.upsample2(x, ld, out, ld, N, self.H, self.W, ld, False)
+        else:
+            K.upsample_nearest(x, ld, out, ld, N, self.H, self.W, ld, self.s, False)
         st['ld'] = ld
         return out
 
@@ -1023,7 +1043,10 @@ class UpStep:
         N = da.shape[0]
         ld = st['ld']
         dx = K.empty((N, self.H, self.W, ld), da)
-        K.upsample2(da, da.shape[-1], dx, ld, N, self.H, self.W, ld, True)
+        if self.s == 2:
+            K.upsample2(da, da.shape[-1], dx, ld, N, self.H, self.W, ld, True)
+        else:
+            K.upsample_nearest(da, da.shape[-1], dx, ld, N, self.H, self.W, ld, self.s, True)
         return dx, []
 
 

@@ -1,5 +1,5 @@
-// Implicit-GEMM convolutions on tcgen05 for NHWC bf16 activations: Conv2d, ConvTranspose2d (stride 1, and stride 2
-// through its 4 sub-pixel phases), their data gradients (the same kernel with transformed weights / geometry) and the
+// Implicit-GEMM convolutions on tcgen05 for NHWC bf16 activations: Conv2d (stride 1..8), ConvTranspose2d (stride 1, and
+// stride s = 2..8 through its s*s sub-pixel phases), their data gradients (the same kernel with transformed weights / geometry) and the
 // weight gradient (second kernel, MN-major operands, split over the pixel dimension).
 //
 // Replaces nn.Conv2d / nn.ConvTranspose2d of the reference's features / imager stacks
@@ -1030,10 +1030,14 @@ conv_wgrad_halo_kernel(const __grid_constant__ CUtensorMap tmap_g, const __grid_
 static int pow2_floor(int v) { int p = 1; while (p * 2 <= v) p *= 2; return p; }
 static int pow2_ceil(int v) { int p = 1; while (p < v) p *= 2; return p; }
 
-static void tile_shape(int Hq, int Wq, int* TW, int* TH, int* NB) {
-  int tw = pow2_floor(Wq); if (tw > 128) tw = 128;
-  if (tw < Wq && tw * 2 <= 128 && (tw * 2 - Wq) * 4 <= Wq) tw *= 2;   // e.g. W=28 -> 32 rather than 16
+// tile box of the tap-box kernels for input stride s: the strided input box spans TW*s x TH*s elements, and a TMA box
+// dimension is at most 256, so TW and TH are capped at pow2_floor(256 / s) (no cap below 128 for s <= 2)
+static void tile_shape(int Hq, int Wq, int s, int* TW, int* TH, int* NB) {
+  const int cap = min(128, pow2_floor(256 / s));
+  int tw = pow2_floor(Wq); if (tw > cap) tw = cap;
+  if (tw < Wq && tw * 2 <= cap && (tw * 2 - Wq) * 4 <= Wq) tw *= 2;   // e.g. W=28 -> 32 rather than 16
   int th = pow2_ceil(Hq); if (th > 128 / tw) th = 128 / tw;
+  if (th > cap) th = cap;
   *TW = tw; *TH = th; *NB = 128 / (tw * th);
 }
 
@@ -1059,6 +1063,8 @@ static int try_launch_halo(const void* in, int N, int H, int W, int Cin, int ld_
                            const float* bias, int act, double* stats, cudaStream_t stream, const PhaseSpec* phs = nullptr,
                            HaloParams* plan_out = nullptr, int force_cblk = 0, double* score_out = nullptr) {
   if (Wq < 6) return 1;
+  // strides 3..8 read s*s parity planes: more than the plane tables hold and the stage budget fits; the tap-box kernel runs them
+  if (in_stride > 2) return 1;
   // wide layers (Cin > 64 or more than 64 output channels) run on the tap-box kernel: a halo form with 64-channel output tiles
   // and weights streamed per (tap, chunk) measured slower on B200 (DESIGN.md section 6)
   if (Cin > 64 || Cout_pad > 64) return 1;
@@ -1384,6 +1390,7 @@ static int try_launch_wgrad_halo(const void* g, int N, int Hq, int Wq, int Cg, i
   // tap_ids: position of tap t in dW when the list is a subset of the layer's taps (per-plane launches, jvae_conv_wgrad);
   // dry_run: plan only (is the geometry covered?)
   if (Wq < 6) return 1;
+  if (in_stride > 2) return 1;          // s*s parity planes for s >= 3: the tap-box kernel runs them
   WHaloParams p;
   memset(&p, 0, sizeof(p));
   const int st = in_stride;
@@ -1655,7 +1662,7 @@ int jvae_conv_gather_gemm(const void* in, int N, int H, int W, int Cin, int ld_i
   JVAE_CHECK_ARG(ld_out >= Cout, "ld_out < Cout");
   JVAE_CHECK_ARG((Cout_pad % 16) == 0 && Cout_pad >= 16 && Cout_pad >= Cout, "Cout_pad must be a multiple of 16, >= Cout");
   JVAE_CHECK_ARG(!stats || Cout_pad <= 2048, "statistics epilogue supports up to 2048 channels");
-  JVAE_CHECK_ARG(in_stride == 1 || in_stride == 2, "input stride 1 or 2");
+  JVAE_CHECK_ARG(in_stride >= 1 && in_stride <= 8, "input stride 1..8");
   JVAE_CHECK_ARG((((uintptr_t)in | (uintptr_t)wmat | (uintptr_t)out) & 15) == 0, "16-byte alignment");
   int rc = try_launch_halo(in, N, H, W, Cin, ld_in, wmat, Cout_pad, ldw, ntaps, tap_dy, tap_dx, in_stride, Hq, Wq, out, Ho, Wo,
                            Cout, ld_out, out_sy, out_sx, out_oy, out_ox, bias, act, stats, (cudaStream_t)stream);
@@ -1663,7 +1670,7 @@ int jvae_conv_gather_gemm(const void* in, int N, int H, int W, int Cin, int ld_i
   ConvParams p;
   memset(&p, 0, sizeof(p));
   p.N = N; p.Hq = Hq; p.Wq = Wq;
-  tile_shape(Hq, Wq, &p.TW, &p.TH, &p.NB);
+  tile_shape(Hq, Wq, in_stride, &p.TW, &p.TH, &p.NB);
   p.tiles_x = (Wq + p.TW - 1) / p.TW; p.tiles_y = (Hq + p.TH - 1) / p.TH; p.tiles_n = (N + p.NB - 1) / p.NB;
   p.BN = Cout_pad > 256 ? 256 : Cout_pad;
   if (Cout_pad > 256) JVAE_CHECK_ARG((Cout_pad % 256) == 0, "Cout_pad > 256 must be a multiple of 256");
@@ -1744,7 +1751,7 @@ int jvae_conv_wgrad(const void* dy, int N, int Hq, int Wq, int Cout, int ld_dy, 
   JVAE_CHECK_ARG(dy && x && dw && tap_dy && tap_dx, "null pointer");
   JVAE_CHECK_ARG(ntaps >= 1 && ntaps <= CONV_MAX_TAPS, "1..64 taps");
   JVAE_CHECK_ARG((ld_dy % 8) == 0 && (ld_x % 8) == 0, "channel strides must be multiples of 8");
-  JVAE_CHECK_ARG(in_stride == 1 || in_stride == 2, "input stride 1 or 2");
+  JVAE_CHECK_ARG(in_stride >= 1 && in_stride <= 8, "input stride 1..8");
   int rc = try_launch_wgrad_halo(dy, N, Hq, Wq, Cout, ld_dy, x, H, W, Cin, ld_x, ntaps, tap_dy, tap_dx, in_stride, dw,
                                  dw_ld_tap, dw_ld_co, dw_ld_ci, (cudaStream_t)stream);
   if (rc <= 0) return rc;
@@ -1773,7 +1780,7 @@ int jvae_conv_wgrad(const void* dy, int N, int Hq, int Wq, int Cout, int ld_dy, 
   WgradParams p;
   memset(&p, 0, sizeof(p));
   p.N = N; p.Hq = Hq; p.Wq = Wq;
-  tile_shape(Hq, Wq, &p.TW, &p.TH, &p.NB);
+  tile_shape(Hq, Wq, in_stride, &p.TW, &p.TH, &p.NB);
   p.tiles_x = (Wq + p.TW - 1) / p.TW; p.tiles_y = (Hq + p.TH - 1) / p.TH; p.tiles_n = (N + p.NB - 1) / p.NB;
   p.num_tiles = p.tiles_x * p.tiles_y * p.tiles_n;
   p.Cblk_y = cblk_of(Cout); p.Cblk_x = cblk_of(Cin);
@@ -1827,7 +1834,7 @@ int jvae_conv_wgrad_emulate(const float* dy, int N, int Hq, int Wq, int Cout, in
   JVAE_CHECK_ARG(dy && x && dw && tap_dy && tap_dx, "null pointer");
   JVAE_CHECK_ARG(ntaps >= 1 && ntaps <= CONV_MAX_TAPS, "1..64 taps");
   JVAE_CHECK_ARG((ld_dy % 8) == 0 && (ld_x % 8) == 0, "channel strides must be multiples of 8");
-  JVAE_CHECK_ARG(in_stride == 1 || in_stride == 2, "input stride 1 or 2");
+  JVAE_CHECK_ARG(in_stride >= 1 && in_stride <= 8, "input stride 1..8");
   if (launches) *launches = 0;
   WHaloParams p;
   int rc = try_launch_wgrad_halo(dy, N, Hq, Wq, Cout, ld_dy, x, H, W, Cin, ld_x, ntaps, tap_dy, tap_dx, in_stride, dw, dw_ld_tap, dw_ld_co,
@@ -1877,7 +1884,7 @@ int jvae_conv_halo_emulate(const float* in, int N, int H, int W, int Cin, int ld
   JVAE_CHECK_ARG(in && wmat && out && tap_dy && tap_dx, "null pointer");
   JVAE_CHECK_ARG(ntaps >= 1 && ntaps <= CONV_MAX_TAPS, "1..64 taps");
   JVAE_CHECK_ARG(nphases == 0 || (nphases >= 2 && nphases <= 4 && phase_ntaps && phase_oy && phase_ox), "0 or 2..4 phases with their tables");
-  JVAE_CHECK_ARG(in_stride == 1 || in_stride == 2, "input stride 1 or 2");
+  JVAE_CHECK_ARG(in_stride >= 1 && in_stride <= 8, "input stride 1..8");
   JVAE_CHECK_ARG((Cout_pad % 16) == 0 && Cout_pad >= Cout && ld_out >= Cout && (ld_in % 8) == 0 && (ldw % 8) == 0, "bad channel layout");
   HaloParams p;
   PhaseSpec ps = {nphases, phase_ntaps, phase_oy, phase_ox};

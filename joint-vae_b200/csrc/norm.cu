@@ -1,4 +1,4 @@
-// BatchNorm2d (train / eval), activation backward, bias gradient, 2x2 max pooling and nearest 2x up-sampling on NHWC
+// BatchNorm2d (train / eval), activation backward, bias gradient, max / average pooling and nearest up-sampling on NHWC
 // bf16 activations: the layers that sit between the tcgen05 convolutions of the reference's features / imager stacks
 // (module/vae_layers/conv.py:189-227: Conv -> [BatchNorm2d] -> activation, MaxPool2d / AvgPool2d, UpsamplingNearest2d).
 //
@@ -785,6 +785,91 @@ __global__ void __launch_bounds__(NORM_MAX_THREADS) avgpool_kernel(const __nv_bf
   }
 }
 
+// nearest up-sampling by an integer factor s (UpsamplingNearest2d(scale_factor=s)).  Forward: one thread per OUTPUT pixel
+// copies its source pixel (coalesced stores; the s consecutive readers of a source pixel hit L1).  Backward: one thread per
+// INPUT pixel sums its s x s block of the output gradient in fp32 in a fixed order: no atomics, bit-reproducible.
+template <int V>
+__global__ void __launch_bounds__(NORM_MAX_THREADS) upsample_nearest_kernel(const __nv_bfloat16* __restrict__ src, int ld_src,
+                                                                            __nv_bfloat16* __restrict__ dst, int ld_dst, int H,
+                                                                            int W, int s, size_t P, int nchunk, int ppb,
+                                                                            int backward) {
+  // forward: P = N * sH * sW output pixels, src = small.  backward: P = N * H * W input pixels, src = large gradient.
+  const int chunk = threadIdx.x % nchunk, pl = threadIdx.x / nchunk;
+  const int Wb = W * s, Hb = H * s;
+  for (size_t p = (size_t)blockIdx.x * ppb + pl; p < P; p += (size_t)gridDim.x * ppb) {
+    float v[V];
+    if (!backward) {
+      const int ox = (int)(p % Wb), oy = (int)((p / Wb) % Hb);
+      const size_t n = p / ((size_t)Wb * Hb);
+      Vec<V>::load(src + ((n * H + oy / s) * W + ox / s) * ld_src + chunk * V, v);
+      Vec<V>::store(dst + p * ld_dst + chunk * V, v);
+    } else {
+      const int x = (int)(p % W), y = (int)((p / W) % H);
+      const size_t n = p / ((size_t)W * H);
+      float t[V];
+#pragma unroll
+      for (int e = 0; e < V; ++e) v[e] = 0.f;
+      for (int i = 0; i < s; ++i) {
+        const __nv_bfloat16* row = src + ((n * Hb + (size_t)y * s + i) * Wb + (size_t)x * s) * ld_src + chunk * V;
+        for (int j = 0; j < s; ++j) {
+          Vec<V>::load(row + (size_t)j * ld_src, t);
+#pragma unroll
+          for (int e = 0; e < V; ++e) v[e] += t[e];
+        }
+      }
+      Vec<V>::store(dst + p * ld_dst + chunk * V, v);
+    }
+  }
+}
+
+// average pooling with torch's AvgPool2d semantics for kernel (kh, kw), stride (sh, sw), padding (ph, pw): floor output
+// size, count_include_pad=True (the divisor is always kh * kw).  Forward: one thread per output pixel.  Backward in gather
+// form, one thread per INPUT pixel summing dout / (kh * kw) over the windows that cover it: no atomics, every input pixel
+// written once (pixels no window covers get zero).
+struct AvgGeo { int H, W, Ho, Wo, kh, kw, sh, sw, ph, pw; };
+
+template <int V>
+__global__ void __launch_bounds__(NORM_MAX_THREADS) avgpool_pad_kernel(const __nv_bfloat16* __restrict__ src, int ld_src,
+                                                                       __nv_bfloat16* __restrict__ dst, int ld_dst, AvgGeo q,
+                                                                       size_t P, int nchunk, int ppb, int backward) {
+  const int chunk = threadIdx.x % nchunk, pl = threadIdx.x / nchunk;
+  const float div = (float)(q.kh * q.kw);
+  for (size_t pp = (size_t)blockIdx.x * ppb + pl; pp < P; pp += (size_t)gridDim.x * ppb) {
+    float acc[V], t[V];
+#pragma unroll
+    for (int e = 0; e < V; ++e) acc[e] = 0.f;
+    if (!backward) {      // src = input (N, H, W), dst = output (N, Ho, Wo)
+      const int ox = (int)(pp % q.Wo), oy = (int)((pp / q.Wo) % q.Ho);
+      const size_t n = pp / ((size_t)q.Wo * q.Ho);
+      const int y0 = max(oy * q.sh - q.ph, 0), y1 = min(oy * q.sh - q.ph + q.kh, q.H);
+      const int x0 = max(ox * q.sw - q.pw, 0), x1 = min(ox * q.sw - q.pw + q.kw, q.W);
+      for (int iy = y0; iy < y1; ++iy)
+        for (int ix = x0; ix < x1; ++ix) {
+          Vec<V>::load(src + ((n * q.H + iy) * q.W + ix) * ld_src + chunk * V, t);
+#pragma unroll
+          for (int e = 0; e < V; ++e) acc[e] += t[e];
+        }
+#pragma unroll
+      for (int e = 0; e < V; ++e) acc[e] /= div;
+    } else {              // src = output gradient (N, Ho, Wo), dst = input gradient (N, H, W)
+      const int ix = (int)(pp % q.W), iy = (int)((pp / q.W) % q.H);
+      const size_t n = pp / ((size_t)q.W * q.H);
+      // windows o with o*s - p <= i <= o*s - p + k - 1
+      int oy0 = iy + q.ph - q.kh + 1, ox0 = ix + q.pw - q.kw + 1;
+      oy0 = oy0 <= 0 ? 0 : (oy0 + q.sh - 1) / q.sh;
+      ox0 = ox0 <= 0 ? 0 : (ox0 + q.sw - 1) / q.sw;
+      const int oy1 = min((iy + q.ph) / q.sh, q.Ho - 1), ox1 = min((ix + q.pw) / q.sw, q.Wo - 1);
+      for (int oy = oy0; oy <= oy1; ++oy)
+        for (int ox = ox0; ox <= ox1; ++ox) {
+          Vec<V>::load(src + ((n * q.Ho + oy) * q.Wo + ox) * ld_src + chunk * V, t);
+#pragma unroll
+          for (int e = 0; e < V; ++e) acc[e] += t[e] / div;
+        }
+    }
+    Vec<V>::store(dst + pp * ld_dst + chunk * V, acc);
+  }
+}
+
 // out = act(a + b): the join of a residual block (torchvision BasicBlock / Bottleneck: out += identity; relu)
 template <int V>
 __global__ void __launch_bounds__(NORM_MAX_THREADS) add_act_kernel(const __nv_bfloat16* __restrict__ a, int ld_a,
@@ -1174,6 +1259,35 @@ int jvae_avgpool(const void* src, int ld_src, void* dst, int ld_dst, int N, int 
   const Geo g = make_geo(Ps, C, vec ? 8 : 1);
   NORM_DISPATCH(vec, avgpool_kernel, g, 0, (cudaStream_t)stream, reinterpret_cast<const __nv_bfloat16*>(src), ld_src,
                 reinterpret_cast<__nv_bfloat16*>(dst), ld_dst, H, W, k, Ps, g.nchunk, g.ppb, backward);
+  return JVAE_OK;
+}
+
+int jvae_upsample_nearest(const void* src, int ld_src, void* dst, int ld_dst, int N, int H, int W, int C, int s, int backward,
+                          void* stream) {
+  JVAE_CHECK_ARG(src && dst && N > 0 && H > 0 && W > 0 && C > 0 && ld_src >= C && ld_dst >= C, "bad arguments");
+  JVAE_CHECK_ARG(s >= 1 && (long long)H * s <= (1 << 20) && (long long)W * s <= (1 << 20), "up-sampling factor >= 1, output sides up to 2^20");
+  const bool vec = vec_ok(C, {ld_src, ld_dst}, {src, dst});
+  JVAE_CHECK_ARG(vec ? C <= 8 * NORM_MAX_THREADS : C <= NORM_MAX_THREADS, "too many channels for this layout");
+  const size_t P = backward ? (size_t)N * H * W : (size_t)N * H * s * W * s;
+  const Geo g = make_geo(P, C, vec ? 8 : 1);
+  NORM_DISPATCH(vec, upsample_nearest_kernel, g, 0, (cudaStream_t)stream, reinterpret_cast<const __nv_bfloat16*>(src), ld_src,
+                reinterpret_cast<__nv_bfloat16*>(dst), ld_dst, H, W, s, P, g.nchunk, g.ppb, backward);
+  return JVAE_OK;
+}
+
+int jvae_avgpool_pad(const void* src, int ld_src, void* dst, int ld_dst, int N, int H, int W, int C, int kh, int kw, int sh, int sw,
+                     int ph, int pw, int backward, void* stream) {
+  JVAE_CHECK_ARG(src && dst && N > 0 && H > 0 && W > 0 && C > 0 && ld_src >= C && ld_dst >= C, "bad arguments");
+  JVAE_CHECK_ARG(kh >= 1 && kw >= 1 && sh >= 1 && sw >= 1 && ph >= 0 && pw >= 0, "bad window");
+  JVAE_CHECK_ARG(2 * ph <= kh && 2 * pw <= kw, "padding must be at most half the kernel");
+  JVAE_CHECK_ARG(H + 2 * ph >= kh && W + 2 * pw >= kw, "the window is larger than the padded map");
+  const bool vec = vec_ok(C, {ld_src, ld_dst}, {src, dst});
+  JVAE_CHECK_ARG(vec ? C <= 8 * NORM_MAX_THREADS : C <= NORM_MAX_THREADS, "too many channels for this layout");
+  AvgGeo q{H, W, (H + 2 * ph - kh) / sh + 1, (W + 2 * pw - kw) / sw + 1, kh, kw, sh, sw, ph, pw};
+  const size_t P = backward ? (size_t)N * H * W : (size_t)N * q.Ho * q.Wo;
+  const Geo g = make_geo(P, C, vec ? 8 : 1);
+  NORM_DISPATCH(vec, avgpool_pad_kernel, g, 0, (cudaStream_t)stream, reinterpret_cast<const __nv_bfloat16*>(src), ld_src,
+                reinterpret_cast<__nv_bfloat16*>(dst), ld_dst, q, P, g.nchunk, g.ppb, backward);
   return JVAE_OK;
 }
 
