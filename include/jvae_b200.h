@@ -199,6 +199,16 @@ enum jvae_gemm_mode {
 int jvae_gemm_bf16(int mode, int M, int N, int K, const void* a, int lda, const void* b, int ldb,
                    const float* bias, int act, void* out_bf16, float* out_f32, int ldd,
                    float* col_stats, int accumulate, void* stream);
+/* The forward of Linear -> activation -> Dropout(p) in training mode (layers.py:177-181, cvae.py:207-211): jvae_gemm_bf16
+ * (mode NT only; accumulate 0 and col_stats NULL) whose epilogue multiplies act(.) by keep[row, col] / (1 - p).
+ *   keep[row, col] = word (col & 3) of Philox4x32-10(counter (col >> 2, row, pos_lo, pos_hi), key (seed_lo, seed_hi))
+ *                    >= floor(p * 2^32),   pos = offset + *offset_dev (offset_dev: one uint64 on the device, or NULL)
+ * so the mask depends on (seed, pos, row, col) alone.  p in [0, 1]; p == 1 writes zeros.  Advancing the device word after
+ * every call (the sampler's stream position, jvae_sample_fwd) gives a replayed CUDA graph fresh masks. */
+int jvae_gemm_bf16_dropout(int mode, int M, int N, int K, const void* a, int lda, const void* b, int ldb,
+                           const float* bias, int act, void* out_bf16, float* out_f32, int ldd,
+                           float* col_stats, int accumulate, float p, uint64_t seed, uint64_t offset,
+                           const uint64_t* offset_dev, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Convolutions as implicit GEMM on tcgen05, NHWC bf16 activations (nn.Conv2d / nn.ConvTranspose2d of the
@@ -310,6 +320,13 @@ int jvae_cast_f32_bf16_ld(const float* src, int ld_src, void* dst, int ld_dst, s
  * dbias (C) f32 += sum over pixels of dy (NULL = not wanted) */
 int jvae_act_bwd(const void* da, int ld_da, const void* a_out, int ld_a, size_t P, int C, int act, void* dy, int ld_dy,
                  float* dbias, void* stream);
+/* Backward of jvae_gemm_bf16_dropout's epilogue, in one launch: dz (M,N) bf16 = da * keep / (1 - p) * act', the mask
+ * regenerated from the same (p, seed, offset, *offset_dev) as the forward (pass a device copy of the position the forward read);
+ * act' from the saved post-dropout output a_out (relu: a_out > 0; leaky: sign of a_out; sigmoid: s (1 - s) with
+ * s = a_out (1 - p); none: 1, a_out may be NULL).  dbias (N) f32 = sum over rows of dz (WRITTEN, not accumulated), summed
+ * in a fixed order without atomics; either output may be NULL.  Any N; da, a_out, dz bf16 with leading dimensions >= N. */
+int jvae_act_dropout_bwd(const void* da, int ld_da, const void* a_out, int ld_a, int M, int N, int act, float p, uint64_t seed,
+                         uint64_t offset, const uint64_t* offset_dev, void* dz, int ld_dz, float* dbias, void* stream);
 /* MaxPool2d(k, stride >= k, padding 0, floor mode): out (N,(H-k)/stride+1,(W-k)/stride+1,C) */
 int jvae_maxpool_fwd(const void* in, int N, int H, int W, int C, int ld_in, int k, int stride, void* out, int ld_out, void* stream);
 /* gradient to the first maximum of each window (torch tie rule); `in` is the pooling input */

@@ -89,6 +89,8 @@ def lib():
         if not hasattr(L, name):
             raise NativeError(f'{LIB_PATH} does not export {name}: stale build')
     L.jvae_gemm_bf16.argtypes = [c_int, c_int, c_int, c_int, P, c_int, P, c_int, P, c_int, P, P, c_int, P, c_int, P]
+    L.jvae_gemm_bf16_dropout.argtypes = [c_int, c_int, c_int, c_int, P, c_int, P, c_int, P, c_int, P, P, c_int, P, c_int,
+                                         c_float, c_u64, c_u64, P, P]
     L.jvae_selftest.argtypes = [c_int]
     L.jvae_probe_descriptors.argtypes = [c_int]
     L.jvae_probe_poison.argtypes = [ctypes.c_uint, P]
@@ -113,6 +115,7 @@ def lib():
                                     P, P]
     L.jvae_bn_bwd.argtypes = [P, c_int, P, c_int, c_size_t, c_int, P, P, P, c_int, P, P, c_int, P, P, P]
     L.jvae_act_bwd.argtypes = [P, c_int, P, c_int, c_size_t, c_int, c_int, P, c_int, P, P]
+    L.jvae_act_dropout_bwd.argtypes = [P, c_int, P, c_int, c_int, c_int, c_int, c_float, c_u64, c_u64, P, P, c_int, P, P]
     L.jvae_bn_stats_ld.argtypes = [P, c_size_t, c_int, c_int, P, c_int, P]
     L.jvae_bn_preact_fwd.argtypes = [P, c_size_t, c_int, c_int, P, c_int, P, P, c_float, c_float, P, P, P, c_int, c_int, P,
                                      c_int, P, P]
@@ -491,6 +494,15 @@ def gemm_bf16(mode, M, N, K, a, lda, b, ldb, *, bias=None, act=0, out_bf16=None,
                                ldd if ldd is not None else N, ptr(col_stats), int(accumulate), stream()))     # accumulate: 0 / 1 / n >= 2 (split-K)
 
 
+def gemm_bf16_dropout(M, N, K, a, lda, b, ldb, *, p, seed, offset=0, offset_dev=None, bias=None, act=0, out_bf16=None,
+                      out_f32=None, ldd=None):
+    """include/jvae_b200.h: jvae_gemm_bf16_dropout -- act(a b^T + bias) * keep / (1 - p), the keep-mask drawn at stream position
+    offset + offset_dev[0] (offset_dev: int64 (1,) device tensor or None)"""
+    check(lib().jvae_gemm_bf16_dropout(GEMM_NT, M, N, K, ptr2d(a), lda, ptr2d(b), ldb, ptr(bias), act, ptr(out_bf16),
+                                       ptr(out_f32), ldd if ldd is not None else N, None, 0, float(p), seed, offset,
+                                       ptr(offset_dev), stream()))
+
+
 def rawptr(t):
     """device pointer of a tensor the caller has laid out itself (NHWC activations with padded channel strides)"""
     if t is None:
@@ -652,6 +664,12 @@ def cast_f32_bf16_ld(src, ld_src, dst, ld_dst, P, C):
 
 def act_bwd(da, ld_da, a_out, ld_a, P, C, act, dy, ld_dy, dbias):
     check(lib().jvae_act_bwd(rawptr(da), ld_da, rawptr(a_out), ld_a, P, C, act, rawptr(dy), ld_dy, rawptr(dbias), stream()))
+
+
+def act_dropout_bwd(da, ld_da, a_out, ld_a, M, N, act, p, seed, offset, offset_dev, dz, ld_dz, dbias):
+    """include/jvae_b200.h: jvae_act_dropout_bwd (dbias is written, not accumulated)"""
+    check(lib().jvae_act_dropout_bwd(rawptr(da), ld_da, rawptr(a_out), ld_a, M, N, act, float(p), seed, offset,
+                                     rawptr(offset_dev), rawptr(dz), ld_dz, rawptr(dbias), stream()))
 
 
 def maxpool_fwd(inp, N, H, W, C, ld_in, k, stride, out, ld_out):

@@ -93,4 +93,40 @@ __device__ __forceinline__ void st_stream16(void* p, uint4 v) {
                :: "l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
 }
 
+// ---------------------------------------------------------------- counter-based random numbers
+__device__ __forceinline__ uint32_t mulhi32(uint32_t a, uint32_t b) { return __umulhi(a, b); }
+
+// Philox4x32-10 (Salmon et al., SC'11), counter c[4], key k[2]
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+  const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    const uint32_t hi0 = mulhi32(M0, c.x), lo0 = M0 * c.x;
+    const uint32_t hi1 = mulhi32(M1, c.z), lo1 = M1 * c.z;
+    c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+    k.x += W0;
+    k.y += W1;
+  }
+  return c;
+}
+
+// Dropout keep-mask of the dense layers (jvae_gemm_bf16_dropout forward, jvae_act_dropout_bwd backward): element (row, col)
+// of the call at stream position `offset` is kept iff word (col & 3) of
+//     philox4x32_10(counter = (col >> 2, row, offset_lo, offset_hi), key = (seed_lo, seed_hi))
+// is >= drop_thresh = floor(p * 2^32) (a 64-bit threshold: p == 1 gives 2^32, which drops everything).  The mask depends
+// on nothing but (seed, offset, row, col): not on tile shapes, leading dimensions or which kernel regenerates it.
+// dropout_keep4 returns the keep bits of the four columns col4 .. col4 + 3 (col4 a multiple of 4) in bits 0..3.
+__device__ __forceinline__ uint32_t dropout_keep4(uint64_t seed, uint64_t offset, uint32_t row, uint32_t col4,
+                                                  uint64_t drop_thresh) {
+  const uint4 r = philox4x32_10(make_uint4(col4 >> 2, row, (uint32_t)offset, (uint32_t)(offset >> 32)),
+                                make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+  return (uint32_t)(r.x >= drop_thresh) | ((uint32_t)(r.y >= drop_thresh) << 1) | ((uint32_t)(r.z >= drop_thresh) << 2) |
+         ((uint32_t)(r.w >= drop_thresh) << 3);
+}
+// drop_thresh of a dropout probability p in [0, 1]
+inline uint64_t dropout_threshold(float p) { return (uint64_t)floor((double)p * 4294967296.0); }
+__device__ __forceinline__ bool dropout_keep(uint64_t seed, uint64_t offset, uint32_t row, uint32_t col, uint64_t drop_thresh) {
+  return (dropout_keep4(seed, offset, row, col & ~3u, drop_thresh) >> (col & 3)) & 1u;
+}
+
 }  // namespace jvae

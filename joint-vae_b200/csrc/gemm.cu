@@ -25,6 +25,10 @@ struct GemmParams {
   const float* bias;
   __nv_bfloat16* out_bf16;
   float* out_f32;
+  // dropout (the DROPOUT kernels only): keep-mask of csrc/common.cuh at stream position drop_offset + *drop_offset_dev
+  uint64_t seed, drop_offset, drop_thresh;
+  const uint64_t* drop_offset_dev;
+  float keep_scale;   // 1 / (1 - p); 0 when p == 1
 };
 
 template <int BN>
@@ -44,7 +48,8 @@ __device__ __forceinline__ float apply_act(float v, int act) {
   return v;
 }
 
-template <int BN, bool A_MN, bool B_MN>
+// DROPOUT: the epilogue multiplies act(.) by keep(row, col) / (1 - p) (dense-layer dropout, layers.py:177-181, cvae.py:207-211)
+template <int BN, bool A_MN, bool B_MN, bool DROPOUT>
 __global__ void __launch_bounds__(GEMM_THREADS)
 gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b, GemmParams p) {
   using S = GemmSmem<BN>;
@@ -134,6 +139,19 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
   } else {
     // ================= epilogue: warps 2..5, TMEM lane quarter = warp % 4 =================
     const int q = warp & 3;
+    // DROPOUT: the keep bits of the thread's row in the tile's BN columns (8 Philox draws per 32 columns), drawn while the
+    // MMAs run; kb[0] always holds the current chunk's (shifted down once per chunk: no dynamically indexed registers)
+    uint32_t kb[BN / 32];
+    if (DROPOUT) {
+      const uint64_t off = p.drop_offset + (p.drop_offset_dev ? *p.drop_offset_dev : 0ull);
+#pragma unroll
+      for (int c = 0; c < BN / 32; ++c) {
+        kb[c] = 0;
+#pragma unroll
+        for (int j = 0; j < 32; j += 4)
+          kb[c] |= dropout_keep4(p.seed, off, (uint32_t)(m0 + q * 32 + lane), (uint32_t)(n0 + c * 32 + j), p.drop_thresh) << j;
+      }
+    }
     mbar_wait(accum_bar, 0);
     tc_fence_after();
     const int row = m0 + q * 32 + lane;
@@ -141,6 +159,12 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
 #pragma unroll 1
     for (int c0 = 0; c0 < BN; c0 += 32) {
       if (n0 + c0 >= p.N) break;   // warp-uniform
+      uint32_t keep = 0;
+      if (DROPOUT) {
+        keep = kb[0];
+#pragma unroll
+        for (int c = 0; c + 1 < BN / 32; ++c) kb[c] = kb[c + 1];
+      }
       uint32_t r[32];
       tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, r);
       tmem_ld_wait();
@@ -171,6 +195,10 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
       } else if (p.act == JVAE_ACT_LEAKY) {
 #pragma unroll
         for (int j = 0; j < 32; ++j) v[j] = v[j] > 0.f ? v[j] : JVAE_LEAKY_SLOPE * v[j];
+      }
+      if (DROPOUT) {
+#pragma unroll
+        for (int j = 0; j < 32; ++j) v[j] = ((keep >> j) & 1u) ? v[j] * p.keep_scale : 0.f;
       }
       const size_t off = (size_t)row * p.ldd + n0 + c0;
       const bool full = (n0 + c0 + 32 <= p.N);
@@ -283,12 +311,12 @@ static int operand_tmap(CUtensorMap* t, const void* base, bool mn_major, int R, 
   return make_tmap_bf16(t, base, 2, dims, strides, box, nullptr, 128);
 }
 
-template <int BN, bool A_MN, bool B_MN>
+template <int BN, bool A_MN, bool B_MN, bool DROPOUT>
 static int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const GemmParams& p, cudaStream_t st) {
   using S = GemmSmem<BN>;
   static bool attr_done = false;
   if (!attr_done) {
-    JVAE_CUDA(cudaFuncSetAttribute(gemm_bf16_kernel<BN, A_MN, B_MN>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::TOTAL));
+    JVAE_CUDA(cudaFuncSetAttribute(gemm_bf16_kernel<BN, A_MN, B_MN, DROPOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::TOTAL));
     attr_done = true;
   }
   dim3 grid((p.M + GEMM_BM - 1) / GEMM_BM, (p.N + BN - 1) / BN, p.ksplit > 1 ? p.ksplit : 1);
@@ -297,18 +325,15 @@ static int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const GemmP
   const int num_kb = p.ksplit > 1 ? (num_kb_all + p.ksplit - 1) / p.ksplit : num_kb_all;
   q.stages = num_kb < S::STAGES ? (num_kb < 2 ? 2 : num_kb) : S::STAGES;
   const size_t smem = (size_t)q.stages * S::STAGE_BYTES + 256 + 1024;
-  gemm_bf16_kernel<BN, A_MN, B_MN><<<grid, GEMM_THREADS, smem, st>>>(ta, tb, q);
+  gemm_bf16_kernel<BN, A_MN, B_MN, DROPOUT><<<grid, GEMM_THREADS, smem, st>>>(ta, tb, q);
   JVAE_LAUNCH_CHECK();
   return JVAE_OK;
 }
 
-}  // namespace jvae
-
-using namespace jvae;
-
-extern "C" int jvae_gemm_bf16(int mode, int M, int N, int K, const void* a, int lda, const void* b, int ldb,
-                              const float* bias, int act, void* out_bf16, float* out_f32, int ldd, float* col_stats,
-                              int accumulate, void* stream) {
+// argument checks, tensor maps and parameters shared by both entry points; *bn receives the N tile
+static int prepare_gemm(int mode, int M, int N, int K, const void* a, int lda, const void* b, int ldb, const float* bias, int act,
+                        void* out_bf16, float* out_f32, int ldd, float* col_stats, int accumulate, CUtensorMap* ta,
+                        CUtensorMap* tb, GemmParams* p, int* bn) {
   JVAE_CHECK_ARG(mode >= JVAE_GEMM_NT && mode <= JVAE_GEMM_TN, "mode must be NT, NN or TN");
   JVAE_CHECK_ARG(M > 0 && N > 0 && K > 0, "M, N, K must be positive");
   JVAE_CHECK_ARG(a && b && (out_bf16 || out_f32), "a, b and one output are required");
@@ -325,17 +350,35 @@ extern "C" int jvae_gemm_bf16(int mode, int M, int N, int K, const void* a, int 
   const bool b_mn = (mode != JVAE_GEMM_NT);
   JVAE_CHECK_ARG(lda >= (a_mn ? M : K) && ldb >= (b_mn ? N : K), "leading dimension smaller than the row length");
   const int BN = (N > 64) ? 128 : 64;
+  int rc = operand_tmap(ta, a, a_mn, M, K, lda, GEMM_BM);
+  if (rc) return rc;
+  rc = operand_tmap(tb, b, b_mn, N, K, ldb, BN);
+  if (rc) return rc;
+  *p = GemmParams{};
+  p->M = M; p->N = N; p->K = K; p->ldd = ldd; p->act = act; p->accumulate = accumulate ? 1 : 0;
+  p->ksplit = accumulate >= 2 ? accumulate : 1;
+  p->bias = bias; p->out_bf16 = reinterpret_cast<__nv_bfloat16*>(out_bf16); p->out_f32 = out_f32;
+  *bn = BN;
+  return JVAE_OK;
+}
+
+}  // namespace jvae
+
+using namespace jvae;
+
+extern "C" int jvae_gemm_bf16(int mode, int M, int N, int K, const void* a, int lda, const void* b, int ldb,
+                              const float* bias, int act, void* out_bf16, float* out_f32, int ldd, float* col_stats,
+                              int accumulate, void* stream) {
   CUtensorMap ta, tb;
-  int rc = operand_tmap(&ta, a, a_mn, M, K, lda, GEMM_BM);
-  if (rc) return rc;
-  rc = operand_tmap(&tb, b, b_mn, N, K, ldb, BN);
-  if (rc) return rc;
   GemmParams p;
-  p.M = M; p.N = N; p.K = K; p.ldd = ldd; p.act = act; p.accumulate = accumulate ? 1 : 0;
-  p.ksplit = accumulate >= 2 ? accumulate : 1;
-  p.bias = bias; p.out_bf16 = reinterpret_cast<__nv_bfloat16*>(out_bf16); p.out_f32 = out_f32;
+  int BN;
+  const int rc = prepare_gemm(mode, M, N, K, a, lda, b, ldb, bias, act, out_bf16, out_f32, ldd, col_stats, accumulate, &ta,
+                              &tb, &p, &BN);
+  if (rc) return rc;
+  const bool a_mn = (mode == JVAE_GEMM_TN);
+  const bool b_mn = (mode != JVAE_GEMM_NT);
   cudaStream_t st = (cudaStream_t)stream;
-#define JVAE_GEMM_CASE(bn, am, bm) return launch_gemm<bn, am, bm>(ta, tb, p, st)
+#define JVAE_GEMM_CASE(bn, am, bm) return launch_gemm<bn, am, bm, false>(ta, tb, p, st)
   if (BN == 128) {
     if (!a_mn && !b_mn) JVAE_GEMM_CASE(128, false, false);
     if (!a_mn && b_mn) JVAE_GEMM_CASE(128, false, true);
@@ -346,4 +389,27 @@ extern "C" int jvae_gemm_bf16(int mode, int M, int N, int K, const void* a, int 
     JVAE_GEMM_CASE(64, true, true);
   }
 #undef JVAE_GEMM_CASE
+}
+
+extern "C" int jvae_gemm_bf16_dropout(int mode, int M, int N, int K, const void* a, int lda, const void* b, int ldb,
+                                      const float* bias, int act, void* out_bf16, float* out_f32, int ldd, float* col_stats,
+                                      int accumulate, float p, uint64_t seed, uint64_t offset, const uint64_t* offset_dev,
+                                      void* stream) {
+  JVAE_CHECK_ARG(p >= 0.f && p <= 1.f, "dropout probability p must be in [0, 1]");
+  JVAE_CHECK_ARG(mode == JVAE_GEMM_NT, "dropout applies to the forward GEMM (mode NT)");
+  JVAE_CHECK_ARG(accumulate == 0, "dropout does not accumulate or split the reduction");
+  JVAE_CHECK_ARG(col_stats == nullptr, "dropout takes no col_stats");
+  CUtensorMap ta, tb;
+  GemmParams q;
+  int BN;
+  const int rc = prepare_gemm(mode, M, N, K, a, lda, b, ldb, bias, act, out_bf16, out_f32, ldd, nullptr, 0, &ta, &tb, &q, &BN);
+  if (rc) return rc;
+  q.seed = seed;
+  q.drop_offset = offset;
+  q.drop_offset_dev = offset_dev;
+  q.drop_thresh = dropout_threshold(p);
+  q.keep_scale = p < 1.f ? 1.f / (1.f - p) : 0.f;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (BN == 128) return launch_gemm<128, false, false, true>(ta, tb, q, st);
+  return launch_gemm<64, false, false, true>(ta, tb, q, st);
 }

@@ -577,6 +577,68 @@ __global__ void __launch_bounds__(NORM_MAX_THREADS) act_bwd_kernel(const __nv_bf
   if (dbias) block_channel_reduce_f32<V, 1>(acc, chunk, C, s_acc, dbias);
 }
 
+// Dense-layer dropout backward: dz = da * keep(row, col) / (1 - p) * f'(.), keep regenerated from (seed, offset) with the
+// forward's dropout_keep4 (csrc/common.cuh); f' from the saved post-dropout output a_out (relu: a_out > 0, leaky: its sign,
+// sigmoid: s (1 - s) with s = a_out (1 - p)); dbias[c] = sum_row dz[row, c].  A block owns CT column chunks of V columns
+// over ALL rows (any width N: the grid grows with N, nothing is bounded by the block size), so each bias entry is summed by
+// one block in a fixed order (per-thread partials, then a shared-memory tree): no atomics, bit-identical run to run.
+constexpr int DROP_BWD_THREADS = 256;
+template <int V, int CT>
+__global__ void __launch_bounds__(DROP_BWD_THREADS) act_dropout_bwd_kernel(const __nv_bfloat16* __restrict__ da, int ld_da,
+                                                                           const __nv_bfloat16* __restrict__ aout, int ld_a,
+                                                                           int M, int N, int act, uint64_t seed, uint64_t offset,
+                                                                           const uint64_t* __restrict__ offset_dev,
+                                                                           uint64_t drop_thresh, float keep_scale, float keep_p,
+                                                                           __nv_bfloat16* dz, int ld_dz, float* dbias) {
+  constexpr int RT = DROP_BWD_THREADS / CT;      // threads along the rows
+  __shared__ float s_part[RT * CT * V];
+  const int ct = threadIdx.x % CT, rt = threadIdx.x / CT;
+  const int col0 = (blockIdx.x * CT + ct) * V;
+  const bool active = col0 < N;                  // V == 8 needs N % 8 == 0: a chunk is whole or absent
+  if (offset_dev) offset += *offset_dev;
+  float acc[V];
+#pragma unroll
+  for (int j = 0; j < V; ++j) acc[j] = 0.f;
+  if (active) {
+    for (int row = rt; row < M; row += RT) {
+      float g[V], o[V];
+      Vec<V>::load(da + (size_t)row * ld_da + col0, g);
+      if (act != JVAE_ACT_NONE) Vec<V>::load(aout + (size_t)row * ld_a + col0, o);
+      uint32_t keep;
+      if (V == 8)
+        keep = dropout_keep4(seed, offset, (uint32_t)row, (uint32_t)col0, drop_thresh) |
+               (dropout_keep4(seed, offset, (uint32_t)row, (uint32_t)col0 + 4, drop_thresh) << 4);
+      else
+        keep = dropout_keep(seed, offset, (uint32_t)row, (uint32_t)col0, drop_thresh);
+#pragma unroll
+      for (int j = 0; j < V; ++j) {
+        float d = 1.f;
+        if (act == JVAE_ACT_RELU) d = o[j] > 0.f ? 1.f : 0.f;
+        else if (act == JVAE_ACT_LEAKY) d = o[j] > 0.f ? 1.f : JVAE_LEAKY_SLOPE;
+        else if (act == JVAE_ACT_SIGMOID) { const float sg = o[j] * keep_p; d = sg * (1.f - sg); }
+        g[j] = ((keep >> j) & 1u) ? g[j] * keep_scale * d : 0.f;
+        acc[j] += g[j];
+      }
+      if (dz) Vec<V>::store(dz + (size_t)row * ld_dz + col0, g);
+    }
+  }
+  if (!dbias) return;                            // uniform for the grid
+#pragma unroll
+  for (int j = 0; j < V; ++j) s_part[(rt * CT + ct) * V + j] = acc[j];
+  __syncthreads();
+  for (int h = RT / 2; h > 0; h >>= 1) {
+    if (rt < h) {
+#pragma unroll
+      for (int j = 0; j < V; ++j) s_part[(rt * CT + ct) * V + j] += s_part[((rt + h) * CT + ct) * V + j];
+    }
+    __syncthreads();
+  }
+  if (rt == 0 && active) {
+#pragma unroll
+    for (int j = 0; j < V; ++j) dbias[col0 + j] = s_part[ct * V + j];
+  }
+}
+
 // ------------------------------------------------------------------------------------------------ pooling / up-sampling
 // k x k max pooling with stride s >= k, no padding, floor mode: out (N, (H-k)/s+1, (W-k)/s+1, C)
 template <int V>
@@ -1320,6 +1382,33 @@ int jvae_add_act(const void* a, int ld_a, const void* b, int ld_b, size_t P, int
   NORM_DISPATCH(vec, add_act_kernel, g, 0, (cudaStream_t)stream, reinterpret_cast<const __nv_bfloat16*>(a), ld_a,
                 reinterpret_cast<const __nv_bfloat16*>(b), ld_b, reinterpret_cast<__nv_bfloat16*>(out), ld_out, P, act,
                 g.nchunk, g.ppb);
+  return JVAE_OK;
+}
+
+int jvae_act_dropout_bwd(const void* da, int ld_da, const void* a_out, int ld_a, int M, int N, int act, float p, uint64_t seed,
+                         uint64_t offset, const uint64_t* offset_dev, void* dz, int ld_dz, float* dbias, void* stream) {
+  JVAE_CHECK_ARG(p >= 0.f && p <= 1.f, "dropout probability p must be in [0, 1]");
+  JVAE_CHECK_ARG(da && M > 0 && N > 0 && ld_da >= N, "bad arguments");
+  JVAE_CHECK_ARG(act == JVAE_ACT_NONE || (a_out && ld_a >= N), "activation output missing");
+  JVAE_CHECK_ARG(dz || dbias, "nothing to compute");
+  JVAE_CHECK_ARG(!dz || ld_dz >= N, "ld_dz < N");
+  const bool vec = vec_ok(N, {ld_da, a_out ? ld_a : 8, dz ? ld_dz : 8}, {da, a_out, dz});
+  const uint64_t thresh = dropout_threshold(p);
+  const float keep_scale = p < 1.f ? 1.f / (1.f - p) : 0.f;
+  const auto* A = reinterpret_cast<const __nv_bfloat16*>(da);
+  const auto* O = reinterpret_cast<const __nv_bfloat16*>(a_out);
+  auto* Z = reinterpret_cast<__nv_bfloat16*>(dz);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (vec) {          // 2 threads x 8 columns per row: 32-byte row segments
+    act_dropout_bwd_kernel<8, 2><<<(N / 8 + 1) / 2, DROP_BWD_THREADS, 0, st>>>(A, ld_da, O, ld_a, M, N, act, seed, offset,
+                                                                              offset_dev, thresh, keep_scale, 1.f - p, Z,
+                                                                              ld_dz, dbias);
+  } else {            // a warp reads 32 consecutive columns of a row
+    act_dropout_bwd_kernel<1, 32><<<(N + 31) / 32, DROP_BWD_THREADS, 0, st>>>(A, ld_da, O, ld_a, M, N, act, seed, offset,
+                                                                             offset_dev, thresh, keep_scale, 1.f - p, Z,
+                                                                             ld_dz, dbias);
+  }
+  JVAE_LAUNCH_CHECK();
   return JVAE_OK;
 }
 

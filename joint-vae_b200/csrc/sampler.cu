@@ -9,22 +9,6 @@ namespace jvae {
 
 constexpr int SAMPLE_THREADS = 128;
 
-__device__ __forceinline__ uint32_t mulhi32(uint32_t a, uint32_t b) { return __umulhi(a, b); }
-
-// Philox4x32-10 (Salmon et al., SC'11), counter c[4], key k[2]
-__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
-  const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const uint32_t hi0 = mulhi32(M0, c.x), lo0 = M0 * c.x;
-    const uint32_t hi1 = mulhi32(M1, c.z), lo1 = M1 * c.z;
-    c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
-    k.x += W0;
-    k.y += W1;
-  }
-  return c;
-}
-
 __device__ __forceinline__ float u01(uint32_t r) { return ((float)(r >> 8) + 0.5f) * (1.0f / 16777216.0f); }
 
 // one draw for flat element index idx of stream (seed, offset)

@@ -11,7 +11,14 @@ from torch import nn
 
 from . import _native as nat
 
-_rng_counters = {}      # device -> int64[1]: position of the sampler's Philox stream
+_rng_counters = {}      # device -> int64[1]: position of the Philox stream of the sampler and the dense-layer dropout
+
+
+def _rng_counter(device):
+    ctr = _rng_counters.get(device)
+    if ctr is None:
+        ctr = _rng_counters[device] = torch.zeros(1, dtype=torch.int64, device=device)
+    return ctr
 
 # Parameter epochs.  The fused Adam (csrc/optim.cu) and the BatchNorm kernels (running statistics) write parameters and
 # buffers through raw pointers, which autograd's version counters never see.  Every cache of derived weights (bf16
@@ -73,38 +80,62 @@ def _weight_bf16(w):
 
 
 class _LinearFn(torch.autograd.Function):
-    """y = act(x W^T + b) on tcgen05 (csrc/gemm.cu); dgrad / wgrad reuse the same kernel with MN-major operands."""
+    """y = act(x W^T + b) on tcgen05 (csrc/gemm.cu); dgrad / wgrad reuse the same kernel with MN-major operands.
+    dropout = p (training-mode nn.Dropout after the activation): the GEMM epilogue multiplies by a Philox keep-mask / (1 - p)
+    drawn at the device-side stream position (advanced after the call, like the sampler's), and the backward regenerates
+    the mask from a device copy of that position (jvae_act_dropout_bwd) instead of keeping it."""
 
     @staticmethod
-    def forward(ctx, x, w, b, act, out_dtype):
+    def forward(ctx, x, w, b, act, out_dtype, dropout):
         M, K = x.shape
         N = w.shape[0]
         xb = _bf16_ld8(x.detach())
         wb = _weight_bf16(w)
         out = torch.empty((M, N), dtype=out_dtype, device=x.device)
-        nat.gemm_bf16(nat.GEMM_NT, M, N, K, xb, _ld(xb), wb, _ld(wb), bias=b.detach() if b is not None else None,
-                      act=nat.ACT[act], out_bf16=out if out_dtype == torch.bfloat16 else None,
-                      out_f32=out if out_dtype == torch.float32 else None, ldd=N)
+        bias = b.detach() if b is not None else None
+        pos = None
+        if dropout is None:
+            nat.gemm_bf16(nat.GEMM_NT, M, N, K, xb, _ld(xb), wb, _ld(wb), bias=bias, act=nat.ACT[act],
+                          out_bf16=out if out_dtype == torch.bfloat16 else None,
+                          out_f32=out if out_dtype == torch.float32 else None, ldd=N)
+        else:
+            if out_dtype != torch.bfloat16:
+                raise NotImplementedError('the dropout GEMM writes bf16 activations')
+            ctr = _rng_counter(x.device)
+            pos = ctr.clone()           # the position this call draws at (the counter moves on before the backward)
+            ctx.seed = torch.initial_seed() & 0xFFFFFFFFFFFFFFFF
+            nat.gemm_bf16_dropout(M, N, K, xb, _ld(xb), wb, _ld(wb), p=dropout, seed=ctx.seed, offset_dev=ctr, bias=bias,
+                                  act=nat.ACT[act], out_bf16=out, ldd=N)
+            ctr.add_(1)
         ctx.act = act
+        ctx.dropout = dropout
         ctx.has_bias = b is not None
         ctx.x_dtype = x.dtype
-        ctx.save_for_backward(xb, wb, out if act in ('relu', 'sigmoid', 'leaky') else None)
+        ctx.save_for_backward(xb, wb, out if act in ('relu', 'sigmoid', 'leaky') else None, pos)
         return out
 
     @staticmethod
     def backward(ctx, dy):
-        xb, wb, out = ctx.saved_tensors
+        xb, wb, out, pos = ctx.saved_tensors
         M, K = xb.shape
         N = wb.shape[0]
-        if ctx.act == 'relu':
+        db = None
+        if ctx.dropout is not None:     # dz = dy * keep / (1 - p) * act' and the bias gradient, one launch
+            da = dy.to(torch.bfloat16).contiguous()
+            dzb = torch.empty((M, _r8(N)), dtype=torch.bfloat16, device=dy.device)[:, :N]
+            if ctx.has_bias and ctx.needs_input_grad[2]:
+                db = torch.empty(N, dtype=torch.float32, device=dy.device)
+            nat.act_dropout_bwd(da, _ld(da), out, N, M, N, nat.ACT[ctx.act], ctx.dropout, ctx.seed, 0, pos, dzb, _ld(dzb), db)
+        elif ctx.act == 'relu':
             dy = dy * (out > 0)
         elif ctx.act == 'sigmoid':
             o = out.float()
             dy = dy.float() * o * (1 - o)
         elif ctx.act == 'leaky':        # the output keeps the sign of the pre-activation
             dy = torch.where(out > 0, dy, dy * nat.LEAKY_SLOPE)
-        dzb = _bf16_ld8(dy)
-        dx = dw = db = None
+        if ctx.dropout is None:
+            dzb = _bf16_ld8(dy)
+        dx = dw = None
         if ctx.needs_input_grad[0]:
             dx = torch.empty((M, K), dtype=ctx.x_dtype, device=dy.device)
             nat.gemm_bf16(nat.GEMM_NN, M, K, N, dzb, _ld(dzb), wb, _ld(wb),
@@ -113,16 +144,17 @@ class _LinearFn(torch.autograd.Function):
         if ctx.needs_input_grad[1]:
             dw = torch.empty((N, K), dtype=torch.float32, device=dy.device)
             nat.gemm_bf16(nat.GEMM_TN, N, K, M, dzb, _ld(dzb), xb, _ld(xb), out_f32=dw, ldd=K)
-        if ctx.has_bias and ctx.needs_input_grad[2]:
+        if ctx.has_bias and ctx.needs_input_grad[2] and ctx.dropout is None:
             db = dy.float().sum(0)
-        return dx, dw, db, None, None
+        return dx, dw, db, None, None, None
 
 
-def linear(x, w, b, act='linear', out_dtype=torch.bfloat16):
-    """x (M,K) -> act(x W^T + b) (M,N).  act in linear|relu|sigmoid."""
+def linear(x, w, b, act='linear', out_dtype=torch.bfloat16, dropout=None):
+    """x (M,K) -> act(x W^T + b) (M,N).  act in linear|relu|sigmoid|leaky.  dropout = p: followed by a training-mode
+    Dropout(p) (bf16 output only)."""
     if not x.is_cuda:
         raise nat.NativeError('joint-vae_b200 runs on CUDA devices only (there is no CPU fallback); got a CPU tensor')
-    return _LinearFn.apply(x, w, b, act, out_dtype)
+    return _LinearFn.apply(x, w, b, act, out_dtype, dropout)
 
 
 _ACT_OF = {nn.ReLU: 'relu', nn.Sigmoid: 'sigmoid', nn.Identity: 'linear', nn.LeakyReLU: 'leaky'}
@@ -148,7 +180,9 @@ def _is_conv_type(m):
 
 def run_sequential(seq, x, out_dtype=None, image_out=False):
     """Executes an nn.Sequential container built by the reference-style constructors.
-    Linear(+ReLU/Sigmoid/Identity) pairs become one fused GEMM; conv-type runs go to run_conv_stack.
+    Linear(+ReLU/Sigmoid/Identity)(+Dropout) runs become one fused GEMM: the Dropout is applied in the GEMM epilogue when the
+    container is training and skipped in eval mode; a Dropout anywhere else raises NotImplementedError.  Conv-type runs go to
+    run_conv_stack.
     image_out: a conv stack that ends the container returns its result as a channels_last bf16 tensor (the layout the
     fused ELBO kernel reads) instead of fp32 NCHW."""
     mods = list(seq)
@@ -164,8 +198,13 @@ def run_sequential(seq, x, out_dtype=None, image_out=False):
             if i + 1 < n and _act_name(mods[i + 1]) is not None:
                 act = _act_name(mods[i + 1])
                 i += 1
-            dt = out_dtype if (last_linear and out_dtype is not None) else torch.bfloat16
-            x = linear(x, m.weight, m.bias, act=act, out_dtype=dt)
+            p = None
+            if i + 1 < n and isinstance(mods[i + 1], nn.Dropout):
+                if seq.training:
+                    p = float(mods[i + 1].p)
+                i += 1
+            dt = out_dtype if (last_linear and out_dtype is not None and p is None) else torch.bfloat16
+            x = linear(x, m.weight, m.bias, act=act, out_dtype=dt, dropout=p)
         elif _is_conv_type(m):
             j = i
             while j < n and (_is_conv_type(mods[j]) or type(mods[j]) in _ACT_OF):
@@ -175,7 +214,8 @@ def run_sequential(seq, x, out_dtype=None, image_out=False):
             x = run_conv_stack(mods[i:j], x, image_out=image_out and (j == n or tail_is_view))
             i = j - 1
         elif isinstance(m, nn.Dropout):
-            x = torch.nn.functional.dropout(x, m.p, seq.training)
+            raise NotImplementedError(f'{type(m).__name__} at index {i} of the container: dropout has a native kernel only '
+                                      'after a Linear (+ activation)')
         elif type(m) in _ACT_OF:
             x = m(x)
         elif any(True for _ in m.parameters()):
@@ -204,9 +244,7 @@ class _SampleFn(torch.autograd.Function):
         head = nat.f32c(head.detach())
         ctr = None
         if eps_in is None:      # Philox stream position on the device, advanced after every draw (graph replays stay fresh)
-            ctr = _rng_counters.get(head.device)
-            if ctr is None:
-                ctr = _rng_counters[head.device] = torch.zeros(1, dtype=torch.int64, device=head.device)
+            ctr = _rng_counter(head.device)
         mu, lv, z, _, eps, en = nat.sample_fwd(head, L, K, eps_in=nat.f32c(eps_in), seed=seed, offset=offset,
                                                is_sampled=is_sampled, uniform=uniform, offset_dev=ctr)
         if ctr is not None:
